@@ -42,6 +42,8 @@ BYTES_CORE = 59          # SURVEY.md section 8(d): 25 B read + 34 B written per 
 BYTES_ONEHOT_F32 = 1024  # fp32 (16 classes x 16 cells) observation written per env step
 BURN_IN = 256            # steps from reset() to steady-state boards (SURVEY.md section 8d, config 3)
 STATS_EVERY = 64         # BASELINE configs[3]: the episode statistics are all-reduced every 64 steps (24 integers)
+DUMP_GAMES = 1 << 15     # --dump-outputs: games sampled from the batch (1 KiB of fp32 one-hot + 0.2 KiB of other fields each)
+DUMP_SEED = 2048         # --dump-outputs: seed of that sample, so that the same --games-per-gpu always gives the same slots
 
 
 def parse_args() -> argparse.Namespace:
@@ -65,7 +67,13 @@ def parse_args() -> argparse.Namespace:
                    help="CPU arm: the staged Numba reference (oracle/_ref), the C port (oracle/), or the first that is available")
     p.add_argument("--burn-in", type=int, default=BURN_IN, help="untimed steps from reset() to steady state")
     p.add_argument("--clock-interval-ms", type=float, default=50.0, help="NVML sampling period during the timed region")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step returned (a fixed sample of the games) as "
+                        "DIR/<name>.npy in float32 or float64, to compare two builds output for output; rank 0 only")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def workload_name(games_per_gpu: int, burn_in: int = BURN_IN) -> str:
@@ -514,6 +522,39 @@ def pcie_ceiling(torch, dist, dev, world: int, h2d_bytes: int, d2h_bytes: int, r
     }
 
 
+def dump_outputs(env, result, out_dir: str, slot_base: int) -> None:
+    """Write what the last timed step returned, so that two builds can be compared output for output on the same command
+    line: the fields of its ``VecStepResult``, the fused one-hot observation and the game ids for a fixed, seeded sample of
+    DUMP_GAMES games (their global slots in ``slot.npy``), which of those games the step's auto-reset restarted, how many
+    it restarted in all, and the episode statistics of the whole batch.  Integers wider than 16 bits are written as
+    float64 (exact), everything else as float32: at most ~40 MB."""
+    import numpy as np
+    import torch
+
+    m = env._size
+    sel = np.sort(np.random.default_rng(DUMP_SEED).choice(m, size=min(m, DUMP_GAMES), replace=False))
+    idx = torch.from_numpy(sel).to(env.device)
+    out = {"slot": torch.from_numpy(sel + slot_base)}
+    for key in result.keys():
+        try:
+            out[key] = result[key][idx]
+        except KeyError:  # `merged` is not tracked on the timed path
+            continue
+    out["onehot"] = env.observations_onehot()[idx]
+    out["id"] = env._id[idx]
+    (reset,) = env.last_reset()
+    was_reset = torch.zeros((m,), dtype=torch.bool, device=env.device)
+    was_reset[reset.long()] = True
+    out["reset"] = was_reset[idx]
+    out["reset_count"] = torch.tensor([reset.numel()])
+    out["episode_stats"] = env.episode_stats_tensor()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        t = t.cpu()
+        wide = t.dtype == torch.float64 or (not t.dtype.is_floating_point and t.dtype.itemsize > 2)
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.to(torch.float64 if wide else torch.float32).numpy())
+
+
 def run_b200_arm(args: argparse.Namespace) -> None:
     import numpy as np
     import torch
@@ -583,6 +624,7 @@ def run_b200_arm(args: argparse.Namespace) -> None:
             pending.append((None, None, sums, mx))
 
     fused = not args.no_fused_reset
+    last_result = [None]  # what the last step returned to its caller (--dump-outputs)
 
     def run_steps(e, n: int, kernel_events=None) -> int:
         reduces = 0
@@ -593,7 +635,7 @@ def run_b200_arm(args: argparse.Namespace) -> None:
                 kernel_events[i][0].record()
             # fused: the auto-reset rides inside the step kernel (same arrays afterwards as prepare() + step_random(),
             # tests/test_fused_autoreset.py); a one-block-per-32k-games scan of the terminated flags ranks the resets first
-            e.step_random(auto_reset=fused)
+            last_result[0] = e.step_random(auto_reset=fused)
             if kernel_events is not None:
                 kernel_events[i][1].record()
             if kernel_events is not None and (i + 1) % stats_every == 0:
@@ -635,6 +677,8 @@ def run_b200_arm(args: argparse.Namespace) -> None:
     if os.environ.get("ML2048_BENCH_DEBUG"):
         print(f"[debug] prepare gaps ms: min {gaps[0]:.3f} p50 {gaps[len(gaps)//2]:.3f} p90 {gaps[int(len(gaps)*0.9)]:.3f} max {gaps[-1]:.3f}",
               file=sys.stderr)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, last_result[0], args.dump_outputs, slot_base)
 
     # the collective by itself: the same two all-reduces, blocking, back to back (device-timed, max over ranks)
     collective_ms = None
@@ -930,6 +974,9 @@ def bind_to_gpu_numa_node(local_rank: int) -> str:
 
 
 def main() -> None:
+    # the benchmark writes nothing into the tree it runs from (which may be read-only): not even bytecode of the modules
+    # build() never imported, such as oracle/oracle.py of the CPU baseline
+    sys.dont_write_bytecode = True
     args = parse_args()
     # exactly ONE line may reach stdout (the driver parses it): everything libraries print to fd 1 (NCCL's version
     # banner, for one) is sent to stderr, and the JSON line is written to the saved descriptor at the end

@@ -12,7 +12,7 @@ infrastructure).  From it these tests import ``VecRunner`` + ``RunnerStats`` (ru
     ``(use, step, game)`` buffers) and the ``eval_perf.py:66-102`` loop are replayed line for line;
   * ``_data[slot]["id"].item()`` (replay.py:147-151) is served from one host snapshot per prepare(), not nine gathers a slot.
 
-CPU part (no GPU): the staged tree is intact and imports.
+CPU part (no GPU): the staged tree is intact and imports.  The ``_data`` lookup test needs no staged tree.
 """
 
 from __future__ import annotations
@@ -177,9 +177,8 @@ def test_trainer_on_stepped_copies_and_lockstep_with_the_numba_reference(refpkg)
 
 
 @pytest.mark.gpu
-@needs_ref
 @pytest.mark.parametrize("m", [3000, 65536, (1 << 20) + 1])
-def test_data_view_serves_recorder_lookups_without_per_slot_round_trips(refpkg, m):
+def test_data_view_serves_recorder_lookups_without_per_slot_round_trips(m):
     """replay.py:147-151 reads ``game._data[slot]["id"].item()`` per reset slot in a Python loop -- 65 536 times at
     eval_perf.py's first prepare().  The view serves them from ONE host snapshot (or, above 2^20 games, one gather per
     call), and fancy/slice/negative keys agree with the plain field arrays."""
