@@ -15,6 +15,9 @@
 // against the CPU oracle without a GPU; the #else branch below emulates the four intrinsics it uses.
 #pragma once
 #include <stdint.h>
+#if !defined(__CUDACC__)
+#include <math.h>  // expf / logf / fmaxf of the sampler; included here because <cmath> breaks when first opened inside the namespace
+#endif
 
 #if defined(__CUDACC__)
 #define ML2048_FN __device__ __forceinline__
@@ -636,8 +639,8 @@ ML2048_FN uint32_t slot_word(uint64_t slot, uint64_t counter, uint64_t seed, uin
 // Masked categorical sample (policy/actor_critic.py:56-76): invalid actions get finfo.min, the logits are
 // normalised as torch's Categorical does (x - logsumexp(x), logsumexp = max + log(sum(exp(x - max)))), one
 // uniform u in [0,1) picks the action by inverse CDF.  `mask_bits` bit k = action k valid.  Returns the action
-// and its log-probability.  (Device only: uses expf/logf.)
-#if defined(__CUDACC__)
+// and its log-probability.  The host build (tests/host_shim) uses the C library's expf/logf, the device build CUDA's; both
+// are checked against a float64 reference.
 ML2048_FN uint32_t sample_masked_categorical(float l0, float l1, float l2, float l3, uint32_t mask_bits, uint32_t rnd,
                                              float &log_prob)
 {
@@ -660,6 +663,5 @@ ML2048_FN uint32_t sample_masked_categorical(float l0, float l1, float l2, float
     log_prob = la - lse;
     return action;
 }
-#endif
 
 }  // namespace ml2048

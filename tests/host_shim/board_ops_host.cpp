@@ -130,4 +130,14 @@ void hs_first_empty_batch(const uint8_t *keys, const uint8_t *boards, int64_t n,
     for (int64_t i = 0; i < n; ++i) cells[i] = hs_first_empty(keys + 16 * i, boards + 16 * i);
 }
 
+// logits (n,4) f32, bits (n,) = 4-bit valid masks, words (n,) = the policy's uniform words
+void hs_sample_masked_categorical_batch(const float *logits, const uint8_t *bits, const uint32_t *words, int64_t n,
+                                        uint8_t *actions, float *log_probs)
+{
+    for (int64_t i = 0; i < n; ++i) {
+        const float *l = logits + 4 * i;
+        actions[i] = (uint8_t)sample_masked_categorical(l[0], l[1], l[2], l[3], bits[i], words[i], log_probs[i]);
+    }
+}
+
 }  // extern "C"

@@ -2,7 +2,8 @@
 The product's device arithmetic (ml2048_b200/csrc/board_ops.cuh) compiled as plain C++ (tests/host_shim)
 and checked against the CPU oracle / golden fixtures WITHOUT a GPU: every 4-cell line in every board
 position and direction (18^4 x 4 x 4), the reference-generated board set, random boards for the mask,
-the replay spawn position, and Philox against its published known-answer vectors.
+the replay spawn position, and Philox against its published known-answer vectors.  The masked categorical sampler is
+checked against the float64 reference of tests/_rollout_ref.py.
 """
 
 from __future__ import annotations
@@ -42,6 +43,9 @@ def shim():
     lib.hs_philox.argtypes = [vp, vp, vp]
     lib.hs_philox2.argtypes = [vp, u32, vp]
     lib.hs_slot_draws.argtypes = [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint64, u32, vp]
+    lib.hs_slot_word.argtypes = [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint64, u32]
+    lib.hs_slot_word.restype = u32
+    lib.hs_sample_masked_categorical_batch.argtypes = [vp, vp, vp, i64, vp, vp]
     return lib
 
 
@@ -263,13 +267,80 @@ def test_slot_draws_key_schedule(shim):
 def test_slot_word_serves_slot_pairs(shim):
     """slot_word: the policy / spawn word of a global slot is one half of the Philox block of its slot PAIR (index = slot >> 1;
     even slot -> .x, odd slot -> .y), for every stream tag."""
-    shim.hs_slot_word.argtypes = [ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint32]
-    shim.hs_slot_word.restype = ctypes.c_uint32
     out = np.zeros(2, np.uint32)
     for slot in (0, 1, 2, 3, 1000, 1001, (1 << 33) + 4, (1 << 33) + 5, 2**40 - 1):
         for counter, seed, tag in ((0, 0, 0), (77, 123, 0), (77, 123, 0x40000000), ((3 << 32) + 1, (9 << 32) + 4, 0)):
             shim.hs_slot_draws(slot >> 1, counter, seed, tag, out.ctypes.data)
             assert shim.hs_slot_word(slot, counter, seed, tag) == int(out[slot & 1])
+
+
+def test_policy_words_reference(shim):
+    """The tests' NumPy policy words (_rollout_ref.policy_words) == slot_word of the header and == the slot-pair formula over
+    the library's host Philox2x32-10, for slot bases odd and beyond 2^32, counters and seeds beyond 2^32."""
+    from _rollout_ref import policy_words
+
+    from ml2048_b200 import _lib, build
+
+    build.build()  # nvcc cross-compiles without a GPU; no-op when up to date
+    lib = _lib.load()
+    out2 = np.zeros(2, np.uint32)
+    for base, counter, seed in ((0, 0, 0), (5001, 77, 123), ((1 << 34) + 17, (3 << 32) + 1, (9 << 32) + 4),
+                                ((1 << 33) + 1, 2**64 - 1, 2**64 - 1)):
+        slots = base + np.arange(64, dtype=np.uint64)
+        got = policy_words(slots, counter, seed)
+        for s, word in zip(slots.tolist(), got.tolist()):
+            assert word == shim.hs_slot_word(s, counter, seed, 0), (s, counter, seed)
+            key = (seed & 0xFFFFFFFF) ^ (((seed >> 32) * 0x9E3779B9) & 0xFFFFFFFF)
+            pair = s >> 1
+            c = np.array([pair & 0xFFFFFFFF, (counter & 0xFFFFFFFF) ^ (((counter >> 32) * 0x85EBCA6B) & 0xFFFFFFFF)
+                          ^ (((pair >> 32) * 0xC2B2AE35) & 0xFFFFFFFF)], np.uint32)
+            lib.ml2048_philox2x32_10(c.ctypes.data, key, out2.ctypes.data)
+            assert word == int(out2[s & 1]), (s, counter, seed)
+
+
+def _host_sampler(shim, words):
+    def sample(logits, valid):
+        n = logits.shape[0]
+        bits = ((valid != 0) * (1 << np.arange(4))).sum(axis=1).astype(np.uint8)
+        actions = np.empty(n, np.uint8)
+        log_probs = np.empty(n, np.float32)
+        shim.hs_sample_masked_categorical_batch(np.ascontiguousarray(logits, np.float32).ctypes.data, bits.ctypes.data,
+                                                words.ctypes.data, n, actions.ctypes.data, log_probs.ctypes.data)
+        return actions, log_probs
+
+    return sample
+
+
+def test_masked_categorical_sampler_against_float64(shim):
+    """sample_masked_categorical compiled for the host, per logit class (randn*3, one dominant logit 80-120 above the rest,
+    +-1e4, +-1e30, ties, and u placed on a CDF boundary) over all 16 masks with valid bytes 1..255: the inverse-CDF action
+    of the float64 reference (either neighbour within 4*2^-24 of a boundary) and its log_softmax within
+    2^-22 (|l_a| + |max logit|) + 2^-21."""
+    import _rollout_ref as ref
+
+    rng = np.random.default_rng(2024)
+    n = 1 << 16
+    words = ref.policy_words((1 << 34) + 17 + np.arange(n, dtype=np.uint64), (3 << 32) + 1, 0x9E3779B97F4A7C15)
+    sample = _host_sampler(shim, words)
+    seen = {}
+    for name in ref.LOGIT_CLASSES:
+        logits = ref.sampler_logits(name, rng, words)
+        valid = ref.random_masks(rng, n)
+        if name == "boundary":
+            valid = ref.boundary_valid(valid)
+        actions, log_probs = sample(logits, valid)
+        seen[name] = ref.check_sampler(logits, valid, words, actions, log_probs, adversarial=name == "boundary", what=name)
+    assert seen["boundary"]["boundary_rows"] > n // 4  # the adversarial class does reach the neighbour rule
+
+
+def test_masked_categorical_sampler_exact_cases(shim):
+    """One valid / no valid action, equal logits (including uniforms on the 1/3 and 2/3 boundaries), NaN / +-inf logits
+    masked or valid: exact outcomes (_rollout_ref.check_sampler_exact)."""
+    import _rollout_ref as ref
+
+    words = ref.policy_words(5001 + np.arange(4099, dtype=np.uint64), 77, 123)
+    words[:8] = (np.array([0x555555, 0x555556, 0xAAAAAA, 0xAAAAAB] * 2, np.uint32) << 8) | np.arange(8, dtype=np.uint32) * 31
+    ref.check_sampler_exact(_host_sampler(shim, words), words, np.random.default_rng(7))
 
 
 def test_hypothesis_boards_against_oracle(shim, oracle):
