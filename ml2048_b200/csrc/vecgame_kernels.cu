@@ -15,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <type_traits>
 #include <utility>
 
 #include "../../include/ml2048_b200.h"
@@ -207,11 +208,14 @@ __device__ __forceinline__ void write_onehot_warp(uint4 board, void *out_base, i
         store_streaming(out + piece, P::make(&board, 0, piece));
 }
 
-__device__ __forceinline__ void write_onehot_warp_dyn(int dtype, uint4 board, void *out_base, int64_t game, int lane)
+// Calls f(std::integral_constant<int, dtype>()) for the one-hot dtype of a prepare(): the writers of the reset rows are
+// compiled per dtype.  Any other value writes nothing (the host rejects it before the launch).
+template <class F>
+__device__ __forceinline__ void with_onehot_dtype(int dtype, F &&f)
 {
-    if (dtype == ML2048_ONEHOT_F32) write_onehot_warp<ML2048_ONEHOT_F32>(board, out_base, game, lane);
-    else if (dtype == ML2048_ONEHOT_BF16) write_onehot_warp<ML2048_ONEHOT_BF16>(board, out_base, game, lane);
-    else if (dtype == ML2048_ONEHOT_U8) write_onehot_warp<ML2048_ONEHOT_U8>(board, out_base, game, lane);
+    if (dtype == ML2048_ONEHOT_F32) f(std::integral_constant<int, ML2048_ONEHOT_F32>());
+    else if (dtype == ML2048_ONEHOT_BF16) f(std::integral_constant<int, ML2048_ONEHOT_BF16>());
+    else if (dtype == ML2048_ONEHOT_U8) f(std::integral_constant<int, ML2048_ONEHOT_U8>());
 }
 
 // The random inputs of one prepare(): scalar arguments, or the pre-drawn schedule entry a CUDA graph replays.
@@ -222,10 +226,14 @@ struct PrepDraws {
     const uint8_t *perm_table;
 };
 
-__device__ __forceinline__ PrepDraws load_prep_draws(const ml2048_prepare_args &a)
+// The draws of a prepare(): the scalar arguments of `a`, or when `scheduled` the prepare() half of its schedule entry
+// (prepare() draws with the entry's Philox counter, the step with the next one: step_draws).  `a` is an ml2048_prepare_args,
+// or the ml2048_step_args of a step with the auto-reset fused in (reset_draws).
+template <class Args>
+__device__ __forceinline__ PrepDraws prep_draws(const Args &a, uint64_t philox_counter, bool scheduled)
 {
-    PrepDraws d{a.rand_base, a.two_mask, a.philox_counter, a.randperm};
-    if (a.sched) {
+    PrepDraws d{a.rand_base, a.two_mask, philox_counter, a.randperm};
+    if (scheduled) {
         const ml2048_sched_entry e = a.sched[*a.sched_cursor];
         d.rand_base = e.rand_base;
         d.two_mask = e.two_mask;
@@ -272,6 +280,89 @@ __device__ __forceinline__ uint4 fresh_board(const PrepDraws &d, uint64_t slot, 
     return make_uint4(r0, r1, r2, r3);
 }
 
+// ---- what the two step kernels share --------------------------------------------------------
+
+// What a step launch draws once: the step's random schedule.
+struct StepDraws {
+    int64_t rand_seed;
+    uint32_t two_mask;
+    uint64_t philox_counter;
+    const uint8_t *keys_table;
+};
+
+// The scalar arguments, or (`scheduled`) the step half of the pre-drawn entry a CUDA graph replays, whose cursor the launch
+// then advances.
+__device__ __forceinline__ StepDraws step_draws(const ml2048_step_args &a, bool scheduled)
+{
+    StepDraws d{a.rand_seed, a.two_mask, a.philox_counter, a.randperm_keys};
+    if (scheduled) {
+        const int64_t cursor = *a.sched_cursor;
+        const ml2048_sched_entry e = a.sched[cursor];
+        d.rand_seed = e.rand_seed;
+        d.two_mask = e.two_mask;
+        d.philox_counter = e.philox_counter + 1ull;
+        d.keys_table += (int64_t)e.table * a.table_stride;
+        if (a.sched_cursor_next && blockIdx.x == 0 && threadIdx.x == 0) *a.sched_cursor_next = cursor + 1;
+    }
+    return d;
+}
+
+// The draws of the prepare() that a step with the auto-reset fused in stands in for.  Its 2-vs-4 mask is the step's (one
+// schedule entry serves both): reusing the step's register instead of loading the entry's field again keeps the pair kernel
+// from spilling more.
+__device__ __forceinline__ PrepDraws reset_draws(const ml2048_step_args &a, const StepDraws &step, bool scheduled)
+{
+    PrepDraws d = prep_draws(a, a.prepare_philox_counter, scheduled);
+    d.two_mask = step.two_mask;
+    return d;
+}
+
+// Row (rand_seed + global slot) mod 1024 of the spawn keys (game_numba.py:681, :733); the low bits of the 32-bit sum are those of
+// the 64-bit one.
+__device__ __forceinline__ uint32_t spawn_row(int64_t rand_seed, uint64_t slot)
+{
+    return ((uint32_t)rand_seed + (uint32_t)slot) & (uint32_t)(kRandRows - 1);
+}
+
+// The fused auto-reset of finished game g + j (see ml2048_step_args::reset_rank): a fresh board and its mask, written back
+// into the INPUT buffers (prev_state / prev_valid_actions of this step are the post-reset board and mask,
+// game_numba.py:672-673), id = id_base + order (`order`: the slot-ordered rank of the game among this launch's resets,
+// :641-644), entry `order` of the index list, age 0.  The caller plays the returned board from step 0, score 0; the step's own
+// stores write the rest.  (The pair kernel passes its first game as a 32-bit g and j = 0 or 1, so that the reset computes its
+// addresses the way the rest of that kernel does; a 64-bit g0 + j changes the SASS of the whole kernel.)
+template <int kRng, typename Index>
+__device__ __forceinline__ uint4 reset_in_step(const ml2048_step_args &a, const PrepDraws &d, Index g, int j, int32_t id_base,
+                                               int32_t order, bool write_index, bool clear_age, uint32_t &mask)
+{
+    const uint4 bd = fresh_board<kRng, true>(d, (uint64_t)(a.slot_base + g + j), a.philox_seed, mask);
+    reinterpret_cast<uint4 *>(const_cast<void *>(a.board_in))[g + j] = bd;
+    reinterpret_cast<uint32_t *>(const_cast<void *>(a.valid_in))[g + j] = mask;
+    a.id[g + j] = id_base + order;
+    if (write_index && (int64_t)order < a.num_games) a.reset_indices[order] = (int64_t)g + j;
+    if (clear_age) a.age[g + j] = 0;
+    return bd;
+}
+
+// reward_fn (game_numba.py:728, :408-504) of a move from `old` to `now` that fused `f` and gained `gain`; kNormalReward:
+// reward_fn_normal, known at compile time.
+template <bool kNormalReward>
+__device__ __forceinline__ float step_reward(int32_t kind, const Fusions &f, uint4 now, uint4 old, float gain)
+{
+    if (kNormalReward || kind == ML2048_REWARD_NORMAL) return gain;
+    if (kind == ML2048_REWARD_IMPROVED) {
+        // potential shaping on cell 0, game_numba.py:455-466 (all terms are exact integers in f32: |extra| <= 2^23)
+        const uint32_t s0 = now.x & 0xffu, p0 = old.x & 0xffu;
+        const int extra = (s0 ? (64 << s0) : 0) - (p0 ? (64 << p0) : 0);
+        return gain + (float)extra;
+    }
+    if (kind == ML2048_REWARD_RANK) return (float)fusion_rank(f);
+    if (kind == ML2048_REWARD_MAXCELL) {
+        const uint32_t cur = max_cell(now.x, now.y, now.z, now.w), prev = max_cell(old.x, old.y, old.z, old.w);
+        return (float)fusion_count(f) + ((cur > prev) ? (float)(1u << cur) : 0.0f);
+    }
+    return gain;
+}
+
 // ---- the step kernel ------------------------------------------------------------------------
 
 // direction -> permute selectors of the move (board_ops.cuh): 128 bytes that live in L1; a game's row is fetched with two
@@ -313,20 +404,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
     const bool live = g < a.num_games;
     uint4 out_board = make_uint4(0, 0, 0, 0);
 
-    // per-step random schedule: scalar arguments, or the pre-drawn entry a CUDA graph replays
-    int64_t rand_seed = a.rand_seed;
-    uint32_t two_mask = a.two_mask;
-    uint64_t philox_counter = a.philox_counter;
-    const uint8_t *keys_table = a.randperm_keys;
-    if (a.sched) {
-        const int64_t cursor = *a.sched_cursor;
-        const ml2048_sched_entry e = a.sched[cursor];
-        rand_seed = e.rand_seed;
-        two_mask = e.two_mask;
-        philox_counter = e.philox_counter + 1ull;
-        keys_table += (int64_t)e.table * a.table_stride;
-        if (a.sched_cursor_next && blockIdx.x == 0 && threadIdx.x == 0) *a.sched_cursor_next = cursor + 1;
-    }
+    const StepDraws draws = step_draws(a, a.sched != nullptr);
 
     // fused auto-reset: which lanes of this warp hold a finished game (all non-exited lanes vote; a finished game is one
     // whose mask is all zero, game_numba.py:734-735)
@@ -358,21 +436,8 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
             const uint32_t group = (uint32_t)g >> 5;
             const int32_t order = __ldg(a.reset_chunk_base + (group >> 10)) + __ldg(a.reset_rank + group) +
                                   __popc(over_lanes & ((1u << (threadIdx.x & 31)) - 1u));
-            // the PREPARE draws of this runner step (scalar arguments, or the pre-drawn schedule entry)
-            PrepDraws d{a.rand_base, two_mask, a.prepare_philox_counter, a.randperm};
-            if (a.sched) {
-                const ml2048_sched_entry e = a.sched[*a.sched_cursor];
-                d.rand_base = e.rand_base;
-                d.philox_counter = e.philox_counter;
-                d.perm_table += (int64_t)e.table * a.table_stride;
-            }
-            bd = fresh_board<kRng, true>(d, (uint64_t)(a.slot_base + g), a.philox_seed, mask_now);
-            // prev_state / prev_valid_actions of this step are the post-reset board and mask (game_numba.py:672-673)
-            reinterpret_cast<uint4 *>(const_cast<void *>(a.board_in))[g] = bd;
-            reinterpret_cast<uint32_t *>(const_cast<void *>(a.valid_in))[g] = mask_now;
-            a.id[g] = (int32_t)*a.reset_id_base + order;
-            if (a.reset_indices && (int64_t)order < a.num_games) a.reset_indices[order] = g;
-            if (a.age) a.age[g] = 0;
+            bd = reset_in_step<kRng>(a, reset_draws(a, draws, a.sched != nullptr), g, 0, (int32_t)*a.reset_id_base, order,
+                                     a.reset_indices != nullptr, a.age != nullptr, mask_now);
             was_reset = true;
         }
     }
@@ -382,8 +447,8 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
         // one uniform word per game-step from the policy stream and (Philox mode) one from the spawn stream; a Philox2x32-10
         // block serves the two slots of a pair (board_ops.cuh: slot_word)
         u32x2 rnd = {0u, 0u};  // .x picks the spawn cell (Philox mode), .y is the policy's uniform word
-        if (kRng == ML2048_RNG_PHILOX) rnd.x = slot_word(slot, philox_counter, a.philox_seed, kSpawnStream);
-        if (a.action_mode != ML2048_ACTIONS_GIVEN) rnd.y = slot_word(slot, philox_counter, a.philox_seed, 0u);
+        if (kRng == ML2048_RNG_PHILOX) rnd.x = slot_word(slot, draws.philox_counter, a.philox_seed, kSpawnStream);
+        if (a.action_mode != ML2048_ACTIONS_GIVEN) rnd.y = slot_word(slot, draws.philox_counter, a.philox_seed, 0u);
         uint32_t action;
         const auto current_mask = [&]() -> uint32_t { return mask_now; };
         const uint32_t *sel_row;  // the move's permute selectors (board_ops.cuh)
@@ -431,23 +496,8 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
         if (moved) {
             // reward_fn (:728) and the score increment (:729-731)
             const float gain = fusion_gain(f);  // an exact integer < 2^22
-            float reward;
-            if (a.reward_kind == ML2048_REWARD_NORMAL) {
-                reward = gain;
-            } else if (a.reward_kind == ML2048_REWARD_IMPROVED) {
-                // potential shaping on cell 0, game_numba.py:455-466 (all terms are exact integers in f32: |extra| <= 2^23)
-                const uint32_t s0 = r0 & 0xffu, p0 = bd.x & 0xffu;
-                const int extra = (s0 ? (64 << s0) : 0) - (p0 ? (64 << p0) : 0);
-                reward = gain + (float)extra;
-            } else if (a.reward_kind == ML2048_REWARD_RANK) {
-                reward = (float)fusion_rank(f);
-            } else if (a.reward_kind == ML2048_REWARD_MAXCELL) {
-                const uint32_t cur = max_cell(r0, r1, r2, r3), old = max_cell(bd.x, bd.y, bd.z, bd.w);
-                reward = (float)fusion_count(f) + ((cur > old) ? (float)(1u << cur) : 0.0f);
-            } else {
-                reward = gain;
-            }
-                        // step count and score are the halves of ONE 8-byte record per game: one load, one store, one stream
+            const float reward = step_reward<false>(a.reward_kind, f, make_uint4(r0, r1, r2, r3), bd, gain);
+            // step count and score are the halves of ONE 8-byte record per game: one load, one store, one stream
             int2 *const step_score = reinterpret_cast<int2 *>(a.step) + g;
             // a game reset by this very launch starts from step 0, score 0 (its record still holds the finished game's)
             const int2 old_ss = (kReset && was_reset) ? make_int2(0, 0) : *step_score;
@@ -458,8 +508,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
             const uint32_t n0 = occupied_signs(r0), n1 = occupied_signs(r1), n2 = occupied_signs(r2), n3 = occupied_signs(r3);
             uint32_t cell;
             if (kRng == ML2048_RNG_REPLAY) {
-                const uint32_t row = (uint32_t)((uint64_t)(rand_seed + (int64_t)slot) % (uint64_t)kRandRows);
-                const uint4 keys = __ldg(reinterpret_cast<const uint4 *>(keys_table) + row);
+                const uint4 keys = __ldg(reinterpret_cast<const uint4 *>(draws.keys_table) + spawn_row(draws.rand_seed, slot));
                 // a move that changed the board leaves at least one empty cell (a slide vacates one, a fusion frees
                 // one), so the search cannot come back empty-handed here
                 cell = first_empty_key(keys.x, keys.y, keys.z, keys.w, n0, n1, n2, n3) & 15u;
@@ -469,7 +518,7 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
                 cell = kth_set_bit16(empties, umulhi32(rnd.x, ne));
             }
             // 2 or 4: tied to the CELL for the table epoch in force (game_numba.py:207), in both modes
-            const uint32_t value = 2u - ((two_mask >> cell) & 1u);
+            const uint32_t value = 2u - ((draws.two_mask >> cell) & 1u);
             if (kThreads == kSmallStepThreads) put_cell_shift(r0, r1, r2, r3, cell, value);  // latency-bound: no table load
             else put_cell(r0, r1, r2, r3, cell, value);
 
@@ -578,8 +627,9 @@ __global__ void __launch_bounds__(kThreads, kThreads == kOneHotStepThreads      
 // part of what it issues there is not game arithmetic: two instructions of address arithmetic for each of nine arrays, the
 // bounds checks, the predicates of the schedule.  A thread that owns TWO ADJACENT games computes every address once (the
 // second game sits at an immediate offset), shares the prologue, and gives the scheduler two independent instruction
-// streams.  Same arithmetic per game as step_kernel (the same board_ops.cuh functions in the same order), same draws (the words
-// of the Philox blocks of the global slot PAIR, which the thread computes once for both of its games), so every array is
+// streams.  Same arithmetic per game as step_kernel (the same board_ops.cuh functions in the same order, and the functions both
+// kernels share: step_draws, reset_draws, reset_in_step, step_reward, spawn_row), same draws (the words of the Philox blocks of
+// the global slot PAIR, which the thread computes once for both of its games), so every array is
 // bit-identical to the one-game-per-thread kernel (tests/test_pair_kernel.py); large batches of the lean configuration are
 // routed here by launch_step.
 // Measured at M = 2^24 (auto-reset fused + random policy / given actions, us per launch):
@@ -605,29 +655,6 @@ struct PairConst {
     uint32_t flags;
 };
 enum : uint32_t { kPairActionsOut = 1u, kPairStats = 2u, kPairAge = 4u, kPairResetIndices = 8u, kPairOddSlotBase = 16u, kPairSched = 32u };
-
-// What a launch draws once: the step's random schedule (scalar arguments, or the pre-drawn entry a CUDA graph replays).
-struct PairEnv {
-    int64_t rand_seed;
-    uint32_t two_mask;
-    uint64_t philox_counter;
-    const uint8_t *keys_table;
-};
-
-__device__ __forceinline__ PairEnv pair_env(const ml2048_step_args &a, const PairConst &x)
-{
-    PairEnv e{a.rand_seed, a.two_mask, a.philox_counter, a.randperm_keys};
-    if (x.flags & kPairSched) {
-        const int64_t cursor = *a.sched_cursor;
-        const ml2048_sched_entry s = a.sched[cursor];
-        e.rand_seed = s.rand_seed;
-        e.two_mask = s.two_mask;
-        e.philox_counter = s.philox_counter + 1ull;
-        e.keys_table += (int64_t)s.table * a.table_stride;
-        if (a.sched_cursor_next && blockIdx.x == 0 && threadIdx.x == 0) *a.sched_cursor_next = cursor + 1;
-    }
-    return e;
-}
 
 // What a thread reads of its two games before it can do anything: 56 bytes, three streams
 struct PairLoad {
@@ -697,13 +724,9 @@ struct GlobalTables {
 // issue slots per game (parameter load, compare, branch).
 // All 32 lanes of a warp call this together (the fused auto-reset votes); a lane past the end of the batch has live0 = false.
 template <int kRng, bool kReset, bool kRandom, bool kNormalReward, class Tables>
-__device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairConst &x, const PairEnv &env, const Tables &tab, uint32_t g0,
-                                          bool live0, bool live1, PairLoad &L)
+__device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairConst &x, const StepDraws &draws, const Tables &tab,
+                                          uint32_t g0, bool live0, bool live1, PairLoad &L)
 {
-    const int64_t rand_seed = env.rand_seed;
-    const uint32_t two_mask = env.two_mask;
-    const uint64_t philox_counter = env.philox_counter;
-
     // one address per array; the second game of the pair is the next element
     uint4 *board_out = reinterpret_cast<uint4 *>(a.board_out) + g0;
     uint32_t *valid_out = reinterpret_cast<uint32_t *>(a.valid_out) + g0;
@@ -733,7 +756,7 @@ __device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairC
         // (launched as a programmatic dependent of the scan: everything above overlapped it; from here on the kernel reads the
         // scan's results and writes the `terminated` flags the scan reads.  A no-op when not launched that way.)
         asm volatile("griddepcontrol.wait;" ::: "memory");
-        // fused auto-reset (see step_kernel): lane l holds slots 2l and 2l+1 of the warp's 64, i.e. of TWO 32-slot groups
+        // fused auto-reset (reset_in_step): lane l holds slots 2l and 2l+1 of the warp's 64, i.e. of TWO 32-slot groups
         // of the scan; ranks count the finished games of the lower lanes of the same half-warp, both games of each
         const bool over0 = live0 && mask_now[0] == 0u, over1 = live1 && mask_now[1] == 0u;
         const uint32_t lanes0 = __ballot_sync(0xffffffffu, over0), lanes1 = __ballot_sync(0xffffffffu, over1);
@@ -745,23 +768,12 @@ __device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairC
             const uint32_t group = g0 >> 5;
             int32_t order = __ldg(a.reset_chunk_base + (group >> 10)) + __ldg(a.reset_rank + group) + __popc(lanes0 & lower) +
                             __popc(lanes1 & lower);
-            PrepDraws d{a.rand_base, two_mask, a.prepare_philox_counter, a.randperm};
-            if (x.flags & kPairSched) {
-                const ml2048_sched_entry e = a.sched[*a.sched_cursor];
-                d.rand_base = e.rand_base;
-                d.philox_counter = e.philox_counter;
-                d.perm_table += (int64_t)e.table * a.table_stride;
-            }
+            const PrepDraws d = reset_draws(a, draws, x.flags & kPairSched);
             const int32_t id_base = (int32_t)*a.reset_id_base;
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
                 if (j == 0 ? over0 : over1) {
-                    bd[j] = fresh_board<kRng, true>(d, (uint64_t)(a.slot_base + g0 + j), a.philox_seed, mask_now[j]);
-                    reinterpret_cast<uint4 *>(const_cast<void *>(a.board_in))[g0 + j] = bd[j];
-                    reinterpret_cast<uint32_t *>(const_cast<void *>(a.valid_in))[g0 + j] = mask_now[j];
-                    a.id[g0 + j] = id_base + order;
-                    if ((x.flags & kPairResetIndices) && (int64_t)order < a.num_games) a.reset_indices[order] = (int64_t)g0 + j;
-                    if (x.flags & kPairAge) a.age[g0 + j] = 0;
+                    bd[j] = reset_in_step<kRng>(a, d, g0, j, id_base, order, x.flags & kPairResetIndices, x.flags & kPairAge, mask_now[j]);
                     ss[j] = make_int2(0, 0);
                     order += 1;
                 }
@@ -776,20 +788,20 @@ __device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairC
     uint32_t policy_word[2] = {0u, 0u}, spawn_word[2] = {0u, 0u};
     if (kRandom) {
         if (!(x.flags & kPairOddSlotBase)) {
-            const u32x2 b = slot_draws_keys(slot0 >> 1, philox_counter, x.policy_keys);
+            const u32x2 b = slot_draws_keys(slot0 >> 1, draws.philox_counter, x.policy_keys);
             policy_word[0] = b.x, policy_word[1] = b.y;
         } else {
-            policy_word[0] = slot_word_keys(slot0, philox_counter, x.policy_keys);
-            policy_word[1] = slot_word_keys(slot0 + 1, philox_counter, x.policy_keys);
+            policy_word[0] = slot_word_keys(slot0, draws.philox_counter, x.policy_keys);
+            policy_word[1] = slot_word_keys(slot0 + 1, draws.philox_counter, x.policy_keys);
         }
     }
     if (kRng == ML2048_RNG_PHILOX) {
         if (!(x.flags & kPairOddSlotBase)) {
-            const u32x2 b = slot_draws_keys(slot0 >> 1, philox_counter, x.spawn_keys);
+            const u32x2 b = slot_draws_keys(slot0 >> 1, draws.philox_counter, x.spawn_keys);
             spawn_word[0] = b.x, spawn_word[1] = b.y;
         } else {
-            spawn_word[0] = slot_word_keys(slot0, philox_counter, x.spawn_keys);
-            spawn_word[1] = slot_word_keys(slot0 + 1, philox_counter, x.spawn_keys);
+            spawn_word[0] = slot_word_keys(slot0, draws.philox_counter, x.spawn_keys);
+            spawn_word[1] = slot_word_keys(slot0 + 1, draws.philox_counter, x.spawn_keys);
         }
     }
 
@@ -823,34 +835,19 @@ __device__ __forceinline__ void pair_body(const ml2048_step_args &a, const PairC
                                      : (action < 4u) && (((r0 ^ bd[j].x) | (r1 ^ bd[j].y) | (r2 ^ bd[j].z) | (r3 ^ bd[j].w)) != 0u);
         if (moved) {
             const float gain = fusion_gain(f);
-            float reward;
-            if (kNormalReward || a.reward_kind == ML2048_REWARD_NORMAL) {
-                reward = gain;
-            } else if (a.reward_kind == ML2048_REWARD_IMPROVED) {
-                const uint32_t s0 = r0 & 0xffu, p0 = bd[j].x & 0xffu;
-                const int extra = (s0 ? (64 << s0) : 0) - (p0 ? (64 << p0) : 0);
-                reward = gain + (float)extra;
-            } else if (a.reward_kind == ML2048_REWARD_RANK) {
-                reward = (float)fusion_rank(f);
-            } else if (a.reward_kind == ML2048_REWARD_MAXCELL) {
-                const uint32_t cur = max_cell(r0, r1, r2, r3), old = max_cell(bd[j].x, bd[j].y, bd[j].z, bd[j].w);
-                reward = (float)fusion_count(f) + ((cur > old) ? (float)(1u << cur) : 0.0f);
-            } else {
-                reward = gain;
-            }
+            const float reward = step_reward<kNormalReward>(a.reward_kind, f, make_uint4(r0, r1, r2, r3), bd[j], gain);
             const float score = __int_as_float(ss[j].y) + gain;
             const int32_t nstep = ss[j].x + 1;
             const uint32_t n0 = occupied_signs(r0), n1 = occupied_signs(r1), n2 = occupied_signs(r2), n3 = occupied_signs(r3);
             uint32_t cell;
             if (kRng == ML2048_RNG_REPLAY) {
-                const uint32_t row = ((uint32_t)rand_seed + (uint32_t)slot) & (uint32_t)(kRandRows - 1);
-                const uint4 keys = tab.keys_row(row);
+                const uint4 keys = tab.keys_row(spawn_row(draws.rand_seed, slot));
                 cell = first_empty_key(keys.x, keys.y, keys.z, keys.w, n0, n1, n2, n3) & 15u;
             } else {
                 const uint32_t empties = empties16(~n0 & kHi, ~n1 & kHi, ~n2 & kHi, ~n3 & kHi);
                 cell = kth_set_bit16(empties, umulhi32(rnd.x, popc32(empties)));
             }
-            put_cell_entry(r0, r1, r2, r3, tab.cell_entry(cell), 2u - ((two_mask >> cell) & 1u));
+            put_cell_entry(r0, r1, r2, r3, tab.cell_entry(cell), 2u - ((draws.two_mask >> cell) & 1u));
             const uint32_t vm = valid_mask(r0, r1, r2, r3);
             const bool dead = vm == 0u;
             if (kPairStores && pair_stores) {
@@ -902,9 +899,9 @@ __global__ void __launch_bounds__(kPairThreads, ML2048_PAIR_MIN_BLOCKS) step_pai
     // latency the warp cannot hide behind its own work
     PairLoad L;
     pair_load<kReset || kRandom>(a, g0, live0, live1, L);
-    const PairEnv env = pair_env(a, x);
-    const GlobalTables tab{reinterpret_cast<const uint4 *>(env.keys_table)};
-    pair_body<kRng, kReset, kRandom, kNormalReward>(a, x, env, tab, g0, live0, live1, L);
+    const StepDraws draws = step_draws(a, x.flags & kPairSched);
+    const GlobalTables tab{reinterpret_cast<const uint4 *>(draws.keys_table)};
+    pair_body<kRng, kReset, kRandom, kNormalReward>(a, x, draws, tab, g0, live0, live1, L);
 }
 
 // A software-pipelined variant of this kernel was built and measured in round 2 and is NOT kept (profiles/pair_loop_experiments_r02.txt): a
@@ -932,57 +929,77 @@ __device__ __forceinline__ uint32_t flags16(uint4 t)  // sixteen 0/1 bytes -> 16
     return ((t.x * m) >> 28) | (((t.y * m) >> 24) & 0xf0u) | (((t.z * m) >> 20) & 0xf00u) | (((t.w * m) >> 16) & 0xf000u);
 }
 
-__device__ __forceinline__ int block_sum_256(int v, int *smem8)
+// Inclusive scan of `v` over the first kWidth lanes of a warp (all 32 lanes take part).
+template <int kWidth>
+__device__ __forceinline__ int warp_inclusive_scan(int v)
 {
+    const int lane = threadIdx.x & 31;
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0) smem8[threadIdx.x >> 5] = v;
+    for (int o = 1; o < kWidth; o <<= 1) {
+        const int n = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += n;
+    }
+    return v;
+}
+
+// Block-wide exclusive scan of `v` over a block of kThreads threads (a multiple of 32): `below` = the sum over the lower
+// threads, `total` = the sum over the block, both in every thread.  One barrier; `warp_tot` (kThreads / 32 ints of shared
+// memory) may be written again only after another one.
+struct BlockScan {
+    int below, total;
+};
+
+template <int kThreads>
+__device__ __forceinline__ BlockScan block_scan(int v, int *warp_tot)
+{
+    static_assert(kThreads % 32 == 0 && kThreads <= 1024, "a block of whole warps");
+    constexpr int kWarps = kThreads / 32;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int inc = warp_inclusive_scan<32>(v);
+    if (lane == 31) warp_tot[warp] = inc;
     __syncthreads();
-    int t = 0;
-#pragma unroll
-    for (int i = 0; i < kPrepThreads / 32; ++i) t += smem8[i];
-    return t;
+    // every warp scans the warp totals itself: no second barrier
+    const int t = lane < kWarps ? warp_tot[lane] : 0;
+    const int w = warp_inclusive_scan<kWarps>(t);
+    return BlockScan{__shfl_sync(0xffffffffu, w - t, warp) + inc - v, __shfl_sync(0xffffffffu, w, kWarps - 1)};
+}
+
+// Exclusive scan of in[0, n) into out[0, n) (`in` may be `out`) by one block of kThreads threads (the block size it is
+// launched with), in passes of kThreads entries that carry the running total from one to the next.  Returns the grand total to
+// every thread.
+template <int kThreads>
+__device__ __forceinline__ int block_scan_passes(const volatile int32_t *in, int32_t *out, int n, int *warp_tot)
+{
+    int carry = 0;
+    for (int base = 0; base < n; base += kThreads) {
+        const int i = base + threadIdx.x;
+        const BlockScan s = block_scan<kThreads>(i < n ? in[i] : 0, warp_tot);
+        if (i < n) out[i] = carry + s.below;
+        carry += s.total;
+        __syncthreads();  // warp_tot is written again by the next pass
+    }
+    return carry;
 }
 
 __global__ void __launch_bounds__(kPrepThreads) prepare_count_kernel(const uint4 *term16, int64_t n16, int32_t *tile_counts)
 {
-    __shared__ int warp_sums[kPrepThreads / 32];
+    __shared__ int warp_tot[kPrepThreads / 32];
     const int64_t i = (int64_t)blockIdx.x * kPrepThreads + threadIdx.x;
     int c = 0;
     if (i < n16) c = __popc(flags16(term16[i]));
-    const int total = block_sum_256(c, warp_sums);
+    const int total = block_scan<kPrepThreads>(c, warp_tot).total;
     if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
 }
 
+constexpr int kPrepScanThreads = 1024;  // the single block of prepare_scan_kernel
+
 // scratch layout: [0, tiles) tile counts -> exclusive offsets; then (8-byte aligned) int64 id_base
-__global__ void __launch_bounds__(1024) prepare_scan_kernel(int32_t *tile_counts, int tiles, int64_t *id_base_slot,
-                                                            int64_t *game_count, int advance, int64_t *reset_count)
+__global__ void __launch_bounds__(kPrepScanThreads) prepare_scan_kernel(int32_t *tile_counts, int tiles, int64_t *id_base_slot,
+                                                                        int64_t *game_count, int advance, int64_t *reset_count)
 {
-    __shared__ int warp_tot[32];
-    __shared__ int carry_s;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    for (int base = 0; base < tiles; base += 1024) {
-        const int i = base + threadIdx.x;
-        const int v = (i < tiles) ? tile_counts[i] : 0;
-        int inc = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int n = __shfl_up_sync(0xffffffffu, inc, o);
-            if ((threadIdx.x & 31) >= o) inc += n;
-        }
-        if ((threadIdx.x & 31) == 31) warp_tot[threadIdx.x >> 5] = inc;
-        __syncthreads();
-        int wbase = 0;
-        for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) wbase += warp_tot[w];
-        const int carry = carry_s;
-        if (i < tiles) tile_counts[i] = carry + wbase + inc - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry_s = carry + wbase + inc;
-        __syncthreads();
-    }
+    __shared__ int warp_tot[kPrepScanThreads / 32];
+    const int total = block_scan_passes<kPrepScanThreads>(tile_counts, tile_counts, tiles, warp_tot);
     if (threadIdx.x == 0) {
-        const int64_t total = carry_s;
         const int64_t base = *game_count;
         *id_base_slot = base;
         if (advance) *game_count = base + total;
@@ -1021,7 +1038,7 @@ __device__ __forceinline__ void write_onehot_of_lanes(const ml2048_prepare_args 
         const uint4 b = make_uint4(__shfl_sync(0xffffffffu, bd.x, src), __shfl_sync(0xffffffffu, bd.y, src),
                                    __shfl_sync(0xffffffffu, bd.z, src), __shfl_sync(0xffffffffu, bd.w, src));
         const long long gg = __shfl_sync(0xffffffffu, g, src);
-        write_onehot_warp_dyn(a.onehot_dtype, b, a.onehot, gg, lane);
+        with_onehot_dtype(a.onehot_dtype, [&](auto k) { write_onehot_warp<decltype(k)::value>(b, a.onehot, gg, lane); });
     }
 }
 
@@ -1035,25 +1052,11 @@ __device__ __forceinline__ int apply_tile(const ml2048_prepare_args &a, int64_t 
     const int64_t i = tile * kPrepThreads + threadIdx.x;
     uint32_t mask = 0u;
     if (i < n16) mask = flags16(reinterpret_cast<const uint4 *>(a.terminated)[i]);
-    const int mine = __popc(mask);
-    // exclusive scan of `mine` over the block
-    int inc = mine;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if ((threadIdx.x & 31) >= o) inc += n;
-    }
-    if ((threadIdx.x & 31) == 31) warp_tot[threadIdx.x >> 5] = inc;
-    __syncthreads();
-    int wbase = 0;
-    for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) wbase += warp_tot[w];
+    const BlockScan s = block_scan<kPrepThreads>(__popc(mask), warp_tot);
     const bool had_any = mask != 0u;
     const int lane = threadIdx.x & 31;
-    const PrepDraws draws = load_prep_draws(a);
-    int tile_total = 0;
-#pragma unroll
-    for (int w = 0; w < kPrepThreads / 32; ++w) tile_total += warp_tot[w];
-    int64_t order = tile_offset + wbase + inc - mine;  // rank among all reset slots
+    const PrepDraws draws = prep_draws(a, a.philox_counter, a.sched != nullptr);
+    int64_t order = tile_offset + s.below;  // rank among all reset slots
 
     // rounds: in each one every lane that still has a finished game resets one; the one-hot rows of the round
     // are then written by the whole warp, one game after the other
@@ -1072,7 +1075,7 @@ __device__ __forceinline__ int apply_tile(const ml2048_prepare_args &a, int64_t 
     }
     // every flag this thread saw is now cleared (entry.fill(0), game_numba.py:638-639)
     if (had_any) reinterpret_cast<uint4 *>(a.terminated)[i] = make_uint4(0, 0, 0, 0);
-    return tile_total;
+    return s.total;
 }
 
 template <int kRng>
@@ -1170,7 +1173,9 @@ __global__ void __launch_bounds__(kPrepThreads, 5) prepare_fused_kernel(const ml
             }
         }
     }
-    const int block_total = block_sum_256(mine, warp_tot);
+    // the block's count, and the rank of this thread's first finished game inside the block (phase 2)
+    const BlockScan in_block = block_scan<kPrepThreads>(mine, warp_tot);
+    const int block_total = in_block.total, my_first = in_block.below;
     if (threadIdx.x == 0) block_counts[blockIdx.x] = block_total;
     grid.sync();
 
@@ -1182,29 +1187,17 @@ __global__ void __launch_bounds__(kPrepThreads, 5) prepare_fused_kernel(const ml
         before += b < (int)blockIdx.x ? c : 0;
     }
     __syncthreads();
-    before = block_sum_256(before, warp_tot);
+    before = block_scan<kPrepThreads>(before, warp_tot).total;
     __syncthreads();
-    all = block_sum_256(all, warp_tot);
-    __syncthreads();
+    all = block_scan<kPrepThreads>(all, warp_tot).total;
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         *a.game_count = id_base + all;
         *a.reset_count = all;
     }
     if (block_total == 0) return;
 
-    // phase 2: rank of this thread's first finished game inside the block (exclusive scan of `mine`)
-    int inc = mine;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if ((threadIdx.x & 31) >= o) inc += n;
-    }
-    if ((threadIdx.x & 31) == 31) warp_tot[threadIdx.x >> 5] = inc;
-    __syncthreads();
-    int my_first = inc - mine;
-    for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) my_first += warp_tot[w];
-
-    const PrepDraws draws = load_prep_draws(a);
+    // phase 2: list this block's finished games in slot order and reset them
+    const PrepDraws draws = prep_draws(a, a.philox_counter, a.sched != nullptr);
     // passes of kFusedListCap games (one pass unless a large share of the block's games is over, e.g. right after reset())
     for (int window = 0; window < block_total; window += kFusedListCap) {
         const int n = block_total - window < kFusedListCap ? block_total - window : kFusedListCap;
@@ -1225,9 +1218,7 @@ __global__ void __launch_bounds__(kPrepThreads, 5) prepare_fused_kernel(const ml
             s_board[j] = reset_slot<kRng>(a, draws, s_list[j], (int64_t)before + window + j, id_base);
         if (a.onehot) {
             __syncthreads();  // the boards are parked
-            if (a.onehot_dtype == ML2048_ONEHOT_F32) write_onehot_listed<ML2048_ONEHOT_F32>(s_board, s_list, n, a.onehot);
-            else if (a.onehot_dtype == ML2048_ONEHOT_BF16) write_onehot_listed<ML2048_ONEHOT_BF16>(s_board, s_list, n, a.onehot);
-            else write_onehot_listed<ML2048_ONEHOT_U8>(s_board, s_list, n, a.onehot);
+            with_onehot_dtype(a.onehot_dtype, [&](auto k) { write_onehot_listed<decltype(k)::value>(s_board, s_list, n, a.onehot); });
         }
         __syncthreads();  // list and boards may be overwritten
     }
@@ -1247,7 +1238,6 @@ __global__ void __launch_bounds__(kScanThreads) autoreset_scan_kernel(const uint
                                                                       int64_t *reset_count, int32_t *scratch)
 {
     __shared__ int warp_tot[kScanThreads / 32];
-    __shared__ int carry_s;
     __shared__ bool last_s;
     // Programmatic dependent launch: the fused step that follows may start (load its boards, which the PREVIOUS step wrote and
     // this kernel does not touch) as soon as every block of this scan is running; it waits (griddepcontrol.wait) before it reads
@@ -1255,35 +1245,15 @@ __global__ void __launch_bounds__(kScanThreads) autoreset_scan_kernel(const uint
     asm volatile("griddepcontrol.launch_dependents;");
     const int chunks = (int)gridDim.x;
     const int64_t i = (int64_t)blockIdx.x * kScanThreads + threadIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int v = 0;
     if (i < groups) {
         v = __popc(flags16(term16[2 * i]));
         if (2 * i + 1 < n16) v += __popc(flags16(term16[2 * i + 1]));  // the padding stops at a multiple of 16 flags
     }
-    int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-    }
-    if (lane == 31) warp_tot[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {  // exclusive scan of the 32 warp totals
-        const int t = warp_tot[lane];
-        int w = t;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int n = __shfl_up_sync(0xffffffffu, w, o);
-            if (lane >= o) w += n;
-        }
-        warp_tot[lane] = w - t;
-        if (lane == 31) carry_s = w;  // chunk total
-    }
-    __syncthreads();
-    if (i < groups) reset_rank[i] = warp_tot[warp] + inc - v;
+    const BlockScan s = block_scan<kScanThreads>(v, warp_tot);
+    if (i < groups) reset_rank[i] = s.below;
     if (threadIdx.x == 0) {
-        scratch[blockIdx.x] = carry_s;
+        scratch[blockIdx.x] = s.total;
         __threadfence();
         last_s = atomicAdd(&scratch[chunks], 1) == chunks - 1;
     }
@@ -1291,30 +1261,8 @@ __global__ void __launch_bounds__(kScanThreads) autoreset_scan_kernel(const uint
     if (!last_s) return;
     // the last block: exclusive scan over the chunk totals (volatile reads: they were written by other blocks)
     __threadfence();
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    const volatile int32_t *totals = scratch;
-    for (int base = 0; base < chunks; base += kScanThreads) {
-        const int c = base + threadIdx.x;
-        const int t = c < chunks ? totals[c] : 0;
-        int w = t;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int n = __shfl_up_sync(0xffffffffu, w, o);
-            if (lane >= o) w += n;
-        }
-        if (lane == 31) warp_tot[warp] = w;
-        __syncthreads();
-        int wbase = 0;
-        for (int k = 0; k < warp; ++k) wbase += warp_tot[k];
-        const int carry = carry_s;
-        if (c < chunks) reset_chunk_base[c] = carry + wbase + w - t;
-        __syncthreads();
-        if (threadIdx.x == kScanThreads - 1) carry_s = carry + wbase + w;
-        __syncthreads();
-    }
+    const int total = block_scan_passes<kScanThreads>(scratch, reset_chunk_base, chunks, warp_tot);
     if (threadIdx.x == 0) {
-        const int64_t total = carry_s;
         const int64_t base = *game_count + (id_offset ? *id_offset : 0);
         *reset_id_base = base;
         if (!id_offset) *game_count = base + total;
@@ -1572,17 +1520,28 @@ int launch_step_onehot(const ml2048_step_args &a, cudaStream_t s)
     return launch_status();
 }
 
-// ML2048_STEP=single in the environment keeps large lean batches on the one-game-per-thread kernel (A/B measurements and the
-// differential test of the two kernels).  Read once, or on every call when ML2048_PREPARE_RECHECK is set.
-inline bool step_mode_is(const char *what)
+// A run-time switch of the environment (A/B measurements and tests): whether `on` holds for the value of variable `name`
+// (null when unset).  Read once, at first use, or on every call when ML2048_PREPARE_RECHECK was set then (the tests switch
+// modes inside one process).  Every caller passes its own lambda and so gets its own instance, with its own cached value.
+template <class On>
+bool env_switch(const char *name, On on)
 {
     static const bool recheck = getenv("ML2048_PREPARE_RECHECK") != nullptr;
-    static const char *at_start = [] { const char *m = getenv("ML2048_STEP"); return m ? strdup(m) : (const char *)nullptr; }();
-    const char *m = recheck ? getenv("ML2048_STEP") : at_start;
-    return m && strcmp(m, what) == 0;
+    static const bool at_start = on(getenv(name));
+    return recheck ? on(getenv(name)) : at_start;
 }
 
-inline bool force_single_step() { return step_mode_is("single"); }
+// ML2048_STEP=single keeps large lean batches on the one-game-per-thread kernel (the differential test of the two kernels).
+inline bool force_single_step()
+{
+    return env_switch("ML2048_STEP", [](const char *m) { return m && strcmp(m, "single") == 0; });
+}
+
+// ML2048_PREPARE=split forces the three-launch auto-reset.
+inline bool force_split_prepare()
+{
+    return env_switch("ML2048_PREPARE", [](const char *m) { return m && m[0] == 's'; });
+}
 
 template <int kRng>
 int launch_step(const ml2048_step_args &a, cudaStream_t s)
@@ -1740,8 +1699,8 @@ int ml2048_prepare_count(const ml2048_prepare_args *args, void *stream)
     clear_stale_error();
     prepare_count_kernel<<<tiles, kPrepThreads, 0, s>>>(reinterpret_cast<const uint4 *>(a.terminated), n16, a.scratch);
     if (const int rc_count = launch_status()) return rc_count;
-    prepare_scan_kernel<<<1, 1024, 0, s>>>(a.scratch, tiles, prepare_id_base_slot(a, tiles), a.game_count, a.id_offset ? 0 : 1,
-                                           a.reset_count);
+    prepare_scan_kernel<<<1, kPrepScanThreads, 0, s>>>(a.scratch, tiles, prepare_id_base_slot(a, tiles), a.game_count,
+                                                       a.id_offset ? 0 : 1, a.reset_count);
     return launch_status();
 }
 
@@ -1796,18 +1755,6 @@ static int launch_prepare_fused(const ml2048_prepare_args &a, cudaStream_t s)
         return ML2048_E_SIZE;
     }
     return e == cudaSuccess ? launch_status() : (int)e;
-}
-
-// ML2048_PREPARE=split in the environment forces the three-launch path (A/B measurements and tests).  The variable is
-// looked up on every call only when ML2048_PREPARE_RECHECK is set when the library first looks (the tests switch modes
-// inside one process); otherwise it is read once.
-static bool force_split_prepare()
-{
-    static const bool recheck = getenv("ML2048_PREPARE_RECHECK") != nullptr;
-    static const bool split_at_start = [] { const char *m = getenv("ML2048_PREPARE"); return m && m[0] == 's'; }();
-    if (!recheck) return split_at_start;
-    const char *m = getenv("ML2048_PREPARE");
-    return m && m[0] == 's';
 }
 
 int ml2048_prepare(const ml2048_prepare_args *args, void *stream)

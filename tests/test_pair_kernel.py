@@ -109,6 +109,29 @@ def test_pair_kernel_fused_rollout_against_the_oracle(ml, oracle, monkeypatch):
 
 
 @pytest.mark.parametrize("rng_mode", ["replay", "philox"])
+@pytest.mark.parametrize("fused", [False, True])
+def test_pair_kernel_graph_replay_equals_eager(ml, monkeypatch, rng_mode, fused):
+    """The in-kernel policy from the device schedule inside a CUDA graph: a step draws with the Philox counter after its
+    prepare()'s, exactly as in eager mode."""
+    monkeypatch.setenv("ML2048_STEP", "pair")
+    m, steps, replays = PAIR_MIN + 3, 8, 8
+    kw = dict(rng_mode=rng_mode, output="torch", track_merged=False, sync_free=True)
+    eager = ml.VecGame(m, "improved", **kw)
+    eager.reset(5)
+    for _ in range(steps * replays):
+        if not fused:
+            eager.prepare()
+        eager.step_random(auto_reset=fused)
+    env = ml.VecGame(m, "improved", **kw)
+    env.reset(5)
+    roll = ml.GraphedRollout(env, steps, window=steps * 3, auto_reset=fused)
+    roll.replay(replays)
+    torch.cuda.synchronize()
+    same_state(eager, env, "graph replay")
+    assert env._game_count == eager._game_count > m
+
+
+@pytest.mark.parametrize("rng_mode", ["replay", "philox"])
 def test_pair_kernel_shard_at_an_odd_slot(ml, monkeypatch, rng_mode):
     """A Philox block serves a PAIR of global slots (slot >> 1).  A shard that starts at an odd global slot has its threads'
     two games in two different blocks: its draws (policy words, Philox spawn cells) must still be those of the whole batch."""
