@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define ML2048_ABI_VERSION 10
+#define ML2048_ABI_VERSION 11
 
 #if defined(__GNUC__)
 #define ML2048_API __attribute__((visibility("default")))
@@ -286,6 +286,12 @@ ML2048_API int ml2048_encode_onehot(const void *board, void *out, int32_t onehot
 
 /* _compute_valid_actions over a batch: game_numba.py:259-289 */
 ML2048_API int ml2048_valid_actions(const void *board, void *valid_out, int64_t num_games, void *stream);
+
+/* the four moves of every board without spawning (game_numba.py:93-134, :408-504 at :728): after [n][4][16],
+ * reward [n][4] f32 (reward_kind; 0 for a direction that does not change the board), valid [n][4] u8,
+ * merged [n][4][16] or null */
+ML2048_API int ml2048_afterstates(const void *board, void *after_out, float *reward_out, uint8_t *valid_out,
+                                  uint8_t *merged_out, int32_t reward_kind, int64_t num_games, void *stream);
 
 /* _update_count (runner.py:120-136): hist[max exponent] += 1 for every game with terminated != 0;
  * with terminated == null: VecGame.summary's histogram over all live boards (game_numba.py:593-596).

@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # the full ABI like the default library
 LIB_PATH = os.environ.get("ML2048_LIB") or os.path.join(_HERE, "libml2048_b200.so")
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 STATS_REPLICAS = 64
 STATS_WORDS = 24  # 20 histogram bins + episodes, score_sum, step_sum, score_max (unsigned long long each)
 
@@ -162,6 +162,7 @@ SYMBOLS = {
     "ml2048_reset_state": (C.c_int, [_VP] * 11 + [_I64, _VP]),
     "ml2048_encode_onehot": (C.c_int, [_VP, _VP, _I32, _I64, _VP]),
     "ml2048_valid_actions": (C.c_int, [_VP, _VP, _I64, _VP]),
+    "ml2048_afterstates": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _I32, _I64, _VP]),
     "ml2048_max_tile_hist": (C.c_int, [_VP, _VP, _I64, _VP, _VP]),
     "ml2048_copy_async": (C.c_int, [_VP, _VP, _I64, _VP]),
     "ml2048_stream_wait": (C.c_int, [_VP]),

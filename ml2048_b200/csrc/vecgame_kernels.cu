@@ -1409,6 +1409,35 @@ __global__ void fill_terminated_kernel(uint8_t *terminated, int64_t num_games, i
     if (i < padded) terminated[i] = (i < num_games) ? 1 : 0;
 }
 
+// ---- afterstates ----------------------------------------------------------------------------
+// The four moves of every board without the spawn: what step(a) computes up to game_numba.py:728, for every a.  One thread per
+// (game, direction): thread t = 4 * game + direction, so the four lanes of a game read the same 16-byte board (one L1 sector)
+// and every output is indexed by t -- a warp stores 512 contiguous bytes of boards, 128 of rewards, 32 of flags, 512 of
+// `merged`.  The move, the reward and the `merged` log are the step kernel's own functions (move_board_sel with a row of
+// d_move_sel, step_reward, fusion_log).  A direction that does not change the board gets reward 0 (the step kernel leaves
+// the stale reward there instead); it fuses nothing, so its `merged` row is 0 as well.
+template <bool kLog>
+__global__ void __launch_bounds__(kStepThreads) afterstates_kernel(const uint4 *board, uint4 *after, float *reward, uint8_t *valid,
+                                                                   uint4 *merged, int32_t reward_kind, int64_t num_games)
+{
+    const int64_t t = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;  // 64-bit: 16 * t passes 2^31 at 2^25 games
+    if (t >= 4 * num_games) return;
+    const uint4 bd = board[t >> 2];
+    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    Fusions f;
+    move_board_sel(r0, r1, r2, r3, d_move_sel + (threadIdx.x & 3u) * kMoveSelRow, f);
+    const uint4 now = make_uint4(r0, r1, r2, r3);
+    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    after[t] = now;
+    reward[t] = moved ? step_reward<false>(reward_kind, f, now, bd, fusion_gain(f)) : 0.0f;
+    valid[t] = moved ? 1 : 0;
+    if (kLog) {
+        uint32_t m0, m1, m2, m3;
+        fusion_log(f, m0, m1, m2, m3);
+        merged[t] = make_uint4(m0, m1, m2, m3);
+    }
+}
+
 // ---- launch helpers -------------------------------------------------------------------------
 
 inline bool misaligned(const void *p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
@@ -1854,6 +1883,26 @@ int ml2048_valid_actions(const void *board, void *valid_out, int64_t num_games, 
     clear_stale_error();
     valid_kernel<<<grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4 *>(board),
                                                                                 reinterpret_cast<uint32_t *>(valid_out), num_games);
+    return launch_status();
+}
+
+int ml2048_afterstates(const void *board, void *after_out, float *reward_out, uint8_t *valid_out, uint8_t *merged_out, int32_t reward_kind,
+                       int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!board || !after_out || !reward_out || !valid_out) return ML2048_E_NULL;
+    if (misaligned(board, 16) || misaligned(after_out, 16) || misaligned(merged_out, 16) || misaligned(reward_out, 4)) return ML2048_E_ALIGN;
+    if (reward_kind < 0 || reward_kind > ML2048_REWARD_MAXCELL) return ML2048_E_ENUM;
+    const int64_t grid = (num_games + kStepThreads / 4 - 1) / (kStepThreads / 4);  // four threads per game
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint4 *b = reinterpret_cast<const uint4 *>(board);
+    uint4 *after = reinterpret_cast<uint4 *>(after_out), *merged = reinterpret_cast<uint4 *>(merged_out);
+    clear_stale_error();
+    if (merged)
+        afterstates_kernel<true><<<(unsigned)grid, kStepThreads, 0, s>>>(b, after, reward_out, valid_out, merged, reward_kind, num_games);
+    else
+        afterstates_kernel<false><<<(unsigned)grid, kStepThreads, 0, s>>>(b, after, reward_out, valid_out, merged, reward_kind, num_games);
     return launch_status();
 }
 

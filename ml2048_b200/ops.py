@@ -4,6 +4,8 @@
     gae_advantages              the recurrence of compute_gae, gae.py:50, :65-68
     encode_onehot               CNNEncoder.forward's input encoding, policy/_network.py:86-95
     valid_actions               _compute_valid_actions, game_numba.py:259-289
+    afterstates                 all four moves of every board up to the spawn: _step_kernel + reward_fn, game_numba.py:93-134,
+                                :408-504 at :728 (moved board, reward, "the move changes the board", optionally `merged`)
 """
 
 from __future__ import annotations
@@ -13,6 +15,7 @@ from typing import Optional
 import torch
 
 from . import _lib
+from .rewards import reward_kind
 
 _ONEHOT = {torch.float32: _lib.ONEHOT_F32, torch.bfloat16: _lib.ONEHOT_BF16, torch.uint8: _lib.ONEHOT_U8}
 
@@ -109,3 +112,60 @@ def valid_actions(board: torch.Tensor) -> torch.Tensor:
         rc = lib.ml2048_valid_actions(board.data_ptr(), out.data_ptr(), board.shape[0], _stream(board))
     _lib.check(rc, "ml2048_valid_actions")
     return out
+
+
+# afterstates() outputs: key (VecStepResult's names) -> (shape after M, dtype)
+_AFTERSTATES = {
+    "state": ((4, 16), torch.uint8),
+    "reward": ((4,), torch.float32),
+    "valid_actions": ((4,), torch.uint8),
+    "merged": ((4, 16), torch.uint8),
+}
+
+
+def afterstates(board: torch.Tensor, *, reward_fn=None, merged: bool = False, out: Optional[dict] = None) -> dict:
+    """The four moves of every board, without the spawn and without touching any environment state.
+
+    ``board``: (M,16) uint8/int8 boards.  Returns a dict of CUDA tensors, direction-major per board (0 left, 1 right,
+    2 up, 3 down):
+
+        "state"          (M,4,16) uint8    the board after the move (no tile spawned)
+        "reward"         (M,4)    float32  reward_fn of that move, bit for bit what step(a) returns; 0 where the move
+                                           does not change the board
+        "valid_actions"  (M,4)    uint8    1 iff the move changes the board (== ops.valid_actions(board))
+        "merged"         (M,4,16) uint8    only with merged=True: fusions per exponent, as step() logs them
+
+    ``reward_fn`` selects one of the four reward functions like ``VecGame(reward_fn=...)`` (default: normal).
+    ``out``: preallocated tensors under the same keys (any subset; "merged" only with merged=True), so that the call can be
+    captured in a CUDA graph.  Cells must be 0..17, as for every op here; nothing is checked on the device."""
+    if not isinstance(board, torch.Tensor) or board.dtype not in (torch.uint8, torch.int8) or board.ndim != 2 or board.shape[1] != 16:
+        raise ValueError("board must be uint8/int8 (M,16)")
+    kind = reward_kind(reward_fn)
+    keys = ("state", "reward", "valid_actions", "merged") if merged else ("state", "reward", "valid_actions")
+    out = {} if out is None else out
+    if not isinstance(out, dict):
+        raise ValueError("out must be a dict of tensors")
+    unknown = set(out) - set(keys)
+    if unknown:
+        raise ValueError(f"out has entries afterstates does not write: {sorted(unknown)}")
+    _cuda(board, "board")
+    m = board.shape[0]
+    res = {}
+    for k in keys:
+        shape, dtype = _AFTERSTATES[k]
+        shape = (m,) + shape
+        t = out.get(k)
+        if t is None:
+            t = torch.empty(shape, dtype=dtype, device=board.device)
+        elif not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == dtype and tuple(t.shape) == shape
+                  and t.device == board.device):
+            raise ValueError(f"out[{k!r}] must be a contiguous {dtype} tensor {shape} on {board.device}")
+        res[k] = t
+    if m == 0:
+        return res
+    lib = _lib.load()
+    with torch.cuda.device(board.device):
+        rc = lib.ml2048_afterstates(board.data_ptr(), res["state"].data_ptr(), res["reward"].data_ptr(), res["valid_actions"].data_ptr(),
+                                    res["merged"].data_ptr() if merged else None, kind, m, _stream(board))
+    _lib.check(rc, "ml2048_afterstates")
+    return res

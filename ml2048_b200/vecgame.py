@@ -677,6 +677,19 @@ class VecGame:
             raise RuntimeError("construct VecGame(..., onehot='f32'|'bf16'|'u8') to fuse the one-hot encoding")
         return self._onehot
 
+    def afterstates(self, *, merged: bool = False) -> dict:
+        """The four moves of every current board without the spawn (``ops.afterstates`` with this environment's
+        ``reward_fn``): "state" (M,4,16), "reward" (M,4) -- what ``step(a)`` would return, 0 where the move does not change
+        the board --, "valid_actions" (M,4) and, with ``merged=True``, "merged" (M,4,16).  CUDA tensors in torch mode, NumPy
+        arrays (fresh copies) in NumPy mode.  Changes no state: boards, counters, schedule and host generator stay as they are."""
+        from .ops import afterstates
+
+        with self._guard:
+            res = afterstates(self._board[self._cur], reward_fn=self._reward_fn, merged=merged)
+        if self._output == "numpy":
+            return {k: v.cpu().numpy() for k, v in res.items()}
+        return res
+
     def prepare(self):
         """game_numba.py:619-658: refresh tables with probability 0.1, draw an offset, reset every
         terminated slot in ascending order.  Returns ``(indices,)``."""
