@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define ML2048_ABI_VERSION 11
+#define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
 #define ML2048_API __attribute__((visibility("default")))
@@ -292,6 +292,31 @@ ML2048_API int ml2048_valid_actions(const void *board, void *valid_out, int64_t 
  * merged [n][4][16] or null */
 ML2048_API int ml2048_afterstates(const void *board, void *after_out, float *reward_out, uint8_t *valid_out,
                                   uint8_t *merged_out, int32_t reward_kind, int64_t num_games, void *stream);
+
+/* n-tuple network (no reference counterpart): K = num_tuples (1..16) tuples of len[t] (1..6) distinct cells (cell = row*4+col,
+ * 0..15) given as HOST arrays cells [K][6] (entries past len[t] ignored) and len [K].  weights: num_weights = sum_t 16^len[t]
+ * float32 entries, tuple t's table from offset sum_{u<t} 16^len[u].  V(s) = sum over t = 0..K-1 (outer), g = 0..7 (inner) of
+ * weights[offset_t + idx_t,g(s)] as float32 adds from 0.0f, where image g maps cell (r,c) to (r,c) (r,3-c) (3-r,c) (3-r,3-c)
+ * (c,r) (c,3-r) (3-c,r) (3-c,3-r) and idx = sum_j min(cell_j, 15) << 4j: any byte gives an in-bounds index, exponents >= 16
+ * share the entries of 15.  value [n] f32. */
+ML2048_API int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                   int32_t num_tuples, float *value_out, int64_t num_games, void *stream);
+
+/* greedy afterstate move: q_a = reward_a + V(afterstate_a) over the directions that change the board (reward_a and
+ * afterstate_a as ml2048_afterstates gives them); the largest q wins, NaN ranks as -inf, ties go to the smallest direction.
+ * Writes the action (u8 or i64: exactly one non-null), the chosen afterstate [n][16], its reward and its value.  A board with
+ * no valid direction: action 0, afterstate = board, reward 0, value 0. */
+ML2048_API int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                    int32_t num_tuples, int32_t reward_kind, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                                    float *reward_out, float *value_out, int64_t num_games, void *stream);
+
+/* one synchronous TD(0) batch: delta[i] = alpha * (target[i] - V(after[i])) with the weights as they were before the call
+ * (0 where mask[i] == 0; mask may be null = all games), then weights[entry] += delta[i] for every masked-in game and each of
+ * its 8 * K entries.  The adds are float atomics: their order within one entry is unspecified, so the weights are
+ * reproducible up to the fp32 rounding of that order (delta is deterministic). */
+ML2048_API int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                       int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                       float *delta_out, int64_t num_games, void *stream);
 
 /* _update_count (runner.py:120-136): hist[max exponent] += 1 for every game with terminated != 0;
  * with terminated == null: VecGame.summary's histogram over all live boards (game_numba.py:593-596).

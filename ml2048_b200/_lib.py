@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # the full ABI like the default library
 LIB_PATH = os.environ.get("ML2048_LIB") or os.path.join(_HERE, "libml2048_b200.so")
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 STATS_REPLICAS = 64
 STATS_WORDS = 24  # 20 histogram bins + episodes, score_sum, step_sum, score_max (unsigned long long each)
 
@@ -163,6 +163,9 @@ SYMBOLS = {
     "ml2048_encode_onehot": (C.c_int, [_VP, _VP, _I32, _I64, _VP]),
     "ml2048_valid_actions": (C.c_int, [_VP, _VP, _I64, _VP]),
     "ml2048_afterstates": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _I32, _I64, _VP]),
+    "ml2048_ntuple_value": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _VP, _I64, _VP]),
+    "ml2048_ntuple_greedy": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _I32, _VP, _VP, _VP, _VP, _VP, _I64, _VP]),
+    "ml2048_ntuple_td_update": (C.c_int, [_VP, _VP, _VP, C.c_float, _VP, _I64, _VP, _VP, _I32, _VP, _I64, _VP]),
     "ml2048_max_tile_hist": (C.c_int, [_VP, _VP, _I64, _VP, _VP]),
     "ml2048_copy_async": (C.c_int, [_VP, _VP, _I64, _VP]),
     "ml2048_stream_wait": (C.c_int, [_VP]),

@@ -664,4 +664,110 @@ ML2048_FN uint32_t sample_masked_categorical(float l0, float l1, float l2, float
     return action;
 }
 
+// ---- n-tuple networks -----------------------------------------------------------------------
+// K <= 16 tuples of 1..6 distinct cells; tuple t owns one float32 table of 16^len entries, all tables back to back in tuple
+// order.  A board's value sums, for every tuple and each of the board's 8 symmetric images, the table entry indexed by the
+// image's cells under the tuple: idx = sum_j min(cell_j, 15) << 4j.  Clamping makes every byte value an in-bounds index (the
+// board is never trusted to stay below 16); tiles 2^16 (exponent 16) and above share the entries of 2^15.
+constexpr int kNTupleMaxTuples = 16;
+constexpr int kNTupleMaxLen = 6;
+
+// Image g (0..7) of a board s holds in cell 4r+c the cell ntuple_sym_src(g, 4r+c) of s:
+// (r,c) (r,3-c) (3-r,c) (3-r,3-c) (c,r) (c,3-r) (3-c,r) (3-c,3-r) -- bit 2 of g transposes, bit 1 flips rows, bit 0 columns.
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+constexpr uint32_t ntuple_sym_src(uint32_t g, uint32_t cell)
+{
+    const uint32_t r = cell >> 2, c = cell & 3u;
+    const uint32_t rt = (g & 4u) ? c : r, ct = (g & 4u) ? r : c;
+    return 4u * ((g & 2u) ? 3u - rt : rt) + ((g & 1u) ? 3u - ct : ct);
+}
+
+// The network as the kernels take it, by value (a kernel parameter: two networks in one process and CUDA-graph capture need
+// no device symbol).  src4[t][g][j] = 4 * the ORIGINAL cell that image g puts under cell j of tuple t, i.e. the bit position of
+// that cell's field in ntuple_nibbles.  offset[t] < 16 * 16^6 = 2^28: 32 bits hold every entry index.
+struct NTupleSpec {
+    uint32_t num_tuples;
+    uint32_t len[kNTupleMaxTuples];
+    uint32_t offset[kNTupleMaxTuples];
+    uint8_t src4[kNTupleMaxTuples][8][8];  // rows padded to 8
+};
+
+// Host side: expand validated tuples (cells [K][6], len [K]) into the kernels' form.  Returns the total number of entries.
+inline int64_t ntuple_expand(const uint8_t *cells, const uint8_t *len, int32_t num_tuples, NTupleSpec &s)
+{
+    s = NTupleSpec{};
+    s.num_tuples = (uint32_t)num_tuples;
+    int64_t total = 0;
+    for (int t = 0; t < num_tuples; ++t) {
+        s.len[t] = len[t];
+        s.offset[t] = (uint32_t)total;
+        for (uint32_t g = 0; g < 8; ++g)
+            for (int j = 0; j < len[t]; ++j) s.src4[t][g][j] = (uint8_t)(4u * ntuple_sym_src(g, cells[kNTupleMaxLen * t + j]));
+        total += (int64_t)1 << (4 * len[t]);
+    }
+    return total;
+}
+
+// every byte of x clamped to 15
+#if defined(__CUDACC__)
+ML2048_FN uint32_t min15_bytes(uint32_t x) { return __vminu4(x, 0x0f0f0f0fu); }
+#else
+ML2048_FN uint32_t min15_bytes(uint32_t x)
+{
+    uint32_t d = 0;
+    for (int i = 0; i < 4; ++i) {
+        const uint32_t b = (x >> (8 * i)) & 0xffu;
+        d |= (b < 15u ? b : 15u) << (8 * i);
+    }
+    return d;
+}
+#endif
+
+// The board as sixteen 4-bit fields, cell k (clamped to 15) in bits 4k..4k+3
+ML2048_FN uint64_t ntuple_nibbles(uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3)
+{
+    const uint32_t w[4] = {r0, r1, r2, r3};
+    uint64_t nib = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        uint32_t x = min15_bytes(w[i]);
+        x = (x | (x >> 4)) & 0x00ff00ffu;  // bytes 0 and 2 hold two fields each
+        x = (x | (x >> 8)) & 0xffffu;
+        nib |= (uint64_t)x << (16 * i);
+    }
+    return nib;
+}
+
+// Table index of one tuple image: `src4` = its row of NTupleSpec::src4, `len` = the tuple's length
+ML2048_FN uint32_t ntuple_index(uint64_t nib, const uint8_t *src4, uint32_t len)
+{
+    uint32_t idx = 0;
+#pragma unroll
+    for (uint32_t j = 0; j < (uint32_t)kNTupleMaxLen; ++j)
+        if (j < len) idx |= (uint32_t)((nib >> src4[j]) & 15u) << (4u * j);
+    return idx;
+}
+
+#if defined(__CUDACC__)
+ML2048_FN float load_weight(const float *p) { return __ldg(p); }
+#else
+ML2048_FN float load_weight(const float *p) { return *p; }
+#endif
+
+// V(s): float32 adds from 0.0f in the fixed order t = 0..K-1, g = 0..7 -- bit-reproducible, and a sequential float32 reference
+// matches it exactly
+ML2048_FN float ntuple_value(const float *w, const NTupleSpec &s, uint64_t nib)
+{
+    float acc = 0.0f;
+    for (uint32_t t = 0; t < s.num_tuples; ++t) {
+        const float *tab = w + s.offset[t];
+        const uint32_t len = s.len[t];
+#pragma unroll
+        for (uint32_t g = 0; g < 8; ++g) acc += load_weight(tab + ntuple_index(nib, s.src4[t][g], len));
+    }
+    return acc;
+}
+
 }  // namespace ml2048

@@ -1438,6 +1438,100 @@ __global__ void __launch_bounds__(kStepThreads) afterstates_kernel(const uint4 *
     }
 }
 
+// ---- n-tuple networks -----------------------------------------------------------------------
+// Value, greedy afterstate move and TD(0) update of an n-tuple network (board_ops.cuh: NTupleSpec, ntuple_value).  The spec is
+// a by-value __grid_constant__ parameter: the kernels index it in the constant bank, nothing is copied to local memory.
+// Board offsets are 64-bit (16 * game passes 2^31 at 2^27 games); table entry indices stay below 2^28.
+
+// one thread per board
+__global__ void __launch_bounds__(kStepThreads) ntuple_value_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+                                                                    float *value, int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games) return;
+    const uint4 b = board[i];
+    value[i] = ntuple_value(w, spec, ntuple_nibbles(b.x, b.y, b.z, b.w));
+}
+
+// One thread per (board, direction), thread t = 4 * game + direction as in afterstates_kernel: the move, its reward and its
+// validity are the step kernel's own (move_board_sel, step_reward), the afterstate's value is looked up in registers and the
+// four lanes pick the move with a shuffle argmax -- no afterstate goes to memory.  q = reward + V(afterstate) for a direction
+// that changes the board; NaN ranks as -inf; the largest q wins, ties go to the smallest direction.  A board without a valid
+// direction gets action 0 and its own board, reward 0, value 0.  The lane of the chosen direction writes the outputs.
+__global__ void __launch_bounds__(kStepThreads) ntuple_greedy_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+                                                                     int32_t reward_kind, uint8_t *action_u8, long long *action_i64,
+                                                                     uint4 *after, float *reward, float *value, int64_t num_games)
+{
+    const int64_t t = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    const bool live = t < 4 * num_games;  // all four lanes of a game are live or none: the shuffles below need every lane
+    const uint32_t a = threadIdx.x & 3u;
+    const uint4 bd = live ? board[t >> 2] : make_uint4(0u, 0u, 0u, 0u);
+    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    Fusions f;
+    move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+    const uint4 now = make_uint4(r0, r1, r2, r3);
+    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    float r = 0.0f, v = 0.0f, key = -INFINITY;
+    if (moved) {
+        r = step_reward<false>(reward_kind, f, now, bd, fusion_gain(f));
+        v = ntuple_value(w, spec, ntuple_nibbles(r0, r1, r2, r3));
+        const float q = r + v;
+        key = (q == q) ? q : -INFINITY;
+    }
+    // (valid, key) descending, then direction ascending: a total order, so both butterfly steps leave every lane with the winner
+    uint32_t code = a | (moved ? 4u : 0u);
+#pragma unroll
+    for (int m = 1; m <= 2; m <<= 1) {
+        const float okey = __shfl_xor_sync(0xffffffffu, key, m);
+        const uint32_t ocode = __shfl_xor_sync(0xffffffffu, code, m);
+        const bool ovalid = (ocode & 4u) != 0u, valid = (code & 4u) != 0u;
+        if (ovalid && (!valid || okey > key || (okey == key && (ocode & 3u) < (code & 3u)))) key = okey, code = ocode;
+    }
+    const uint32_t chosen = (code & 4u) ? (code & 3u) : 0u;
+    if (!live || a != chosen) return;
+    const int64_t g = t >> 2;
+    if (action_u8) action_u8[g] = (uint8_t)a;
+    else action_i64[g] = (long long)a;
+    after[g] = now;  // == bd when no direction is valid (direction 0 then leaves the board as it is)
+    reward[g] = r;
+    value[g] = v;
+}
+
+// TD(0), phase 1: delta = alpha * (target - V(afterstate)) for every masked-in game with the weights as they were before the
+// update (phase 2 runs as a second launch); 0 for a masked-out game
+__global__ void __launch_bounds__(kStepThreads) ntuple_td_delta_kernel(const uint4 *after, const float *target, const uint8_t *mask, float alpha,
+                                                                       const float *w, __grid_constant__ const NTupleSpec spec, float *delta,
+                                                                       int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games) return;
+    float d = 0.0f;
+    if (!mask || mask[i]) {
+        const uint4 b = after[i];
+        d = alpha * (target[i] - ntuple_value(w, spec, ntuple_nibbles(b.x, b.y, b.z, b.w)));
+    }
+    delta[i] = d;
+}
+
+// TD(0), phase 2: w[entry] += delta for every masked-in game, tuple and image.  Float atomics (RED.ADD.F32): the order of the
+// adds that different games make to one entry is unspecified, so the weights are reproducible up to the fp32 rounding of
+// that order.
+__global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const uint4 *after, const uint8_t *mask, const float *delta, float *w,
+                                                                         __grid_constant__ const NTupleSpec spec, int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games || (mask && !mask[i])) return;
+    const uint4 b = after[i];
+    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
+    const float d = delta[i];
+    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
+        float *tab = w + spec.offset[k];
+        const uint32_t len = spec.len[k];
+#pragma unroll
+        for (uint32_t g = 0; g < 8; ++g) atomicAdd(tab + ntuple_index(nib, spec.src4[k][g], len), d);
+    }
+}
+
 // ---- launch helpers -------------------------------------------------------------------------
 
 inline bool misaligned(const void *p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
@@ -1457,6 +1551,24 @@ inline int launch_status()
 {
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : (int)e;
+}
+
+// Check an n-tuple network given as host arrays (cells [K][6], len [K]) and expand it into the kernels' NTupleSpec: E_NULL,
+// E_SIZE for K or a length out of range or a weight count other than sum 16^len, E_ENUM for a cell > 15 or a repeated cell
+inline int ntuple_spec(const uint8_t *cells, const uint8_t *len, int32_t num_tuples, int64_t num_weights, NTupleSpec &spec)
+{
+    if (!cells || !len) return ML2048_E_NULL;
+    if (num_tuples < 1 || num_tuples > kNTupleMaxTuples) return ML2048_E_SIZE;
+    for (int t = 0; t < num_tuples; ++t) {
+        if (len[t] < 1 || len[t] > kNTupleMaxLen) return ML2048_E_SIZE;
+        uint32_t seen = 0;
+        for (int j = 0; j < len[t]; ++j) {
+            const uint8_t c = cells[kNTupleMaxLen * t + j];
+            if (c > 15 || ((seen >> c) & 1u)) return ML2048_E_ENUM;
+            seen |= 1u << c;
+        }
+    }
+    return ntuple_expand(cells, len, num_tuples, spec) == num_weights ? 0 : ML2048_E_SIZE;
 }
 
 constexpr int kMaxDevices = 64;
@@ -1903,6 +2015,62 @@ int ml2048_afterstates(const void *board, void *after_out, float *reward_out, ui
         afterstates_kernel<true><<<(unsigned)grid, kStepThreads, 0, s>>>(b, after, reward_out, valid_out, merged, reward_kind, num_games);
     else
         afterstates_kernel<false><<<(unsigned)grid, kStepThreads, 0, s>>>(b, after, reward_out, valid_out, merged, reward_kind, num_games);
+    return launch_status();
+}
+
+int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                        int32_t num_tuples, float *value_out, int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!board || !weights || !value_out) return ML2048_E_NULL;
+    if (misaligned(board, 16) || misaligned(weights, 4) || misaligned(value_out, 4)) return ML2048_E_ALIGN;
+    NTupleSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    clear_stale_error();
+    ntuple_value_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4 *>(board), weights,
+                                                                                             spec, value_out, num_games);
+    return launch_status();
+}
+
+int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                         int32_t num_tuples, int32_t reward_kind, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                         float *reward_out, float *value_out, int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out) return ML2048_E_NULL;
+    if (misaligned(board, 16) || misaligned(weights, 4) || misaligned(action_i64, 8) || misaligned(after_out, 16) ||
+        misaligned(reward_out, 4) || misaligned(value_out, 4))
+        return ML2048_E_ALIGN;
+    if (reward_kind < 0 || reward_kind > ML2048_REWARD_MAXCELL) return ML2048_E_ENUM;
+    NTupleSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    const int64_t grid = (num_games + kStepThreads / 4 - 1) / (kStepThreads / 4);  // four threads per game
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    clear_stale_error();
+    ntuple_greedy_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        reinterpret_cast<const uint4 *>(board), weights, spec, reward_kind, action_u8, reinterpret_cast<long long *>(action_i64),
+        reinterpret_cast<uint4 *>(after_out), reward_out, value_out, num_games);
+    return launch_status();
+}
+
+int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!after || !target || !weights || !delta_out) return ML2048_E_NULL;
+    if (misaligned(after, 16) || misaligned(target, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
+    NTupleSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint4 *b = reinterpret_cast<const uint4 *>(after);
+    clear_stale_error();
+    ntuple_td_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, target, mask, alpha, weights, spec, delta_out, num_games);
+    if (const int rc = launch_status()) return rc;
+    ntuple_td_scatter_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, delta_out, weights, spec, num_games);
     return launch_status();
 }
 

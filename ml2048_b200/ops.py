@@ -6,12 +6,16 @@
     valid_actions               _compute_valid_actions, game_numba.py:259-289
     afterstates                 all four moves of every board up to the spawn: _step_kernel + reward_fn, game_numba.py:93-134,
                                 :408-504 at :728 (moved board, reward, "the move changes the board", optionally `merged`)
+    ntuple_value, ntuple_greedy, ntuple_td_update
+                                an n-tuple network's value, greedy afterstate move and TD(0) batch update (no reference
+                                counterpart; ml2048_b200.ntuple wraps them)
 """
 
 from __future__ import annotations
 
 from typing import Optional
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -169,3 +173,175 @@ def afterstates(board: torch.Tensor, *, reward_fn=None, merged: bool = False, ou
                                     res["merged"].data_ptr() if merged else None, kind, m, _stream(board))
     _lib.check(rc, "ml2048_afterstates")
     return res
+
+
+# ---- n-tuple networks ----------------------------------------------------------------------------------------------------
+
+NTUPLE_MAX_TUPLES, NTUPLE_MAX_LEN = 16, 6
+
+
+def ntuple_spec(tuples) -> tuple:
+    """Check an n-tuple network's tuples on the host and return them as a tuple of tuples of ints.
+
+    1 to 16 tuples, each 1 to 6 distinct cells in 0..15 (cell = row*4 + col).  Raises ValueError otherwise."""
+    try:
+        spec = tuple(tuple(int(c) for c in t) for t in tuples)
+    except TypeError:
+        raise ValueError("tuples must be a sequence of sequences of cells") from None
+    if not 1 <= len(spec) <= NTUPLE_MAX_TUPLES:
+        raise ValueError(f"an n-tuple network has 1..{NTUPLE_MAX_TUPLES} tuples, got {len(spec)}")
+    for t in spec:
+        if not 1 <= len(t) <= NTUPLE_MAX_LEN:
+            raise ValueError(f"a tuple has 1..{NTUPLE_MAX_LEN} cells, got {t}")
+        if any(c < 0 or c > 15 for c in t) or len(set(t)) != len(t):
+            raise ValueError(f"a tuple's cells are distinct and in 0..15, got {t}")
+    return spec
+
+
+def ntuple_num_weights(tuples) -> int:
+    """sum over the tuples of 16^len: the length of the network's one float32 weight tensor"""
+    return sum(16 ** len(t) for t in ntuple_spec(tuples))
+
+
+_SPEC_ARRAYS: dict = {}
+
+
+def _spec_arrays(tuples):
+    """(cells [K][6] u8, len [K] u8, K, number of weights) of checked tuples, cached per spec"""
+    key = tuples if isinstance(tuples, tuple) else None
+    got = _SPEC_ARRAYS.get(key) if key is not None else None
+    if got is None:
+        spec = ntuple_spec(tuples)
+        cells = np.zeros((len(spec), NTUPLE_MAX_LEN), np.uint8)
+        for i, t in enumerate(spec):
+            cells[i, :len(t)] = t
+        got = (cells, np.array([len(t) for t in spec], np.uint8), len(spec), sum(16 ** len(t) for t in spec))
+        if key is not None and len(_SPEC_ARRAYS) < 64:
+            _SPEC_ARRAYS[key] = got
+    return got
+
+
+def _weights_arg(weights: torch.Tensor, n: int, device) -> None:
+    if not (isinstance(weights, torch.Tensor) and weights.is_cuda and weights.is_contiguous() and weights.dtype == torch.float32
+            and weights.ndim == 1):
+        raise ValueError("weights must be a contiguous 1-D float32 CUDA tensor")
+    if weights.numel() != n:
+        raise ValueError(f"weights has {weights.numel()} entries, the tuples need sum 16^len = {n}")
+    if weights.device != device:
+        raise ValueError(f"weights is on {weights.device}, the boards on {device}")
+
+
+def _board_arg(board, name: str = "board") -> None:
+    if not isinstance(board, torch.Tensor) or board.dtype not in (torch.uint8, torch.int8) or board.ndim != 2 or board.shape[1] != 16:
+        raise ValueError(f"{name} must be uint8/int8 (M,16)")
+    _cuda(board, name)
+
+
+def _out_arg(t, shape: tuple, dtype, device, name: str) -> torch.Tensor:
+    if t is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == dtype and tuple(t.shape) == shape
+            and t.device == device):
+        raise ValueError(f"{name} must be a contiguous {dtype} tensor {shape} on {device}")
+    return t
+
+
+def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """V(board) of an n-tuple network: (M,16) uint8/int8 boards -> (M,) float32.
+
+    ``tuples``: the network's cells (see ``ntuple_spec``); ``weights``: its one float32 tensor of sum 16^len entries, tuple t's
+    table after those of tuples 0..t-1.  V sums, for t = 0..K-1 and then each of the board's 8 symmetric images g = 0..7,
+    ``weights[offset_t + sum_j min(image_g[cell_tj], 15) << 4j]`` as float32 adds from 0 in that order: bit-reproducible.
+    Every byte gives an in-bounds index; tiles 2^16 and above share the entries of 2^15.  ``out``: a preallocated (M,)
+    float32 tensor (CUDA-graph capture)."""
+    _board_arg(board)
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, board.device)
+    m = board.shape[0]
+    out = _out_arg(out, (m,), torch.float32, board.device, "out")
+    if m == 0:
+        return out
+    lib = _lib.load()
+    with torch.cuda.device(board.device):
+        rc = lib.ml2048_ntuple_value(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, out.data_ptr(), m,
+                                     _stream(board))
+    _lib.check(rc, "ml2048_ntuple_value")
+    return out
+
+
+_NTUPLE_GREEDY = {"state": ((16,), torch.uint8), "reward": ((), torch.float32), "value": ((), torch.float32)}
+
+
+def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
+                  out: Optional[dict] = None) -> dict:
+    """The greedy afterstate move of every board under an n-tuple network, in one kernel.
+
+    For every direction a that changes the board, q_a = reward_a + V(afterstate_a) in float32, with reward_a and afterstate_a
+    exactly ``afterstates(board, reward_fn=reward_fn)``'s.  The largest q wins; NaN ranks as -inf; ties go to the smallest a.
+    Returns a dict of CUDA tensors:
+
+        "action"  (M,)    action_dtype (int64 or uint8)
+        "state"   (M,16)  uint8    the chosen afterstate (no tile spawned)
+        "reward"  (M,)    float32  its reward
+        "value"   (M,)    float32  V(afterstate)
+
+    A board without a valid move gets action 0, its own board, reward 0 and value 0 (so a TD target reward + value is 0).
+    ``out``: preallocated tensors under the same keys (any subset), so that the call can be captured in a CUDA graph."""
+    _board_arg(board)
+    if action_dtype not in (torch.int64, torch.uint8):
+        raise ValueError("action_dtype must be torch.int64 or torch.uint8")
+    kind = reward_kind(reward_fn)
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, board.device)
+    out = {} if out is None else out
+    if not isinstance(out, dict):
+        raise ValueError("out must be a dict of tensors")
+    unknown = set(out) - {"action", *_NTUPLE_GREEDY}
+    if unknown:
+        raise ValueError(f"out has entries ntuple_greedy does not write: {sorted(unknown)}")
+    m = board.shape[0]
+    res = {"action": _out_arg(out.get("action"), (m,), action_dtype, board.device, "out['action']")}
+    for key, (shape, dtype) in _NTUPLE_GREEDY.items():
+        res[key] = _out_arg(out.get(key), (m,) + shape, dtype, board.device, f"out[{key!r}]")
+    if m == 0:
+        return res
+    act = res["action"].data_ptr()
+    lib = _lib.load()
+    with torch.cuda.device(board.device):
+        rc = lib.ml2048_ntuple_greedy(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, kind,
+                                      act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
+                                      res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), m, _stream(board))
+    _lib.check(rc, "ml2048_ntuple_greedy")
+    return res
+
+
+def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, tuples, *, alpha: float,
+                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One synchronous batch of TD(0) updates of an n-tuple network, in place on ``weights``; returns delta (M,) float32.
+
+    Phase 1: delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game
+    whose ``mask`` byte is 0 (``mask``: (M,) bool/uint8, None = every game).  Phase 2: every entry of every masked-in game,
+    8 per tuple, gets += delta_i.  Phase 2 adds with float atomics, so the order of the adds that several games make to one
+    entry is unspecified: the weights are reproducible only up to the fp32 rounding of that order.  delta is deterministic.
+    ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
+    _board_arg(afterstate, "afterstate")
+    m = afterstate.shape[0]
+    _cuda(target, "target")
+    if target.dtype != torch.float32 or tuple(target.shape) != (m,):
+        raise ValueError(f"target must be float32 ({m},)")
+    if mask is not None:
+        _cuda(mask, "mask")
+        if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,):
+            raise ValueError(f"mask must be bool/uint8 ({m},)")
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, afterstate.device)
+    delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
+    if m == 0:
+        return delta_out
+    lib = _lib.load()
+    with torch.cuda.device(afterstate.device):
+        rc = lib.ml2048_ntuple_td_update(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None,
+                                         float(alpha), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k,
+                                         delta_out.data_ptr(), m, _stream(afterstate))
+    _lib.check(rc, "ml2048_ntuple_td_update")
+    return delta_out
