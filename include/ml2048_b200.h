@@ -9,7 +9,8 @@
  *
  * Conventions
  *   - plain pointers and sizes only; every pointer is a DEVICE pointer unless named host_*;
- *   - the library never allocates, frees or retains memory;  all work is enqueued on `stream`
+ *   - the library never allocates, frees or retains memory (except ml2048_alloc_compressible / ml2048_free_compressible,
+ *     which do nothing else);  all work is enqueued on `stream`
  *     (a cudaStream_t passed as void*) and the call returns immediately: no hidden synchronisation,
  *     CUDA-graph capturable;
  *   - return value: 0 = ok, negative = argument error (ML2048_E_*), positive = cudaError_t of the launch;
@@ -27,6 +28,8 @@
 extern "C" {
 #endif
 
+/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, added without a bump (unlike earlier additions):
+ * they change no existing struct or signature, and a loader that binds them by name fails on a library without them. */
 #define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
@@ -41,6 +44,7 @@ extern "C" {
 #define ML2048_E_SIZE (-3)    /* num_games <= 0 or capacity too small */
 #define ML2048_E_ENUM (-4)    /* bad enum value */
 #define ML2048_E_STRUCT (-5)  /* struct_size does not match this library */
+#define ML2048_E_UNSUPPORTED (-6) /* no CUDA driver or device, or the device lacks the feature */
 
 /* reward_fn, selected by identity on the Python side (game_numba.py:408-504) */
 enum { ML2048_REWARD_NORMAL = 0, ML2048_REWARD_IMPROVED = 1, ML2048_REWARD_RANK = 2, ML2048_REWARD_MAXCELL = 3 };
@@ -372,6 +376,30 @@ ML2048_API uint32_t ml2048_two_threshold(double two_prob);
  * for host callers without a CUDA binding of their own: 0 or a cudaError_t. */
 ML2048_API int ml2048_copy_async(void *dst, const void *src, int64_t bytes, void *stream);
 ML2048_API int ml2048_stream_wait(void *stream);
+
+/* ---- compressible device memory (the only entry points that allocate) ------------------------------------------------
+ * A mostly-zero output written in full every step (the one-hot observation) costs fewer HBM bytes in memory the L2 may
+ * store compressed.  ml2048_alloc_compressible reserves a virtual range of `bytes` rounded up to the allocation granularity
+ * on `device`, backs it with cuMemCreate(allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC) allocations, maps
+ * them and grants read/write access to that device only.  If one allocation is not granted compression, the range is
+ * built again from 8, then 64 equal allocations, each checked on its own; `granted` counts the bytes the driver granted
+ * compression (read back, possibly 0).  The contents are undefined.  Returns 0, ML2048_E_NULL / ML2048_E_SIZE,
+ * ML2048_E_UNSUPPORTED (no driver, no such device, or no generic compression on it; *out is then all zero), or a
+ * positive CUresult of the driver call that failed (nothing stays allocated).
+ * ml2048_free_compressible synchronises the device (work queued on any stream may still write the range), unmaps,
+ * releases and unreserves it, and zeroes *c; a zeroed *c is a no-op. */
+#define ML2048_COMPRESSIBLE_MAX_CHUNKS 64
+typedef struct {
+    uint64_t ptr;      /* device address of the range, 0 when nothing is mapped */
+    uint64_t size;     /* mapped bytes: the request rounded up to the granularity (per allocation) */
+    uint64_t granted;  /* bytes of the range whose allocation the driver granted generic compression */
+    int32_t device;
+    int32_t chunks;    /* equal allocations behind the range */
+    uint64_t handles[ML2048_COMPRESSIBLE_MAX_CHUNKS];
+} ml2048_compressible;
+
+ML2048_API int ml2048_alloc_compressible(int32_t device, int64_t bytes, ml2048_compressible *out);
+ML2048_API int ml2048_free_compressible(ml2048_compressible *c);
 
 /* Philox mode, the host half of one prepare(): the reference refreshes its spawn tables when `random() >= 0.9`
  * (game_numba.py:622-624) and the 2-vs-4 choice then stays tied to the CELL until the next refresh (:207).  The same two

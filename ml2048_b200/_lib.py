@@ -24,7 +24,10 @@ ACT_U8, ACT_I32, ACT_I64 = 0, 1, 2
 ACTIONS_GIVEN, ACTIONS_RANDOM_VALID, ACTIONS_FROM_LOGITS = 0, 1, 2
 ONEHOT_NONE, ONEHOT_F32, ONEHOT_BF16, ONEHOT_U8 = 0, 1, 2, 3
 
-ERRORS = {-1: "null pointer", -2: "misaligned pointer", -3: "bad size", -4: "bad enum", -5: "struct size mismatch"}
+ERRORS = {-1: "null pointer", -2: "misaligned pointer", -3: "bad size", -4: "bad enum", -5: "struct size mismatch",
+          -6: "unsupported (no CUDA driver or device, or no such feature on it)"}
+E_UNSUPPORTED = -6
+COMPRESSIBLE_MAX_CHUNKS = 64
 
 
 class StepArgs(C.Structure):
@@ -135,6 +138,19 @@ class PrepareArgs(C.Structure):
     ]
 
 
+class Compressible(C.Structure):
+    """ml2048_compressible"""
+
+    _fields_ = [
+        ("ptr", C.c_uint64),
+        ("size", C.c_uint64),
+        ("granted", C.c_uint64),
+        ("device", C.c_int32),
+        ("chunks", C.c_int32),
+        ("handles", C.c_uint64 * COMPRESSIBLE_MAX_CHUNKS),
+    ]
+
+
 class Pcg64(C.Structure):
     """ml2048_pcg64"""
 
@@ -169,6 +185,8 @@ SYMBOLS = {
     "ml2048_max_tile_hist": (C.c_int, [_VP, _VP, _I64, _VP, _VP]),
     "ml2048_copy_async": (C.c_int, [_VP, _VP, _I64, _VP]),
     "ml2048_stream_wait": (C.c_int, [_VP]),
+    "ml2048_alloc_compressible": (C.c_int, [_I32, _I64, C.POINTER(Compressible)]),
+    "ml2048_free_compressible": (C.c_int, [C.POINTER(Compressible)]),
     "ml2048_pack_flags": (C.c_int, [_VP, _VP, _VP, _VP, _I64, _VP]),
     "ml2048_unpack_flags": (None, [_VP, _I64, _VP, _VP, _VP, _I32]),
     "ml2048_unpack_flags_sliced": (C.c_int, [_VP, _I32, _VP, _VP, _VP, _VP, _VP, _VP, _I32]),

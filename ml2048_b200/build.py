@@ -10,7 +10,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(_HERE, "csrc", "vecgame_kernels.cu")
 HOST_SRC = os.path.join(_HERE, "csrc", "host_pcg64.cpp")
 HOST_UNPACK_SRC = os.path.join(_HERE, "csrc", "host_unpack.cpp")
-DEPS = [SRC, HOST_SRC, HOST_UNPACK_SRC, os.path.join(_HERE, "csrc", "board_ops.cuh"), os.path.join(os.path.dirname(_HERE), "include", "ml2048_b200.h")]
+COMPRESSIBLE_SRC = os.path.join(_HERE, "csrc", "compressible_alloc.cpp")
+DEPS = [SRC, HOST_SRC, HOST_UNPACK_SRC, COMPRESSIBLE_SRC, os.path.join(_HERE, "csrc", "board_ops.cuh"), os.path.join(os.path.dirname(_HERE), "include", "ml2048_b200.h")]
 LIB = os.path.join(_HERE, "libml2048_b200.so")
 
 NVCC_FLAGS = [
@@ -36,7 +37,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and up_to_date() and not os.environ.get("ML2048_NVCC_EXTRA"):
         return LIB
     extra = os.environ.get("ML2048_NVCC_EXTRA", "").split()  # experiment switches, e.g. -DML2048_STORE_DEFAULT
-    cmd = [nvcc_path(), *NVCC_FLAGS, *extra, "-o", LIB, SRC, HOST_SRC, HOST_UNPACK_SRC]
+    cmd = [nvcc_path(), *NVCC_FLAGS, *extra, "-o", LIB, SRC, HOST_SRC, HOST_UNPACK_SRC, COMPRESSIBLE_SRC]
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")

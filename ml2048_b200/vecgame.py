@@ -58,6 +58,76 @@ _ONEHOT = {
     "u8": (_lib.ONEHOT_U8, torch.uint8),
 }
 
+
+_CUDA_ERROR_OUT_OF_MEMORY = 2
+_PENDING_FREES: list = []  # ranges released while this thread was capturing a CUDA graph, freed by the next _onehot_buffer()
+
+
+class _CompressibleBlock:
+    """Owns one ml2048_alloc_compressible range; tensors made from it (torch.as_tensor keeps a reference to this object)
+    hold it alive, and the range goes back to the driver when the last of them is gone.
+
+    The free synchronises the device, which a CUDA-graph capture forbids: a block released while the current stream is
+    capturing is freed by the next _onehot_buffer() call instead.  A capture in global mode on ANOTHER thread cannot be
+    seen from here; releasing a block then invalidates that capture (and the failed free is reported as a
+    ResourceWarning), so do not drop the last reference to an environment's one-hot while another thread captures."""
+
+    def __init__(self, lib: C.CDLL, device: int, nbytes: int):
+        # bound here, not looked up in __del__: module globals may already be gone when it runs at interpreter exit
+        self._free, self._capturing, self._warn = lib.ml2048_free_compressible, torch.cuda.is_current_stream_capturing, _free_or_warn
+        self._c = _lib.Compressible()
+        rc = lib.ml2048_alloc_compressible(device, nbytes, C.byref(self._c))
+        if rc == _CUDA_ERROR_OUT_OF_MEMORY:  # memory torch's allocator caches but does not use is not free for the driver
+            torch.cuda.empty_cache()
+            rc = lib.ml2048_alloc_compressible(device, nbytes, C.byref(self._c))
+        # out of memory even so: the caller falls back to torch, whose allocator raises its own error if it cannot do better
+        self.ok = rc == 0
+        if rc not in (0, _lib.E_UNSUPPORTED, _CUDA_ERROR_OUT_OF_MEMORY):
+            _lib.check(rc, "ml2048_alloc_compressible")
+        self.granted = int(self._c.granted)
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (int(self._c.ptr), False), "version": 3}
+
+    def __del__(self):
+        c = getattr(self, "_c", None)
+        if c is None or not c.ptr:
+            return
+        if self._capturing():
+            _PENDING_FREES.append(c)
+        else:
+            self._warn(self._free, c)
+
+
+def _free_or_warn(free: Any, c: Any) -> None:
+    size = int(c.size)
+    rc = free(c)
+    if rc != 0:
+        import warnings
+
+        warnings.warn(f"ml2048_free_compressible failed with {rc}: {size} bytes of device memory stay allocated", ResourceWarning)
+
+
+def _onehot_buffer(lib: C.CDLL, m: int, dtype: torch.dtype, dev: torch.device) -> tuple[torch.Tensor, bool]:
+    """The zeroed (m, 16, 16) one-hot observation and whether its memory is compressible.
+
+    The one-hot is 15/16 zeros and the step kernel rewrites all of it every step: in memory allocated with generic
+    compression the L2 writes such lines to HBM compressed, and at M = 2^24 the fused fp32 step takes 2.16 instead of
+    2.78 ms on a B200 (profiles/README.md).  A one-hot that fits in the L2 is not written to HBM every step, so there is
+    nothing to gain, and at M = 2048 the 16-step graph with the fused auto-reset took 8.23 instead of 7.61 us per step
+    in compressible memory: only a one-hot larger than the L2 is allocated there.  The values are the same either way.
+    Plain torch memory also where the device has no generic compression, the driver grants none, the driver is out of
+    memory, or ML2048_ONEHOT_COMPRESSIBLE=0."""
+    while _PENDING_FREES:
+        _free_or_warn(lib.ml2048_free_compressible, _PENDING_FREES.pop())
+    nbytes = m * 256 * torch.empty((), dtype=dtype).element_size()
+    if os.environ.get("ML2048_ONEHOT_COMPRESSIBLE", "1") != "0" and nbytes > torch.cuda.get_device_properties(dev).L2_cache_size:
+        block = _CompressibleBlock(lib, dev.index, nbytes)
+        if block.ok and block.granted > 0:
+            t = torch.as_tensor(block, device=dev)[:nbytes].view(dtype).view(m, 16, 16)
+            return t.zero_(), True
+        del block
+    return torch.zeros((m, 16, 16), dtype=dtype, device=dev), False
+
+
 # the reference's record layout (game_numba.py:537-551), used by the `_data` compatibility view
 DATA_DTYPE = np.dtype(
     [
@@ -307,7 +377,8 @@ class VecGame:
             self._score = self._step_score[:, 1].view(torch.float32)
             if not track_merged:
                 self._merged = None
-            self._onehot = torch.zeros((m, 16, 16), dtype=onehot_dtype, device=dev) if onehot_dtype is not None else None
+            self._onehot, self._onehot_compressed = (_onehot_buffer(self._lib, m, onehot_dtype, dev) if onehot_dtype is not None
+                                                     else (None, False))
             self._actions_out = torch.zeros((m,), dtype=torch.uint8, device=dev)
             # table ring: slot s holds [0] the reference's randperm table and [1] the same table in inverse
             # ("rank key") form.  Eager calls use one slot; a pre-drawn device schedule uses one slot per refresh.
@@ -676,6 +747,11 @@ class VecGame:
         if self._onehot is None:
             raise RuntimeError("construct VecGame(..., onehot='f32'|'bf16'|'u8') to fuse the one-hot encoding")
         return self._onehot
+
+    @property
+    def onehot_compressed(self) -> bool:
+        """Whether the one-hot observation lives in memory the driver granted generic (L2) compression."""
+        return self._onehot_compressed
 
     def afterstates(self, *, merged: bool = False) -> dict:
         """The four moves of every current board without the spawn (``ops.afterstates`` with this environment's
