@@ -28,8 +28,9 @@
 extern "C" {
 #endif
 
-/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, added without a bump (unlike earlier additions):
- * they change no existing struct or signature, and a loader that binds them by name fails on a library without them. */
+/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible and ml2048_expectimax, added without a bump (unlike
+ * earlier additions): they change no existing struct or signature, and a loader that binds them by name fails on a library
+ * without them. */
 #define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
@@ -321,6 +322,23 @@ ML2048_API int ml2048_ntuple_greedy(const void *board, const float *weights, int
 ML2048_API int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
                                        int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
                                        float *delta_out, int64_t num_games, void *stream);
+
+/* expectimax move over an n-tuple network (network arguments as ml2048_ntuple_value), depth 1 or 2 chance layers.  With
+ * after/r/valid as ml2048_afterstates gives them, V the network's value, p2 = (float)two_prob, p4 = 1.0f - p2, and every
+ * operation one float32 operation (no contraction):
+ *   E(s,d) = (t_c1 + t_c2 + ... + t_cn) / n over the empty cells c1 < ... < cn of afterstate s, added in that order from the
+ *            first term, t_c = p2 * M(s + 2 at c, d) + p4 * M(s + 4 at c, d); an outcome of probability 0 is not evaluated;
+ *   M(b,d) = max over valid a of key(r(b,a) + (d == 1 ? V(after(b,a)) : E(after(b,a), d-1))), key(NaN) = -inf, the smallest
+ *            direction's key among equal keys; 0 for a board with no valid move;
+ *   q_a    = r(b,a) + E(after(b,a), depth) for a valid a, -inf otherwise; the action is the argmax of q (NaN as -inf, ties to
+ *            the smallest direction), value = E of its afterstate.
+ * Writes the action (u8 or i64: exactly one non-null), the chosen afterstate [n][16], its reward and value, and q [n][4].  A
+ * board with no valid direction: action 0, afterstate = board, reward 0, value 0, q all -inf.  Cells must be 0..17.
+ * E_ENUM also for depth outside {1, 2} and two_prob outside [0, 1] or NaN. */
+ML2048_API int ml2048_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                 int32_t num_tuples, int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8,
+                                 int64_t *action_i64, void *after_out, float *reward_out, float *value_out, float *q_out, int64_t num_games,
+                                 void *stream);
 
 /* _update_count (runner.py:120-136): hist[max exponent] += 1 for every game with terminated != 0;
  * with terminated == null: VecGame.summary's histogram over all live boards (game_numba.py:593-596).

@@ -1532,6 +1532,268 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const u
     }
 }
 
+// ---- expectimax over an n-tuple network -----------------------------------------------------
+// Definition (tests/_expectimax_ref.py is the same in NumPy; every operation is one float32 operation rounded on its own, so
+// the sums and products below are __fadd_rn / __fmul_rn / __fdiv_rn and nvcc cannot contract them into FMAs).  after(b,a),
+// r(b,a), valid(b,a) are afterstates_kernel's (the step kernel's move_board_sel and step_reward); V is ntuple_value;
+// p2 = float32(two_prob), p4 = 1.0f - p2, both rounded on the host.
+//   E(s, d), s an afterstate (>= 1 empty cell: a move that changed the board leaves one), d >= 1 chance layers left:
+//       for every empty cell c of s in ascending order, t_c = p2 * M(s + tile 2 at c, d) + p4 * M(s + tile 4 at c, d); an
+//       outcome of probability 0 is not evaluated (t_c = p2 * m2 when p4 == 0, p4 * m4 when p2 == 0);
+//       S = t_c1 + t_c2 + ... added in that order from the first term (not from 0.0f: signed zeros survive); E = S / n.
+//   M(b, d) = max over the valid a of key(r(b,a) + (d == 1 ? V(after(b,a)) : E(after(b,a), d - 1))), key(NaN) = -inf; among
+//       equal keys the smallest direction's key is taken (ntuple_greedy's tie rule); 0 for a board without a valid move.
+//   Root, depth D in {1, 2}: q_a = r(b,a) + E(after(b,a), D) for a valid a, -inf otherwise; the action is ntuple_greedy's
+//       argmax of q (NaN as -inf, ties to the smallest direction); value = E(after(b,a*), D).  A board without a valid move:
+//       action 0, its own board, reward 0, value 0, q all -inf.
+// The spawn model is VecGame's marginal law: a uniform empty cell, a 2 with probability two_prob.  (VecGame ties 2-vs-4 to
+// the cell for a table epoch; the search does not model that tie.)  No intermediate board leaves the registers.
+
+// ntuple_greedy_kernel's 4-lane argmax (kept inline there: as a call it compiles to different SASS): lanes 4i..4i+3 hold
+// direction code & 3, bit 2 of code = valid.  (valid, key) descending, then direction ascending is a total order, so both
+// butterfly steps leave every lane of the group with the winner's key and code.
+__device__ __forceinline__ void lane4_argmax(float &key, uint32_t &code)
+{
+#pragma unroll
+    for (int m = 1; m <= 2; m <<= 1) {
+        const float okey = __shfl_xor_sync(0xffffffffu, key, m);
+        const uint32_t ocode = __shfl_xor_sync(0xffffffffu, code, m);
+        const bool ovalid = (ocode & 4u) != 0u, valid = (code & 4u) != 0u;
+        if (ovalid && (!valid || okey > key || (okey == key && (ocode & 3u) < (code & 3u)))) key = okey, code = ocode;
+    }
+}
+
+// 16-bit mask of the empty cells of a board
+__device__ __forceinline__ uint32_t empty_cells(uint4 s)
+{
+    return empties16(~occupied_signs(s.x) & kHi, ~occupied_signs(s.y) & kHi, ~occupied_signs(s.z) & kHi, ~occupied_signs(s.w) & kHi);
+}
+
+// The spawn outcomes of a chance node in evaluation order: outcome o is the (o / per_cell)-th empty cell with tile
+// exponent 1 + (o & 1) when both tiles have a non-zero probability (per_cell = 2), else the one tile that has.
+struct SpawnLaw {
+    float p2, p4;
+    __device__ __forceinline__ uint32_t per_cell() const { return (p2 > 0.0f && p4 > 0.0f) ? 2u : 1u; }
+    __device__ __forceinline__ uint32_t tile(uint32_t o) const { return per_cell() == 2u ? 1u + (o & 1u) : (p2 > 0.0f ? 1u : 2u); }
+};
+
+// E(s, 1) of an afterstate s that the whole warp holds (warp-uniform call; n >= 1 empty cells).  A pass covers 8 outcomes x
+// 4 inner directions: lane = 4 * outcome + direction, the move, reward and value in registers, M by lane4_argmax.  Every
+// lane then reads the pass's 8 M values by shuffle and adds the terms in ascending cell order, so all lanes return E.
+__device__ __forceinline__ float chance1(uint4 s, const float *w, const NTupleSpec &spec, int32_t reward_kind, SpawnLaw law)
+{
+    const uint32_t lane = threadIdx.x & 31u, a = lane & 3u;
+    const uint32_t empties = empty_cells(s), n = popc32(empties);
+    const uint32_t per_cell = law.per_cell(), outcomes = n * per_cell;
+    const float p_one = law.p2 > 0.0f ? law.p2 : law.p4;
+    float sum = 0.0f;
+    for (uint32_t base = 0; base < outcomes; base += 8u) {
+        const uint32_t o = base + (lane >> 2);
+        const bool live = o < outcomes;
+        uint32_t r0 = s.x, r1 = s.y, r2 = s.z, r3 = s.w;
+        put_cell_shift(r0, r1, r2, r3, kth_set_bit16(empties, live ? o / per_cell : 0u), law.tile(o));
+        const uint4 sp = make_uint4(r0, r1, r2, r3);
+        Fusions f;
+        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+        const bool moved = live && ((r0 ^ sp.x) | (r1 ^ sp.y) | (r2 ^ sp.z) | (r3 ^ sp.w)) != 0u;
+        float key = -INFINITY;
+        if (moved) {
+            const float q = step_reward<false>(reward_kind, f, make_uint4(r0, r1, r2, r3), sp, fusion_gain(f)) +
+                            ntuple_value(w, spec, ntuple_nibbles(r0, r1, r2, r3));
+            key = (q == q) ? q : -INFINITY;
+        }
+        uint32_t code = a | (moved ? 4u : 0u);
+        lane4_argmax(key, code);
+        const float m = (code & 4u) ? key : 0.0f;  // M: 0 for a spawned board without a valid move
+        if (per_cell == 2u) {
+#pragma unroll
+            for (uint32_t j = 0; j < 4u; ++j) {
+                const float m2 = __shfl_sync(0xffffffffu, m, 8u * j), m4 = __shfl_sync(0xffffffffu, m, 8u * j + 4u);
+                const float t = __fadd_rn(__fmul_rn(law.p2, m2), __fmul_rn(law.p4, m4));
+                if (base + 2u * j < outcomes) sum = (base == 0u && j == 0u) ? t : __fadd_rn(sum, t);
+            }
+        } else {
+#pragma unroll
+            for (uint32_t j = 0; j < 8u; ++j) {
+                const float t = __fmul_rn(p_one, __shfl_sync(0xffffffffu, m, 4u * j));
+                if (base + j < outcomes) sum = (base == 0u && j == 0u) ? t : __fadd_rn(sum, t);
+            }
+        }
+    }
+    return __fdiv_rn(sum, (float)n);
+}
+
+// The root of lanes 4i..4i+3 (direction = lane & 3) of a board: q = r + e for a valid direction, lane4_argmax over q, the
+// group's lanes write q, the chosen lane the rest.  `e` = E(after(bd, lane & 3), D) (ignored where that move is invalid);
+// `store` is false for groups that hold no board.
+__device__ __forceinline__ void expectimax_root(uint4 bd, float e, bool store, int64_t g, int32_t reward_kind, uint8_t *action_u8,
+                                                long long *action_i64, uint4 *after, float *reward, float *value, float *q_out)
+{
+    const uint32_t a = threadIdx.x & 3u;
+    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    Fusions f;
+    move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+    const uint4 now = make_uint4(r0, r1, r2, r3);
+    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    float r = 0.0f, q = -INFINITY, key = -INFINITY;
+    if (moved) {
+        r = step_reward<false>(reward_kind, f, now, bd, fusion_gain(f));
+        q = __fadd_rn(r, e);
+        key = (q == q) ? q : -INFINITY;
+    }
+    uint32_t code = a | (moved ? 4u : 0u);
+    lane4_argmax(key, code);
+    if (!store) return;
+    q_out[4 * g + a] = q;
+    const uint32_t chosen = (code & 4u) ? (code & 3u) : 0u;
+    if (a != chosen) return;
+    if (action_u8) action_u8[g] = (uint8_t)a;
+    else action_i64[g] = (long long)a;
+    after[g] = now;  // == bd when no direction is valid
+    reward[g] = r;
+    value[g] = moved ? e : 0.0f;
+}
+
+constexpr int kExpectimaxThreads = 256;
+
+#if !defined(ML2048_EXPECTIMAX_WARP_PER_BOARD)
+constexpr int kExpectimax1BoardsPerBlock = kExpectimaxThreads / 128;
+
+// Depth 1, one warp per (board, root direction): warp w of a block takes board 2 * block + w / 4, direction w & 3, and
+// computes E(after, 1) with chance1; lanes 0..7 of warp 0 then pick both boards' moves from shared memory.
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+                                                                         int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
+                                                                         long long *action_i64, uint4 *after, float *reward,
+                                                                         float *value, float *q_out, int64_t num_games)
+{
+    __shared__ float sh_e[kExpectimaxThreads / 32];
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+    const int64_t g = (int64_t)blockIdx.x * kExpectimax1BoardsPerBlock + (warp >> 2);
+    const bool live = g < num_games;
+    const uint4 bd = live ? board[g] : make_uint4(0u, 0u, 0u, 0u);
+    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    Fusions f;
+    move_board_sel(r0, r1, r2, r3, d_move_sel + (warp & 3u) * kMoveSelRow, f);
+    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    float e = 0.0f;
+    if (moved) e = chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law);  // warp-uniform
+    if (lane == 0u) sh_e[warp] = e;
+    __syncthreads();
+    if (warp != 0u) return;
+    const uint32_t slot = lane >> 2;  // the block's boards are slots 0 and 1; the other groups shuffle along
+    const int64_t gs = (int64_t)blockIdx.x * kExpectimax1BoardsPerBlock + slot;
+    const bool store = slot < (uint32_t)kExpectimax1BoardsPerBlock && gs < num_games;
+    expectimax_root(store ? board[gs] : make_uint4(0u, 0u, 0u, 0u), store ? sh_e[lane] : 0.0f, store, gs, reward_kind, action_u8,
+                    action_i64, after, reward, value, q_out);
+}
+#else
+constexpr int kExpectimax1BoardsPerBlock = kExpectimaxThreads / 32;
+
+// Depth 1, one warp per board (the alternative mapping; profiles/expectimax_bench.txt): the warp computes E(after(b,a), 1)
+// for a = 0..3 in turn, lane group 0 picks the move.  No shared memory, no barrier.
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+                                                                         int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
+                                                                         long long *action_i64, uint4 *after, float *reward,
+                                                                         float *value, float *q_out, int64_t num_games)
+{
+    const int64_t g = (int64_t)blockIdx.x * kExpectimax1BoardsPerBlock + (threadIdx.x >> 5);
+    if (g >= num_games) return;  // warp-uniform
+    const uint4 bd = board[g];
+    float mine = 0.0f;
+    for (uint32_t a = 0; a < 4u; ++a) {
+        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        Fusions f;
+        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+        if (((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) == 0u) continue;
+        const float e = chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law);
+        if ((threadIdx.x & 3u) == a) mine = e;
+    }
+    expectimax_root(bd, mine, (threadIdx.x & 31u) < 4u, g, reward_kind, action_u8, action_i64, after, reward, value, q_out);
+}
+#endif
+
+// Depth 2, one block per board.  Its depth-1 chance nodes after(s', a') -- s' = after(b, a) + one spawn outcome o, a' an inner
+// direction -- are numbered root direction-major, then outcome, then a' (at most 4 * 30 * 4 = 480); warp w evaluates nodes
+// w, w + 8, ... with chance1 and stores key(r(s',a') + E(after(s',a'), 1)) and validity in shared memory.  Lane group 0 of warp
+// 0 then folds them, in the definition's fixed order, into M, t_c, S and E for each root direction and picks the move.
+constexpr int kExpectimax2Nodes = 4 * 2 * 15 * 4;
+
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax2_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+                                                                         int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
+                                                                         long long *action_i64, uint4 *after, float *reward,
+                                                                         float *value, float *q_out)
+{
+    __shared__ float sh_key[kExpectimax2Nodes];
+    __shared__ uint8_t sh_ok[kExpectimax2Nodes];
+    const int64_t g = blockIdx.x;
+    const uint4 bd = board[g];
+    const uint32_t per_cell = law.per_cell();
+    uint32_t count[4];  // nodes under root direction a: 4 * outcomes of after(b, a), 0 for an invalid a
+#pragma unroll
+    for (uint32_t a = 0; a < 4u; ++a) {
+        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        Fusions f;
+        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+        const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+        count[a] = moved ? 4u * per_cell * popc32(empty_cells(make_uint4(r0, r1, r2, r3))) : 0u;
+    }
+    const uint32_t total = count[0] + count[1] + count[2] + count[3];
+    for (uint32_t j = threadIdx.x >> 5; j < total; j += kExpectimaxThreads / 32) {
+        uint32_t a = 0u, rem = j;
+#pragma unroll
+        for (uint32_t i = 0; i < 3u; ++i)
+            if (a == i && rem >= count[i]) rem -= count[i], a = i + 1u;
+        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        Fusions f;
+        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+        const uint32_t o = rem >> 2, inner = rem & 3u;
+        put_cell_shift(r0, r1, r2, r3, kth_set_bit16(empty_cells(make_uint4(r0, r1, r2, r3)), o / per_cell), law.tile(o));
+        const uint4 sp = make_uint4(r0, r1, r2, r3);
+        move_board_sel(r0, r1, r2, r3, d_move_sel + inner * kMoveSelRow, f);
+        const bool moved = ((r0 ^ sp.x) | (r1 ^ sp.y) | (r2 ^ sp.z) | (r3 ^ sp.w)) != 0u;
+        float key = -INFINITY;
+        if (moved) {  // warp-uniform
+            const float rr = step_reward<false>(reward_kind, f, make_uint4(r0, r1, r2, r3), sp, fusion_gain(f));
+            const float q = __fadd_rn(rr, chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law));
+            key = (q == q) ? q : -INFINITY;
+        }
+        if ((threadIdx.x & 31u) == 0u) sh_key[j] = key, sh_ok[j] = moved ? 1 : 0;
+    }
+    __syncthreads();
+    if (threadIdx.x >= 32u) return;
+    // every lane group folds the nodes of its direction a = lane & 3 (groups 1..7 repeat group 0's work and store nothing)
+    const uint32_t a = threadIdx.x & 3u;
+    uint32_t start = 0u, nodes = 0u;
+#pragma unroll
+    for (uint32_t i = 0; i < 4u; ++i) {
+        if (i < a) start += count[i];
+        if (i == a) nodes = count[i];
+    }
+    float sum = 0.0f;
+    for (uint32_t c = 0; c < nodes; c += 4u * per_cell) {  // one empty cell of after(b, a) per iteration, ascending
+        float m[2];
+#pragma unroll
+        for (uint32_t t = 0; t < 2u; ++t) {
+            const uint32_t base = start + c + 4u * t;
+            float best = 0.0f;
+            bool any = false;
+            if (t < per_cell) {
+#pragma unroll
+                for (uint32_t i = 0; i < 4u; ++i) {
+                    const float k = sh_key[base + i];
+                    if (sh_ok[base + i] && (!any || k > best)) best = k, any = true;
+                }
+            }
+            m[t] = best;  // 0 for a spawned board without a valid move
+        }
+        const float term = per_cell == 2u ? __fadd_rn(__fmul_rn(law.p2, m[0]), __fmul_rn(law.p4, m[1]))
+                                          : __fmul_rn(law.p2 > 0.0f ? law.p2 : law.p4, m[0]);
+        sum = c == 0u ? term : __fadd_rn(sum, term);
+    }
+    const float e = nodes ? __fdiv_rn(sum, (float)(nodes / (4u * per_cell))) : 0.0f;
+    expectimax_root(bd, e, threadIdx.x < 4u, g, reward_kind, action_u8, action_i64, after, reward, value, q_out);
+}
+
 // ---- launch helpers -------------------------------------------------------------------------
 
 inline bool misaligned(const void *p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
@@ -2052,6 +2314,39 @@ int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_we
     ntuple_greedy_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(
         reinterpret_cast<const uint4 *>(board), weights, spec, reward_kind, action_u8, reinterpret_cast<long long *>(action_i64),
         reinterpret_cast<uint4 *>(after_out), reward_out, value_out, num_games);
+    return launch_status();
+}
+
+int ml2048_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                      int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                      float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out || !q_out) return ML2048_E_NULL;
+    if (misaligned(board, 16) || misaligned(weights, 4) || misaligned(action_i64, 8) || misaligned(after_out, 16) ||
+        misaligned(reward_out, 4) || misaligned(value_out, 4) || misaligned(q_out, 4))
+        return ML2048_E_ALIGN;
+    if (reward_kind < 0 || reward_kind > ML2048_REWARD_MAXCELL || (depth != 1 && depth != 2) || !(two_prob >= 0.0 && two_prob <= 1.0))
+        return ML2048_E_ENUM;
+    NTupleSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    SpawnLaw law;
+    law.p2 = (float)two_prob;
+    law.p4 = 1.0f - law.p2;
+    const int64_t per_block = depth == 1 ? kExpectimax1BoardsPerBlock : 1;
+    const int64_t grid = (num_games + per_block - 1) / per_block;
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    const uint4 *b = reinterpret_cast<const uint4 *>(board);
+    long long *a64 = reinterpret_cast<long long *>(action_i64);
+    uint4 *after = reinterpret_cast<uint4 *>(after_out);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    clear_stale_error();
+    if (depth == 1)
+        expectimax1_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, spec, reward_kind, law, action_u8, a64, after, reward_out,
+                                                                         value_out, q_out, num_games);
+    else
+        expectimax2_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, spec, reward_kind, law, action_u8, a64, after, reward_out,
+                                                                         value_out, q_out);
     return launch_status();
 }
 

@@ -68,6 +68,13 @@ class NTupleNetwork:
         """The move maximising reward + V(afterstate): {"action", "state", "reward", "value"} (``ops.ntuple_greedy``)."""
         return ops.ntuple_greedy(board, self.weights, self.tuples, reward_fn=reward_fn, action_dtype=action_dtype, out=out)
 
+    def expectimax(self, board: torch.Tensor, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
+                   action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None) -> dict:
+        """The expectimax move ``depth`` (1 or 2) chance layers deep: {"action", "state", "reward", "value", "q"}
+        (``ops.ntuple_expectimax``)."""
+        return ops.ntuple_expectimax(board, self.weights, self.tuples, depth=depth, two_prob=two_prob, reward_fn=reward_fn,
+                                     action_dtype=action_dtype, out=out)
+
     def td_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
                   delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One synchronous TD(0) batch toward ``target``; returns delta = alpha * (target - V) (``ops.ntuple_td_update``).
@@ -97,6 +104,25 @@ class GreedyPolicy:
     def sample_actions(self, state: torch.Tensor, valid_actions: torch.Tensor):
         board = state.to(self.net.device, torch.uint8).contiguous()  # exponents fit a byte
         actions = self.net.greedy(board, reward_fn=self.reward_fn)["action"]
+        return actions, torch.zeros(actions.shape, dtype=torch.float32, device=actions.device)
+
+
+class ExpectimaxPolicy:
+    """The network's expectimax move (``NTupleNetwork.expectimax``) as a policy ``DeviceRunner`` accepts:
+    ``sample_actions(state, valid_actions)`` returns (actions int64, log_probs 0).  ``reward_fn`` and ``two_prob`` must be the
+    environment's: the search scores moves with that reward and averages over spawns with that chance of a 2."""
+
+    def __init__(self, net: NTupleNetwork, depth: int = 1, reward_fn=None, two_prob: float = 0.8):
+        if isinstance(depth, bool) or depth not in (1, 2):
+            raise ValueError(f"depth must be 1 or 2, got {depth!r}")
+        self.net = net
+        self.depth = depth
+        self.reward_fn = reward_fn
+        self.two_prob = two_prob
+
+    def sample_actions(self, state: torch.Tensor, valid_actions: torch.Tensor):
+        board = state.to(self.net.device, torch.uint8).contiguous()  # exponents fit a byte
+        actions = self.net.expectimax(board, depth=self.depth, two_prob=self.two_prob, reward_fn=self.reward_fn)["action"]
         return actions, torch.zeros(actions.shape, dtype=torch.float32, device=actions.device)
 
 

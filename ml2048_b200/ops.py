@@ -9,6 +9,7 @@
     ntuple_value, ntuple_greedy, ntuple_td_update
                                 an n-tuple network's value, greedy afterstate move and TD(0) batch update (no reference
                                 counterpart; ml2048_b200.ntuple wraps them)
+    ntuple_expectimax           the expectimax move over such a network, one or two chance layers deep
 """
 
 from __future__ import annotations
@@ -312,6 +313,73 @@ def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_
                                       act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
                                       res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), m, _stream(board))
     _lib.check(rc, "ml2048_ntuple_greedy")
+    return res
+
+
+_NTUPLE_EXPECTIMAX = dict(_NTUPLE_GREEDY, q=((4,), torch.float32))
+
+
+def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
+                      action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None) -> dict:
+    """The expectimax move of every board under an n-tuple network, ``depth`` (1 or 2) chance layers deep, in one kernel.
+
+    Definition (every operation one float32 operation; after, r, valid as ``afterstates(board, reward_fn=reward_fn)`` gives
+    them, V = ``ntuple_value``, p2 = float32(two_prob), p4 = 1 - p2 in float32):
+
+        E(s, d)  chance node of afterstate s: for each empty cell c of s in ascending order
+                 t_c = p2 * M(s + tile 2 at c, d) + p4 * M(s + tile 4 at c, d)  (an outcome of probability 0 is left out);
+                 E = (t_c1 + t_c2 + ...) / n, added in that order starting from the first term
+        M(b, d)  max over valid a of key(r(b,a) + (V(after(b,a)) if d == 1 else E(after(b,a), d - 1))), key(NaN) = -inf,
+                 the smallest direction's key among equal keys; 0 for a board without a valid move
+        q_a      r(b,a) + E(after(b,a), depth) for a valid a, -inf otherwise
+
+    The action is the argmax of q with ``ntuple_greedy``'s rule (NaN ranks as -inf, ties go to the smallest direction).
+    Depth 1 is "2-ply" expectimax in the literature.  The spawn model is VecGame's marginal law: a uniform empty cell, a 2
+    with probability ``two_prob``.  VecGame ties 2-vs-4 to the cell within a table epoch; the search deliberately does not
+    model that tie.  Returns a dict of CUDA tensors:
+
+        "action"  (M,)    action_dtype (int64 or uint8)
+        "state"   (M,16)  uint8    the chosen afterstate (no tile spawned)
+        "reward"  (M,)    float32  its reward
+        "value"   (M,)    float32  E(afterstate, depth)
+        "q"       (M,4)   float32  q of every direction
+
+    A board without a valid move gets action 0, its own board, reward 0, value 0 and q all -inf.  ``out``: preallocated
+    tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.  Cells must be 0..17."""
+    _board_arg(board)
+    if action_dtype not in (torch.int64, torch.uint8):
+        raise ValueError("action_dtype must be torch.int64 or torch.uint8")
+    if isinstance(depth, bool) or depth not in (1, 2):
+        raise ValueError(f"depth must be 1 or 2, got {depth!r}")
+    try:
+        p = float(two_prob)
+    except (TypeError, ValueError):
+        raise ValueError(f"two_prob must be a number in [0, 1], got {two_prob!r}") from None
+    if not 0.0 <= p <= 1.0:
+        raise ValueError(f"two_prob must be in [0, 1], got {two_prob!r}")
+    kind = reward_kind(reward_fn)
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, board.device)
+    out = {} if out is None else out
+    if not isinstance(out, dict):
+        raise ValueError("out must be a dict of tensors")
+    unknown = set(out) - {"action", *_NTUPLE_EXPECTIMAX}
+    if unknown:
+        raise ValueError(f"out has entries ntuple_expectimax does not write: {sorted(unknown)}")
+    m = board.shape[0]
+    res = {"action": _out_arg(out.get("action"), (m,), action_dtype, board.device, "out['action']")}
+    for key, (shape, dtype) in _NTUPLE_EXPECTIMAX.items():
+        res[key] = _out_arg(out.get(key), (m,) + shape, dtype, board.device, f"out[{key!r}]")
+    if m == 0:
+        return res
+    act = res["action"].data_ptr()
+    lib = _lib.load()
+    with torch.cuda.device(board.device):
+        rc = lib.ml2048_expectimax(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, kind, int(depth), p,
+                                   act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
+                                   res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), res["q"].data_ptr(), m,
+                                   _stream(board))
+    _lib.check(rc, "ml2048_expectimax")
     return res
 
 
