@@ -28,9 +28,9 @@
 extern "C" {
 #endif
 
-/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible and ml2048_expectimax, added without a bump (unlike
- * earlier additions): they change no existing struct or signature, and a loader that binds them by name fails on a library
- * without them. */
+/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, ml2048_expectimax and ml2048_tc_update, added without
+ * a bump (unlike earlier additions): they change no existing struct or signature, and a loader that binds them by name fails
+ * on a library without them. */
 #define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
@@ -322,6 +322,23 @@ ML2048_API int ml2048_ntuple_greedy(const void *board, const float *weights, int
 ML2048_API int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
                                        int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
                                        float *delta_out, int64_t num_games, void *stream);
+
+/* one synchronous temporal coherence (TC) batch (Jaskowski 2018): every weight gets its own step size beta_j = |E_j| / A_j,
+ * E_j the running sum of the errors applied to entry j and A_j that of their absolute values.  coherence [N][2] = {E, A} per
+ * weight, float32, 8-byte aligned; accum [N][2] float32 scratch, 8-byte aligned, all zero on entry and left all zero.
+ * Network arguments as ml2048_ntuple_value.  Every operation is one float32 operation (no contraction):
+ *   1. delta[i] = alpha * (target[i] - V(after[i])) with the weights before the call, 0 where mask[i] == 0 (mask may be
+ *      null = all games): ml2048_ntuple_td_update's delta bit for bit;
+ *   2. for every masked-in game and each of its 8 * K entries j (twice if the game hits j twice): dE_j += delta[i],
+ *      dA_j += |delta[i]| (float atomics: order within one entry unspecified, subnormals flushed);
+ *   3. for every entry with dA_j != 0 (NaN counts as non-zero), with E_j, A_j as they were before the call:
+ *      beta_j = (A_j == 0) ? 1 : |E_j| / A_j;  w_j += beta_j * dE_j;  E_j += dE_j;  A_j += dA_j.
+ *      Entries with dA_j == 0 stay as they are, bit for bit.
+ * E and A sum alpha-scaled errors: with a constant alpha beta equals the unscaled rule's; a changing alpha weights older
+ * errors by the alpha they had.  The cost is O(num_games): no pass over the table. */
+ML2048_API int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                float *coherence, float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                int32_t num_tuples, float *delta_out, int64_t num_games, void *stream);
 
 /* expectimax move over an n-tuple network (network arguments as ml2048_ntuple_value), depth 1 or 2 chance layers.  With
  * after/r/valid as ml2048_afterstates gives them, V the network's value, p2 = (float)two_prob, p4 = 1.0f - p2, and every

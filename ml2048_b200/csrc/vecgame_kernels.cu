@@ -1532,6 +1532,74 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const u
     }
 }
 
+// ---- temporal coherence (TC) learning ---------------------------------------------------------
+// Definition (ml2048_tc_update in the header, ops.ntuple_tc_update and tests/_tc_ref.py say the same; every operation is one
+// float32 operation, __fmul_rn / __fadd_rn / __fdiv_rn, no contraction).  C[j] = {E_j, A_j}: the running sum of the errors
+// applied to entry j and of their absolute values.  One synchronous batch:
+//   1. delta_i = alpha * (target_i - V(after_i)) with the weights before the call, 0 for a masked-out game (phase 1 is
+//      ntuple_td_delta_kernel: TD(0)'s delta bit for bit);
+//   2. for every masked-in game and each of its 8K entries j (twice if the game hits j twice): dE_j += delta_i,
+//      dA_j += |delta_i| (float atomics: order within one entry unspecified, subnormals flushed);
+//   3. for every entry with dA_j != 0 (NaN counts as non-zero), with E_j, A_j as they were before the call:
+//      beta_j = (A_j == 0) ? 1 : |E_j| / A_j;  w_j += beta_j * dE_j;  E_j += dE_j;  A_j += dA_j.
+//      Entries with dA_j == 0 stay as they are, bit for bit.
+// E and A sum alpha-scaled errors: with a constant alpha beta is the unscaled rule's, a changing alpha weights older errors
+// by the alpha they had.  The accumulator acc[j] = {dE_j, dA_j} belongs to the caller and is all zero bits on entry and on
+// return.  Cost O(batch): phase 3 walks the batch's own entries, never the table.
+
+// TC, phase 2: one 8-byte vector atomic (RED.E.ADD.F32x2) per lookup into the interleaved {dE, dA} accumulator
+__global__ void __launch_bounds__(kStepThreads) ntuple_tc_accumulate_kernel(const uint4 *after, const uint8_t *mask, const float *delta,
+                                                                            float2 *acc, __grid_constant__ const NTupleSpec spec,
+                                                                            int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games || (mask && !mask[i])) return;
+    const uint4 b = after[i];
+    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
+    const float d = delta[i];
+    const float2 e = make_float2(d, fabsf(d));
+    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
+        float2 *tab = acc + spec.offset[k];
+        const uint32_t len = spec.len[k];
+#pragma unroll
+        for (uint32_t g = 0; g < 8; ++g) atomicAdd(tab + ntuple_index(nib, spec.src4[k][g], len), e);
+    }
+}
+
+// TC, phase 3: one thread per masked-in game walks its own entries and claims each with a 64-bit exchange against 0; only
+// the thread that receives dA != 0 applies the entry, with plain loads and stores (no other thread touches w[j] or C[j] in
+// this launch).  So every accumulated entry is applied exactly once and the accumulator is zero again afterwards.  A plain
+// L2 load first skips the exchange where the word is already zero (an entry claimed by an earlier game: early-game entries are
+// shared by thousands of games): the word only goes from non-zero to zero during this launch, so a zero read is final and a
+// stale non-zero read costs one exchange that returns 0.  The whole word is tested, not only dA, so that a -0 left in dE is
+// still cleared.  -DML2048_TC_APPLY_ALWAYS_EXCHANGE builds the variant without the load (tools/tc_bench.py times both).
+__global__ void __launch_bounds__(kStepThreads) ntuple_tc_apply_kernel(const uint4 *after, const uint8_t *mask, float *w, float2 *coh,
+                                                                       unsigned long long *acc, __grid_constant__ const NTupleSpec spec,
+                                                                       int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games || (mask && !mask[i])) return;
+    const uint4 b = after[i];
+    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
+    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
+        const uint32_t off = spec.offset[k], len = spec.len[k];
+#pragma unroll
+        for (uint32_t g = 0; g < 8; ++g) {
+            const uint32_t j = off + ntuple_index(nib, spec.src4[k][g], len);
+#if !defined(ML2048_TC_APPLY_ALWAYS_EXCHANGE)
+            if (__ldcg(acc + j) == 0ull) continue;
+#endif
+            const unsigned long long word = atomicExch(acc + j, 0ull);
+            const float dE = __uint_as_float((uint32_t)word), dA = __uint_as_float((uint32_t)(word >> 32));
+            if (dA == 0.0f) continue;  // NaN goes on
+            const float2 c = coh[j];
+            const float beta = c.y == 0.0f ? 1.0f : __fdiv_rn(fabsf(c.x), c.y);
+            w[j] = __fadd_rn(w[j], __fmul_rn(beta, dE));
+            coh[j] = make_float2(__fadd_rn(c.x, dE), __fadd_rn(c.y, dA));
+        }
+    }
+}
+
 // ---- expectimax over an n-tuple network -----------------------------------------------------
 // Definition (tests/_expectimax_ref.py is the same in NumPy; every operation is one float32 operation rounded on its own, so
 // the sums and products below are __fadd_rn / __fmul_rn / __fdiv_rn and nvcc cannot contract them into FMAs).  after(b,a),
@@ -2366,6 +2434,32 @@ int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_
     ntuple_td_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, target, mask, alpha, weights, spec, delta_out, num_games);
     if (const int rc = launch_status()) return rc;
     ntuple_td_scatter_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, delta_out, weights, spec, num_games);
+    return launch_status();
+}
+
+int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                     float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
+                     int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!after || !target || !weights || !coherence || !accum || !delta_out) return ML2048_E_NULL;
+    if (misaligned(after, 16) || misaligned(target, 4) || misaligned(weights, 4) || misaligned(coherence, 8) || misaligned(accum, 8) ||
+        misaligned(delta_out, 4))
+        return ML2048_E_ALIGN;
+    NTupleSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint4 *b = reinterpret_cast<const uint4 *>(after);
+    clear_stale_error();
+    ntuple_td_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, target, mask, alpha, weights, spec, delta_out, num_games);
+    if (const int rc = launch_status()) return rc;
+    ntuple_tc_accumulate_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, delta_out, reinterpret_cast<float2 *>(accum), spec,
+                                                                        num_games);
+    if (const int rc = launch_status()) return rc;
+    ntuple_tc_apply_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, weights, reinterpret_cast<float2 *>(coherence),
+                                                                   reinterpret_cast<unsigned long long *>(accum), spec, num_games);
     return launch_status();
 }
 

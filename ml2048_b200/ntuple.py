@@ -3,7 +3,8 @@
 An n-tuple network (Szubert & Jaskowski 2014; Yeh et al. 2016) values a 2048 board as a sum of table entries indexed by the
 4-bit fields of a few cells, over the board's 8 symmetric images (one table per tuple, shared by the images).  Evaluating it,
 choosing the greedy afterstate move with it and updating it are integer byte work on boards plus scattered 4-byte reads and
-adds: each is one kernel here (``ops.ntuple_value``, ``ops.ntuple_greedy``, ``ops.ntuple_td_update``).
+adds: each is one kernel here (``ops.ntuple_value``, ``ops.ntuple_greedy``, ``ops.ntuple_td_update``; temporal coherence
+learning, a step size per weight, is ``ops.ntuple_tc_update`` and ``TDAfterstateLearner(..., rule="tc")``).
 
     net = NTupleNetwork(device="cuda")                        # the standard 4x6 network, zero weights (256 MiB)
     env = VecGame(16384, output="torch", sync_free=True)
@@ -38,6 +39,18 @@ def default_alpha(num_games: int) -> float:
     return DEFAULT_ALPHA_TIMES_GAMES / num_games
 
 
+# Step size of TDAfterstateLearner(rule="tc"): alpha = DEFAULT_TC_ALPHA_TIMES_GAMES / M, for the same reason as above (the
+# batch sums the steps of all M games on shared entries).  tools/tc_bench.py swept c = 0.1 ... 6.4 at M = 4096, 2^14 and 2^16,
+# 30 000 steps each (profiles/tc_bench.txt, B200): again the results depend on c alone (mean score 10.1k / 11.7-11.8k /
+# 13.9-14.0k / 16.3-16.4k / 8.5-9.0k / 4.3-4.9k / 4.0-4.9k for c = 0.1 / 0.2 / 0.4 / 0.8 / 1.6 / 3.2 / 6.4 at all three
+# sizes), and c = 0.8, twice TD(0)'s best, is the best of them.
+DEFAULT_TC_ALPHA_TIMES_GAMES = 0.8
+
+
+def default_tc_alpha(num_games: int) -> float:
+    return DEFAULT_TC_ALPHA_TIMES_GAMES / num_games
+
+
 class NTupleNetwork:
     """An n-tuple value function with its weights on one CUDA device.
 
@@ -58,6 +71,8 @@ class NTupleNetwork:
             self.offsets.append(total)
             total += 16 ** len(t)
         self.weights = torch.zeros((total,), dtype=torch.float32, device=dev)
+        self.coherence: Optional[torch.Tensor] = None  # TC learning's {E, A} per weight, allocated by the first tc_update
+        self._tc_accum: Optional[torch.Tensor] = None  # tc_update's scratch, all zero between calls
 
     def value(self, board: torch.Tensor, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """V of (M,16) boards: (M,) float32 (``ops.ntuple_value``)."""
@@ -81,16 +96,43 @@ class NTupleNetwork:
         The adds are float atomics: the weights are reproducible up to the fp32 rounding of their order."""
         return ops.ntuple_td_update(afterstate, target, self.weights, self.tuples, alpha=alpha, mask=mask, delta_out=delta_out)
 
+    def tc_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
+                  delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One synchronous temporal coherence batch toward ``target``; returns delta = alpha * (target - V)
+        (``ops.ntuple_tc_update``).  The first call allocates ``coherence`` ((N, 2) float32 {E, A} per weight, zeros) and a
+        zero scratch accumulator of the same shape."""
+        if self.coherence is None:
+            self.coherence = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
+        if self._tc_accum is None:
+            self._tc_accum = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
+        return ops.ntuple_tc_update(afterstate, target, self.weights, self.coherence, self._tc_accum, self.tuples, alpha=alpha,
+                                    mask=mask, delta_out=delta_out)
+
     def state_dict(self) -> dict:
-        return {"tuples": [list(t) for t in self.tuples], "weights": self.weights.detach().clone()}
+        state = {"tuples": [list(t) for t in self.tuples], "weights": self.weights.detach().clone()}
+        if self.coherence is not None:
+            state["coherence"] = self.coherence.detach().clone()
+        return state
 
     def load_state_dict(self, state: dict) -> None:
+        """Loads the weights and, when ``state`` has them, the TC coherence sums; a dict without ``"coherence"`` drops any
+        coherence state this network has (the next ``tc_update`` starts from zeros)."""
         if ops.ntuple_spec(state["tuples"]) != self.tuples:
             raise ValueError(f"state_dict is for tuples {state['tuples']}, this network has {self.tuples}")
         w = state["weights"]
         if not isinstance(w, torch.Tensor) or w.dtype != torch.float32 or tuple(w.shape) != tuple(self.weights.shape):
             raise ValueError(f"weights must be float32 {tuple(self.weights.shape)}")
+        c = state.get("coherence")
+        shape = (self.weights.numel(), 2)
+        if c is not None and (not isinstance(c, torch.Tensor) or c.dtype != torch.float32 or tuple(c.shape) != shape):
+            raise ValueError(f"coherence must be float32 {shape}")
         self.weights.copy_(w)
+        if c is None:
+            self.coherence = None
+        elif self.coherence is None:
+            self.coherence = c.detach().to(self.device, copy=True).contiguous()
+        else:
+            self.coherence.copy_(c)
 
 
 class GreedyPolicy:
@@ -133,21 +175,30 @@ class TDAfterstateLearner:
 
     1. ``env.prepare()`` (games that ended in the previous step restart);
     2. greedy afterstate move on the boards (``NTupleNetwork.greedy``);
-    3. TD(0) update of each game's previous afterstate toward reward + value of the move just chosen, or toward 0 for a
-       game that ended in the previous step; games without a previous afterstate (the first step after ``reset()``) are
-       masked out;
+    3. TD(0) (or, with ``rule="tc"``, TC) update of each game's previous afterstate toward reward + value of the move just
+       chosen, or toward 0 for a game that ended in the previous step; games without a previous afterstate (the first step
+       after ``reset()``) are masked out;
     4. ``env.step(action)``.
 
     ``alpha`` defaults to ``default_alpha(M)``.  With ``alpha=0`` step 3 is skipped and the learner plays the greedy policy
-    (evaluation).  Call ``reset(seed)`` instead of ``env.reset`` so that no afterstate of the old games is updated."""
+    (evaluation).  Call ``reset(seed)`` instead of ``env.reset`` so that no afterstate of the old games is updated.
 
-    def __init__(self, env, net: NTupleNetwork, alpha: Optional[float] = None):
+    ``rule``: ``"td0"`` (the default) updates with ``NTupleNetwork.td_update``; ``"tc"`` with temporal coherence learning
+    (``NTupleNetwork.tc_update``: a step size per weight), whose ``alpha`` defaults to ``default_tc_alpha(M)``."""
+
+    def __init__(self, env, net: NTupleNetwork, alpha: Optional[float] = None, rule: str = "td0"):
         if env._output != "torch" or not env._sync_free:
             raise ValueError("TDAfterstateLearner needs VecGame(..., output='torch', sync_free=True)")
         if env.device != net.device:
             raise ValueError(f"the environment is on {env.device}, the network on {net.device}")
-        self.env, self.net = env, net
-        self.alpha = default_alpha(env._size) if alpha is None else float(alpha)
+        if rule not in ("td0", "tc"):
+            raise ValueError(f"rule must be 'td0' or 'tc', got {rule!r}")
+        self.env, self.net, self.rule = env, net, rule
+        if alpha is not None:
+            self.alpha = float(alpha)
+        else:
+            self.alpha = default_tc_alpha(env._size) if rule == "tc" else default_alpha(env._size)
+        self._update = net.tc_update if rule == "tc" else net.td_update
         m, dev = env._size, env.device
         self._out = {"action": torch.zeros((m,), dtype=torch.uint8, device=dev),
                      "state": torch.zeros((m, 16), dtype=torch.uint8, device=dev),
@@ -171,7 +222,7 @@ class TDAfterstateLearner:
         if self.alpha != 0.0:
             torch.add(g["reward"], g["value"], out=self._target)
             self._target.masked_fill_(self._prev_ended, 0.0)
-            self.net.td_update(self._prev_after, self._target, self.alpha, mask=self._has_prev, delta_out=self.delta)
+            self._update(self._prev_after, self._target, self.alpha, mask=self._has_prev, delta_out=self.delta)
         res = env.step(g["action"])
         self._prev_after.copy_(g["state"])
         self._prev_ended.copy_(res["terminated"])

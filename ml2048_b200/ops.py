@@ -10,6 +10,7 @@
                                 an n-tuple network's value, greedy afterstate move and TD(0) batch update (no reference
                                 counterpart; ml2048_b200.ntuple wraps them)
     ntuple_expectimax           the expectimax move over such a network, one or two chance layers deep
+    ntuple_tc_update            a temporal coherence batch update of such a network: per-weight step sizes
 """
 
 from __future__ import annotations
@@ -412,4 +413,52 @@ def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
                                          float(alpha), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k,
                                          delta_out.data_ptr(), m, _stream(afterstate))
     _lib.check(rc, "ml2048_ntuple_td_update")
+    return delta_out
+
+
+def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, coherence: torch.Tensor,
+                     accum: torch.Tensor, tuples, *, alpha: float, mask: Optional[torch.Tensor] = None,
+                     delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One synchronous batch of temporal coherence (TC) updates of an n-tuple network, in place on ``weights`` and
+    ``coherence``; returns delta (M,) float32.
+
+    Every weight has its own step size beta_j = |E_j| / A_j, with ``coherence[j] = (E_j, A_j)`` the running sum of the errors
+    applied to entry j and of their absolute values (Jaskowski 2018).  Every operation is one float32 operation:
+
+    1. delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game whose
+       ``mask`` byte is 0 (``mask``: (M,) bool/uint8, None = every game) -- ``ntuple_td_update``'s delta bit for bit;
+    2. for every masked-in game and each of its 8K entries j (twice if the game hits j twice): dE_j += delta_i,
+       dA_j += |delta_i|, float atomics into ``accum`` (order within one entry unspecified, subnormals flushed);
+    3. for every entry with dA_j != 0 (NaN counts as non-zero), with E_j and A_j as they were before the call:
+       beta_j = 1 if A_j == 0 else |E_j| / A_j;  w_j += beta_j * dE_j;  E_j += dE_j;  A_j += dA_j.
+       Entries with dA_j == 0 stay as they are, bit for bit.
+
+    E and A sum alpha-scaled errors: with a constant alpha, beta is the same as for unscaled errors; a changing alpha weights
+    older errors by the alpha they had.  ``coherence`` and ``accum``: contiguous float32 (N, 2) tensors on the weights'
+    device; ``accum`` is scratch that must be all zero and is left all zero.  ``delta_out``: a preallocated (M,) float32
+    tensor (CUDA-graph capture)."""
+    _board_arg(afterstate, "afterstate")
+    m = afterstate.shape[0]
+    _cuda(target, "target")
+    if target.dtype != torch.float32 or tuple(target.shape) != (m,):
+        raise ValueError(f"target must be float32 ({m},)")
+    if mask is not None:
+        _cuda(mask, "mask")
+        if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,):
+            raise ValueError(f"mask must be bool/uint8 ({m},)")
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, afterstate.device)
+    for name, t in (("coherence", coherence), ("accum", accum)):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float32
+                and tuple(t.shape) == (n, 2) and t.device == afterstate.device):
+            raise ValueError(f"{name} must be a contiguous float32 ({n}, 2) tensor on {afterstate.device}")
+    delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
+    if m == 0:
+        return delta_out
+    lib = _lib.load()
+    with torch.cuda.device(afterstate.device):
+        rc = lib.ml2048_tc_update(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None,
+                                  float(alpha), weights.data_ptr(), coherence.data_ptr(), accum.data_ptr(), n, cells.ctypes.data,
+                                  lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(afterstate))
+    _lib.check(rc, "ml2048_tc_update")
     return delta_out

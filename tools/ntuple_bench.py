@@ -166,10 +166,10 @@ class TorchComposed:
         return delta
 
 
-def learner_run(m: int, alpha: float, steps: int, seed: int = 0, curve_every: int = 0, net=None):
+def learner_run(m: int, alpha: float, steps: int, seed: int = 0, curve_every: int = 0, net=None, rule: str = "td0"):
     net = net or NTupleNetwork()
     env = ml2048_b200.VecGame(m, output="torch", sync_free=True, rng_mode="philox")
-    learner = TDAfterstateLearner(env, net, alpha=alpha)
+    learner = TDAfterstateLearner(env, net, alpha=alpha, rule=rule)
     learner.reset(seed)
     curve, t0 = [], time.perf_counter()
     window = curve_every or max(steps // 4, 1)
