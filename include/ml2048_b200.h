@@ -28,9 +28,9 @@
 extern "C" {
 #endif
 
-/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, ml2048_expectimax and ml2048_tc_update, added without
- * a bump (unlike earlier additions): they change no existing struct or signature, and a loader that binds them by name fails
- * on a library without them. */
+/* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, ml2048_expectimax, ml2048_tc_update,
+ * ml2048_lambda_td_update and ml2048_lambda_tc_update, added without a bump (unlike earlier additions): they change no existing
+ * struct or signature, and a loader that binds them by name fails on a library without them. */
 #define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
@@ -339,6 +339,32 @@ ML2048_API int ml2048_ntuple_td_update(const void *after, const float *target, c
 ML2048_API int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
                                 float *coherence, float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
                                 int32_t num_tuples, float *delta_out, int64_t num_games, void *stream);
+
+/* delayed TD(lambda) (Jaskowski 2018): one synchronous batch that updates each game's afterstate of h learner steps ago toward
+ * a lambda-return truncated at h, then ml2048_ntuple_td_update's rule (w[entry] += delta, float atomics) on its 8 * K entries.
+ * Network arguments as ml2048_ntuple_value.  Game i's window is x_0 ... x_h: x_0 the afterstate being updated, chosen h
+ * learner steps ago; x_h the one chosen this step; rho_k (k = 1..h) the reward of the move that produced x_k; e_k
+ * (k = 0..h-1) = 1 when the environment step after x_k was chosen ended the game; V_k = V(x_k) with the weights as they are
+ * before the call.  Ring (the caller's): after_ring [h+1][M][16] u8 (16-byte aligned), reward_ring [h+1][M] float32,
+ * ended_ring [h+1][M] u8; newest = the slot of x_h, x_k is in slot (newest - (h - k)) mod (h + 1); the ended byte of the newest
+ * slot is not read.  1 <= horizon (= h) <= 16, 0 <= newest <= h (E_SIZE); 0 <= lambda <= 1 (E_ENUM, also for NaN).  With
+ * lf = (float)lambda and c = 1.0f - lf, every operation one float32 operation (no contraction):
+ *   R_{h-1} = e_{h-1} ? 0 : rho_h + V_h
+ *   R_k     = e_k     ? 0 : (rho_{k+1} + c * V_{k+1}) + lf * R_{k+1}      for k = h-2 ... 0
+ *   delta   = alpha * (R_0 - V_0)                                         (0 where mask[i] == 0; mask may be null = all games)
+ * Values after the first end in the window are not looked up.  h = 1 is ml2048_ntuple_td_update's delta with
+ * target = e_0 ? 0 : rho_1 + V_1, bit for bit.  Every delta is computed before any weight is written. */
+ML2048_API int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                       int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                                       const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games,
+                                       void *stream);
+
+/* delayed TC(lambda): ml2048_lambda_td_update's delta, then ml2048_tc_update's phases 2 and 3 on x_0's entries (coherence and
+ * accum as there: [N][2] float32, 8-byte aligned, accum all zero on entry and left all zero). */
+ML2048_API int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                       int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                       float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                       float *delta_out, int64_t num_games, void *stream);
 
 /* expectimax move over an n-tuple network (network arguments as ml2048_ntuple_value), depth 1 or 2 chance layers.  With
  * after/r/valid as ml2048_afterstates gives them, V the network's value, p2 = (float)two_prob, p4 = 1.0f - p2, and every

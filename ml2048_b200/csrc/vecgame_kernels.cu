@@ -1600,6 +1600,54 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_tc_apply_kernel(const uin
     }
 }
 
+// ---- delayed TD(lambda) / TC(lambda) ------------------------------------------------------------
+// Definition (ml2048_lambda_td_update in the header, ops.ntuple_td_lambda_update and tests/_lambda_ref.py say the same; every
+// operation is one float32 operation, __fadd_rn / __fmul_rn, no contraction).  Game i's window is x_0 ... x_h: x_0 the
+// afterstate being updated (chosen h learner steps ago), x_h the one chosen this step; rho_k (k = 1..h) the reward of the move
+// that produced x_k; e_k (k = 0..h-1) = 1 when the environment step after x_k was chosen ended the game; V_k = V(x_k) with the
+// weights as they are before the call (ntuple_value).  With lf = float32(lambda) and c = 1.0f - lf rounded once on the host:
+//   R_{h-1} = e_{h-1} ? 0 : rho_h + V_h
+//   R_k     = e_k     ? 0 : (rho_{k+1} + c * V_{k+1}) + lf * R_{k+1}      for k = h-2 ... 0
+//   delta   = alpha * (R_0 - V_0)                                         (0 for a masked-out game)
+// h = 1 is TD(0)'s delta bit for bit.  Ring: after [h+1][M][16], reward [h+1][M], ended [h+1][M]; x_k is in slot
+// (newest - (h - k)) mod (h + 1) = (newest + 1 + k) mod (h + 1); the ended byte of the newest slot is not read.  The update of
+// x_0's entries is then TD(0)'s scatter or TC's phases 2 and 3 on x_0's slot, launched after this kernel: every delta is
+// computed before any weight is written.
+
+constexpr int kLambdaMaxHorizon = 16;
+
+// one thread per game: the first end in the window fixes where the recursion starts, so the values after it are never
+// looked up (they would be multiplied away by the 0 anyway, and skipping them changes no bit)
+__global__ void __launch_bounds__(kStepThreads) ntuple_lambda_delta_kernel(const uint4 *after, const float *reward, const uint8_t *ended,
+                                                                           const uint8_t *mask, int32_t horizon, int32_t newest, float lf,
+                                                                           float c, float alpha, const float *w,
+                                                                           __grid_constant__ const NTupleSpec spec, float *delta,
+                                                                           int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games) return;
+    float d = 0.0f;
+    if (!mask || mask[i]) {
+        const int32_t slots = horizon + 1;
+        int32_t s0 = newest + 1;  // slot of x_0
+        if (s0 == slots) s0 = 0;
+        auto slot = [&](int32_t k) { const int32_t s = s0 + k; return s >= slots ? s - slots : s; };
+        auto val = [&](int32_t k) {
+            const uint4 b = after[(int64_t)slot(k) * num_games + i];
+            return ntuple_value(w, spec, ntuple_nibbles(b.x, b.y, b.z, b.w));
+        };
+        int32_t top = horizon - 1;  // the first k with e_k = 1 (R_top = 0), else h - 1 (R_top = rho_h + V_h)
+        bool end = false;
+        for (int32_t k = 0; k < horizon && !end; ++k)
+            if (ended[(int64_t)slot(k) * num_games + i]) top = k, end = true;
+        float r = end ? 0.0f : __fadd_rn(reward[(int64_t)slot(horizon) * num_games + i], val(horizon));
+        for (int32_t k = top - 1; k >= 0; --k)
+            r = __fadd_rn(__fadd_rn(reward[(int64_t)slot(k + 1) * num_games + i], __fmul_rn(c, val(k + 1))), __fmul_rn(lf, r));
+        d = __fmul_rn(alpha, __fsub_rn(r, val(0)));
+    }
+    delta[i] = d;
+}
+
 // ---- expectimax over an n-tuple network -----------------------------------------------------
 // Definition (tests/_expectimax_ref.py is the same in NumPy; every operation is one float32 operation rounded on its own, so
 // the sums and products below are __fadd_rn / __fmul_rn / __fdiv_rn and nvcc cannot contract them into FMAs).  after(b,a),
@@ -2459,6 +2507,68 @@ int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask
                                                                         num_games);
     if (const int rc = launch_status()) return rc;
     ntuple_tc_apply_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, weights, reinterpret_cast<float2 *>(coherence),
+                                                                   reinterpret_cast<unsigned long long *>(accum), spec, num_games);
+    return launch_status();
+}
+
+// Checks and phase 1 shared by ml2048_lambda_td_update and ml2048_lambda_tc_update.  On success `x0` is x_0's slot of the
+// after ring, ready for the rule's own update launches.
+static int lambda_delta(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                        float lambda, const uint8_t *mask, float alpha, const float *weights, int64_t num_weights, const uint8_t *cells,
+                        const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, cudaStream_t s, NTupleSpec &spec,
+                        int64_t &grid, const uint4 *&x0)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!after_ring || !reward_ring || !ended_ring || !weights || !delta_out) return ML2048_E_NULL;
+    if (misaligned(after_ring, 16) || misaligned(reward_ring, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
+    if (horizon < 1 || horizon > kLambdaMaxHorizon || newest < 0 || newest > horizon) return ML2048_E_SIZE;
+    if (!(lambda >= 0.0f && lambda <= 1.0f)) return ML2048_E_ENUM;  // NaN fails both
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    grid = (num_games + kStepThreads - 1) / kStepThreads;
+    if (grid > 0x7fffffff) return ML2048_E_SIZE;
+    const uint4 *ring = reinterpret_cast<const uint4 *>(after_ring);
+    x0 = ring + (int64_t)(newest == horizon ? 0 : newest + 1) * num_games;
+    const float c = 1.0f - lambda;
+    clear_stale_error();
+    ntuple_lambda_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha,
+                                                                       weights, spec, delta_out, num_games);
+    return launch_status();
+}
+
+int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                            float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights, const uint8_t *cells,
+                            const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+{
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    NTupleSpec spec;
+    int64_t grid = 0;
+    const uint4 *x0 = nullptr;
+    if (const int rc = lambda_delta(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells,
+                                    len, num_tuples, delta_out, num_games, s, spec, grid, x0))
+        return rc;
+    ntuple_td_scatter_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, delta_out, weights, spec, num_games);
+    return launch_status();
+}
+
+int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                            float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence, float *accum,
+                            int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
+                            int64_t num_games, void *stream)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!coherence || !accum) return ML2048_E_NULL;
+    if (misaligned(coherence, 8) || misaligned(accum, 8)) return ML2048_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    NTupleSpec spec;
+    int64_t grid = 0;
+    const uint4 *x0 = nullptr;
+    if (const int rc = lambda_delta(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells,
+                                    len, num_tuples, delta_out, num_games, s, spec, grid, x0))
+        return rc;
+    ntuple_tc_accumulate_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, delta_out, reinterpret_cast<float2 *>(accum), spec,
+                                                                        num_games);
+    if (const int rc = launch_status()) return rc;
+    ntuple_tc_apply_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
                                                                    reinterpret_cast<unsigned long long *>(accum), spec, num_games);
     return launch_status();
 }

@@ -4,7 +4,9 @@ An n-tuple network (Szubert & Jaskowski 2014; Yeh et al. 2016) values a 2048 boa
 4-bit fields of a few cells, over the board's 8 symmetric images (one table per tuple, shared by the images).  Evaluating it,
 choosing the greedy afterstate move with it and updating it are integer byte work on boards plus scattered 4-byte reads and
 adds: each is one kernel here (``ops.ntuple_value``, ``ops.ntuple_greedy``, ``ops.ntuple_td_update``; temporal coherence
-learning, a step size per weight, is ``ops.ntuple_tc_update`` and ``TDAfterstateLearner(..., rule="tc")``).
+learning, a step size per weight, is ``ops.ntuple_tc_update`` and ``TDAfterstateLearner(..., rule="tc")``; their delayed
+lambda-return forms are ``ops.ntuple_td_lambda_update`` / ``ntuple_tc_lambda_update`` and ``TDAfterstateLearner(...,
+horizon=h, lam=lam)``).
 
     net = NTupleNetwork(device="cuda")                        # the standard 4x6 network, zero weights (256 MiB)
     env = VecGame(16384, output="torch", sync_free=True)
@@ -51,6 +53,13 @@ def default_tc_alpha(num_games: int) -> float:
     return DEFAULT_TC_ALPHA_TIMES_GAMES / num_games
 
 
+# Step size of TDAfterstateLearner(rule="tc", horizon=h > 1): alpha = DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES / M.
+# tools/lambda_bench.py swept c = 0.2 ... 3.2 at M = 2^14 for the best (h, lambda) = (2, 0.25) of its sweep at c = 0.8, 30 000
+# steps each (profiles/lambda_bench.txt, B200): mean score 12.0k / 14.2k / 8.9k / 4.1k / 4.0k for c = 0.2 / 0.4 / 0.8 / 1.6 /
+# 3.2, so delayed TC(lambda) takes half of TC's step size.  TD(lambda)'s best c is TD(0)'s 0.4.
+DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES = 0.4
+
+
 class NTupleNetwork:
     """An n-tuple value function with its weights on one CUDA device.
 
@@ -71,8 +80,9 @@ class NTupleNetwork:
             self.offsets.append(total)
             total += 16 ** len(t)
         self.weights = torch.zeros((total,), dtype=torch.float32, device=dev)
-        self.coherence: Optional[torch.Tensor] = None  # TC learning's {E, A} per weight, allocated by the first tc_update
-        self._tc_accum: Optional[torch.Tensor] = None  # tc_update's scratch, all zero between calls
+        # TC learning's {E, A} per weight and the TC updates' scratch (all zero between calls), allocated by the first TC update
+        self.coherence: Optional[torch.Tensor] = None
+        self._tc_accum: Optional[torch.Tensor] = None
 
     def value(self, board: torch.Tensor, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """V of (M,16) boards: (M,) float32 (``ops.ntuple_value``)."""
@@ -96,17 +106,37 @@ class NTupleNetwork:
         The adds are float atomics: the weights are reproducible up to the fp32 rounding of their order."""
         return ops.ntuple_td_update(afterstate, target, self.weights, self.tuples, alpha=alpha, mask=mask, delta_out=delta_out)
 
+    def _tc_alloc(self) -> None:
+        if self.coherence is None:
+            self.coherence = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
+        if self._tc_accum is None:
+            self._tc_accum = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
+
     def tc_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
                   delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One synchronous temporal coherence batch toward ``target``; returns delta = alpha * (target - V)
         (``ops.ntuple_tc_update``).  The first call allocates ``coherence`` ((N, 2) float32 {E, A} per weight, zeros) and a
         zero scratch accumulator of the same shape."""
-        if self.coherence is None:
-            self.coherence = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
-        if self._tc_accum is None:
-            self._tc_accum = torch.zeros((self.weights.numel(), 2), dtype=torch.float32, device=self.device)
+        self._tc_alloc()
         return ops.ntuple_tc_update(afterstate, target, self.weights, self.coherence, self._tc_accum, self.tuples, alpha=alpha,
                                     mask=mask, delta_out=delta_out)
+
+    def td_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
+                         alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
+                         delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One synchronous delayed TD(lambda) batch over the caller's ring of each game's last h + 1 afterstates; returns
+        delta = alpha * (R_0 - V(x_0)) (``ops.ntuple_td_lambda_update``)."""
+        return ops.ntuple_td_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.tuples, alpha=alpha,
+                                           lam=lam, mask=mask, delta_out=delta_out)
+
+    def tc_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
+                         alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
+                         delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One synchronous delayed TC(lambda) batch (``ops.ntuple_tc_lambda_update``); ``coherence`` and the scratch
+        accumulator are allocated as by ``tc_update``."""
+        self._tc_alloc()
+        return ops.ntuple_tc_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.coherence,
+                                           self._tc_accum, self.tuples, alpha=alpha, lam=lam, mask=mask, delta_out=delta_out)
 
     def state_dict(self) -> dict:
         state = {"tuples": [list(t) for t in self.tuples], "weights": self.weights.detach().clone()}
@@ -184,20 +214,37 @@ class TDAfterstateLearner:
     (evaluation).  Call ``reset(seed)`` instead of ``env.reset`` so that no afterstate of the old games is updated.
 
     ``rule``: ``"td0"`` (the default) updates with ``NTupleNetwork.td_update``; ``"tc"`` with temporal coherence learning
-    (``NTupleNetwork.tc_update``: a step size per weight), whose ``alpha`` defaults to ``default_tc_alpha(M)``."""
+    (``NTupleNetwork.tc_update``: a step size per weight), whose ``alpha`` defaults to ``default_tc_alpha(M)``.
 
-    def __init__(self, env, net: NTupleNetwork, alpha: Optional[float] = None, rule: str = "td0"):
+    ``horizon`` = h > 1 makes the rule delayed TD(lambda) / TC(lambda) (``NTupleNetwork.td_lambda_update`` /
+    ``tc_lambda_update``, lambda = ``lam``): the learner keeps each game's last h + 1 afterstates, rewards and end flags in a
+    ring, and step T (counted from ``reset()``) writes x_T and its reward into slot T mod (h + 1) straight from the greedy
+    kernel and, after ``env.step``, the game's end flag.  Steps 0 .. h-1 update nothing; from step h on, each step updates
+    the afterstate of step T - h (slot (T + 1) mod (h + 1)) toward the lambda-return over the window up to x_T, truncated at
+    the first end in it.  So the last h afterstates of a run are never updated.  ``delta`` is the delta of the afterstate
+    updated in the step (0 while nothing is).  With ``rule="tc"`` and h > 1, ``alpha`` defaults to
+    ``DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES / M``.  ``horizon=1`` is the TD(0) / TC learner above, whatever ``lam`` is."""
+
+    def __init__(self, env, net: NTupleNetwork, alpha: Optional[float] = None, rule: str = "td0", horizon: int = 1,
+                 lam: float = 0.5):
         if env._output != "torch" or not env._sync_free:
             raise ValueError("TDAfterstateLearner needs VecGame(..., output='torch', sync_free=True)")
         if env.device != net.device:
             raise ValueError(f"the environment is on {env.device}, the network on {net.device}")
         if rule not in ("td0", "tc"):
             raise ValueError(f"rule must be 'td0' or 'tc', got {rule!r}")
+        if isinstance(horizon, bool) or not isinstance(horizon, int) or not 1 <= horizon <= ops.NTUPLE_LAMBDA_MAX_HORIZON:
+            raise ValueError(f"horizon must be an int in 1..{ops.NTUPLE_LAMBDA_MAX_HORIZON}, got {horizon!r}")
+        if isinstance(lam, bool) or not isinstance(lam, (int, float)) or not 0.0 <= lam <= 1.0:
+            raise ValueError(f"lam must be a number in [0, 1], got {lam!r}")
+        self.horizon, self.lam = horizon, float(lam)
         self.env, self.net, self.rule = env, net, rule
         if alpha is not None:
             self.alpha = float(alpha)
         else:
             self.alpha = default_tc_alpha(env._size) if rule == "tc" else default_alpha(env._size)
+            if rule == "tc" and horizon > 1:
+                self.alpha = DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES / env._size
         self._update = net.tc_update if rule == "tc" else net.td_update
         m, dev = env._size, env.device
         self._out = {"action": torch.zeros((m,), dtype=torch.uint8, device=dev),
@@ -209,12 +256,25 @@ class TDAfterstateLearner:
         self._has_prev = torch.zeros((m,), dtype=torch.uint8, device=dev)
         self._target = torch.zeros((m,), dtype=torch.float32, device=dev)
         self.delta = torch.zeros((m,), dtype=torch.float32, device=dev)  # the last update's alpha * TD error (0: masked out)
+        if horizon > 1:
+            slots = horizon + 1
+            self._lambda_update = net.tc_lambda_update if rule == "tc" else net.td_lambda_update
+            self._after_ring = torch.zeros((slots, m, 16), dtype=torch.uint8, device=dev)
+            self._reward_ring = torch.zeros((slots, m), dtype=torch.float32, device=dev)
+            self._ended_ring = torch.zeros((slots, m), dtype=torch.uint8, device=dev)
+            self._ring_out = [dict(self._out, state=self._after_ring[s], reward=self._reward_ring[s]) for s in range(slots)]
+            self._steps = 0  # steps since reset(): the window is full from step h on
 
     def reset(self, seed: Optional[int] = None) -> None:
         self.env.reset(seed)
         self._has_prev.zero_()
+        if self.horizon > 1:
+            self._steps = 0
+            self.delta.zero_()
 
     def step(self):
+        if self.horizon > 1:
+            return self._step_lambda()
         env = self.env
         env.prepare()
         board = env.observations()[0]
@@ -227,4 +287,18 @@ class TDAfterstateLearner:
         self._prev_after.copy_(g["state"])
         self._prev_ended.copy_(res["terminated"])
         self._has_prev.fill_(1)
+        return res
+
+    def _step_lambda(self):
+        env, h = self.env, self.horizon
+        env.prepare()
+        board = env.observations()[0]
+        newest = self._steps % (h + 1)
+        g = self.net.greedy(board, reward_fn=env._reward_fn, action_dtype=torch.uint8, out=self._ring_out[newest])
+        if self.alpha != 0.0 and self._steps >= h:
+            self._lambda_update(self._after_ring, self._reward_ring, self._ended_ring, newest, self.alpha, self.lam,
+                                delta_out=self.delta)
+        res = env.step(g["action"])
+        self._ended_ring[newest].copy_(res["terminated"])
+        self._steps += 1
         return res

@@ -11,6 +11,8 @@
                                 counterpart; ml2048_b200.ntuple wraps them)
     ntuple_expectimax           the expectimax move over such a network, one or two chance layers deep
     ntuple_tc_update            a temporal coherence batch update of such a network: per-weight step sizes
+    ntuple_td_lambda_update,    delayed TD(lambda) / TC(lambda): the afterstate of h steps ago toward a lambda-return over
+    ntuple_tc_lambda_update     the caller's ring of each game's last h + 1 afterstates, valued in one kernel
 """
 
 from __future__ import annotations
@@ -461,4 +463,103 @@ def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
                                   float(alpha), weights.data_ptr(), coherence.data_ptr(), accum.data_ptr(), n, cells.ctypes.data,
                                   lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(afterstate))
     _lib.check(rc, "ml2048_tc_update")
+    return delta_out
+
+
+NTUPLE_LAMBDA_MAX_HORIZON = 16
+
+
+def _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask) -> tuple[int, int, float]:
+    """checks of the ring, ``newest``, ``lam`` and ``mask`` shared by the two lambda updates; returns (h, M, lam)"""
+    if not (isinstance(after_ring, torch.Tensor) and after_ring.dtype in (torch.uint8, torch.int8) and after_ring.ndim == 3
+            and after_ring.shape[2] == 16):
+        raise ValueError("after_ring must be uint8/int8 (h+1, M, 16)")
+    slots, m = after_ring.shape[0], after_ring.shape[1]
+    h = slots - 1
+    if not 1 <= h <= NTUPLE_LAMBDA_MAX_HORIZON:
+        raise ValueError(f"after_ring holds h + 1 = {slots} slots: the horizon h must be 1..{NTUPLE_LAMBDA_MAX_HORIZON}")
+    if isinstance(newest, bool) or not isinstance(newest, int) or not 0 <= newest <= h:
+        raise ValueError(f"newest must be an int slot 0..{h}, got {newest!r}")
+    try:
+        lam = float(lam)
+    except (TypeError, ValueError):
+        raise ValueError(f"lam must be a number in [0, 1], got {lam!r}") from None
+    if not 0.0 <= lam <= 1.0:
+        raise ValueError(f"lam must be in [0, 1], got {lam!r}")
+    _cuda(after_ring, "after_ring")
+    dev = after_ring.device
+    for name, t, dtypes in (("reward_ring", reward_ring, (torch.float32,)), ("ended_ring", ended_ring, (torch.bool, torch.uint8))):
+        _cuda(t, name)
+        if t.dtype not in dtypes or tuple(t.shape) != (slots, m) or t.device != dev:
+            raise ValueError(f"{name} must be {'/'.join(str(d) for d in dtypes)} ({slots}, {m}) on {dev}")
+    if mask is not None:
+        _cuda(mask, "mask")
+        if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,) or mask.device != dev:
+            raise ValueError(f"mask must be bool/uint8 ({m},) on {dev}")
+    return h, m, lam
+
+
+def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
+                            weights: torch.Tensor, tuples, *, alpha: float, lam: float, mask: Optional[torch.Tensor] = None,
+                            delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One synchronous batch of delayed TD(lambda) updates of an n-tuple network (Jaskowski 2018), in place on ``weights``:
+    each game's afterstate of h learner steps ago moves toward a lambda-return truncated at h.  Returns delta (M,) float32.
+
+    Game i's window is x_0 ... x_h: x_0 the afterstate being updated, chosen h learner steps ago; x_h the one chosen this
+    step; rho_k (k = 1..h) the reward of the move that produced x_k; e_k (k = 0..h-1) = 1 when the environment step after
+    x_k was chosen ended the game; V_k = V(x_k) (``ntuple_value``) with the weights as they are before the call.  With
+    lf = float32(lam) and c = 1 - lf in float32, every operation one float32 operation:
+
+        R_{h-1} = e_{h-1} ? 0 : rho_h + V_h
+        R_k     = e_k     ? 0 : (rho_{k+1} + c * V_{k+1}) + lf * R_{k+1}      for k = h-2 ... 0
+        delta   = alpha * (R_0 - V_0)                                         (0 for a game whose ``mask`` byte is 0)
+
+    then ``ntuple_td_update``'s phase 2 on x_0's entries (float atomics).  h = 1 is ``ntuple_td_update``'s delta with
+    target = (0 if e_0 else rho_1 + V_1), bit for bit.  Values after the first end in a window are not looked up.
+
+    The ring is the caller's: ``after_ring`` (h+1, M, 16) uint8/int8, ``reward_ring`` (h+1, M) float32, ``ended_ring``
+    (h+1, M) bool/uint8, all contiguous on one device, h = ``after_ring.shape[0] - 1`` in 1..16.  ``newest`` is the slot of
+    x_h; x_k is in slot (newest - (h - k)) mod (h + 1), and ``ended_ring[newest]`` is not read.  ``mask``: (M,) bool/uint8,
+    None = every game.  ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
+    h, m, lam = _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask)
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, after_ring.device)
+    delta_out = _out_arg(delta_out, (m,), torch.float32, after_ring.device, "delta_out")
+    if m == 0:
+        return delta_out
+    lib = _lib.load()
+    with torch.cuda.device(after_ring.device):
+        rc = lib.ml2048_lambda_td_update(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
+                                         mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(), n,
+                                         cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(after_ring))
+    _lib.check(rc, "ml2048_lambda_td_update")
+    return delta_out
+
+
+def ntuple_tc_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
+                            weights: torch.Tensor, coherence: torch.Tensor, accum: torch.Tensor, tuples, *, alpha: float,
+                            lam: float, mask: Optional[torch.Tensor] = None,
+                            delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One synchronous batch of delayed TC(lambda) updates, in place on ``weights`` and ``coherence``; returns delta (M,)
+    float32.  delta is ``ntuple_td_lambda_update``'s (the same window, ring, definition and arguments); the update of x_0's
+    entries is then ``ntuple_tc_update``'s phases 2 and 3: {dE, dA} += {delta, |delta|} into ``accum``, and w += beta * dE,
+    beta = |E| / A (1 where A = 0), {E, A} += {dE, dA} for every entry with dA != 0.  ``coherence`` and ``accum``: contiguous
+    float32 (N, 2) tensors on the ring's device; ``accum`` must be all zero and is left all zero."""
+    h, m, lam = _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask)
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, after_ring.device)
+    for name, t in (("coherence", coherence), ("accum", accum)):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float32
+                and tuple(t.shape) == (n, 2) and t.device == after_ring.device):
+            raise ValueError(f"{name} must be a contiguous float32 ({n}, 2) tensor on {after_ring.device}")
+    delta_out = _out_arg(delta_out, (m,), torch.float32, after_ring.device, "delta_out")
+    if m == 0:
+        return delta_out
+    lib = _lib.load()
+    with torch.cuda.device(after_ring.device):
+        rc = lib.ml2048_lambda_tc_update(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
+                                         mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(),
+                                         coherence.data_ptr(), accum.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k,
+                                         delta_out.data_ptr(), m, _stream(after_ring))
+    _lib.check(rc, "ml2048_lambda_tc_update")
     return delta_out

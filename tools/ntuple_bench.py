@@ -166,10 +166,11 @@ class TorchComposed:
         return delta
 
 
-def learner_run(m: int, alpha: float, steps: int, seed: int = 0, curve_every: int = 0, net=None, rule: str = "td0"):
+def learner_run(m: int, alpha: float, steps: int, seed: int = 0, curve_every: int = 0, net=None, rule: str = "td0",
+                horizon: int = 1, lam: float = 0.5):
     net = net or NTupleNetwork()
     env = ml2048_b200.VecGame(m, output="torch", sync_free=True, rng_mode="philox")
-    learner = TDAfterstateLearner(env, net, alpha=alpha, rule=rule)
+    learner = TDAfterstateLearner(env, net, alpha=alpha, rule=rule, horizon=horizon, lam=lam)
     learner.reset(seed)
     curve, t0 = [], time.perf_counter()
     window = curve_every or max(steps // 4, 1)
