@@ -750,6 +750,18 @@ ML2048_FN uint32_t ntuple_index(uint64_t nib, const uint8_t *src4, uint32_t len)
     return idx;
 }
 
+// Visit the 8K table entries of a board in the fixed order t = 0..K-1, g = 0..7: visit(offset, index) with offset = tuple
+// t's first entry and index = image g's entry within that table, so entry j = offset + index of every weight-sized array.
+template <class Visit>
+ML2048_FN void ntuple_for_each_entry(const NTupleSpec &s, uint64_t nib, Visit &&visit)
+{
+    for (uint32_t t = 0; t < s.num_tuples; ++t) {
+        const uint32_t off = s.offset[t], len = s.len[t];
+#pragma unroll
+        for (uint32_t g = 0; g < 8; ++g) visit(off, ntuple_index(nib, s.src4[t][g], len));
+    }
+}
+
 #if defined(__CUDACC__)
 ML2048_FN float load_weight(const float *p) { return __ldg(p); }
 #else
@@ -761,12 +773,7 @@ ML2048_FN float load_weight(const float *p) { return *p; }
 ML2048_FN float ntuple_value(const float *w, const NTupleSpec &s, uint64_t nib)
 {
     float acc = 0.0f;
-    for (uint32_t t = 0; t < s.num_tuples; ++t) {
-        const float *tab = w + s.offset[t];
-        const uint32_t len = s.len[t];
-#pragma unroll
-        for (uint32_t g = 0; g < 8; ++g) acc += load_weight(tab + ntuple_index(nib, s.src4[t][g], len));
-    }
+    ntuple_for_each_entry(s, nib, [&](uint32_t off, uint32_t idx) { acc += load_weight(w + off + idx); });
     return acc;
 }
 

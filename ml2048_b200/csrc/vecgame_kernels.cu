@@ -1416,6 +1416,17 @@ __global__ void fill_terminated_kernel(uint8_t *terminated, int64_t num_games, i
 // `merged`.  The move, the reward and the `merged` log are the step kernel's own functions (move_board_sel with a row of
 // d_move_sel, step_reward, fusion_log).  A direction that does not change the board gets reward 0 (the step kernel leaves
 // the stale reward there instead); it fuses nothing, so its `merged` row is 0 as well.
+
+// Board `bd` moved in direction `dir` (0..3) without the spawn: the moved board in `now`, what fused in `f`; true iff the move
+// changed the board, i.e. the direction is valid
+__device__ __forceinline__ bool try_move(uint4 bd, uint32_t dir, uint4 &now, Fusions &f)
+{
+    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    move_board_sel(r0, r1, r2, r3, d_move_sel + dir * kMoveSelRow, f);
+    now = make_uint4(r0, r1, r2, r3);
+    return ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+}
+
 template <bool kLog>
 __global__ void __launch_bounds__(kStepThreads) afterstates_kernel(const uint4 *board, uint4 *after, float *reward, uint8_t *valid,
                                                                    uint4 *merged, int32_t reward_kind, int64_t num_games)
@@ -1423,11 +1434,9 @@ __global__ void __launch_bounds__(kStepThreads) afterstates_kernel(const uint4 *
     const int64_t t = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;  // 64-bit: 16 * t passes 2^31 at 2^25 games
     if (t >= 4 * num_games) return;
     const uint4 bd = board[t >> 2];
-    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    uint4 now;
     Fusions f;
-    move_board_sel(r0, r1, r2, r3, d_move_sel + (threadIdx.x & 3u) * kMoveSelRow, f);
-    const uint4 now = make_uint4(r0, r1, r2, r3);
-    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    const bool moved = try_move(bd, threadIdx.x & 3u, now, f);
     after[t] = now;
     reward[t] = moved ? step_reward<false>(reward_kind, f, now, bd, fusion_gain(f)) : 0.0f;
     valid[t] = moved ? 1 : 0;
@@ -1466,15 +1475,13 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_greedy_kernel(const uint4
     const bool live = t < 4 * num_games;  // all four lanes of a game are live or none: the shuffles below need every lane
     const uint32_t a = threadIdx.x & 3u;
     const uint4 bd = live ? board[t >> 2] : make_uint4(0u, 0u, 0u, 0u);
-    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    uint4 now;
     Fusions f;
-    move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
-    const uint4 now = make_uint4(r0, r1, r2, r3);
-    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    const bool moved = try_move(bd, a, now, f);
     float r = 0.0f, v = 0.0f, key = -INFINITY;
     if (moved) {
         r = step_reward<false>(reward_kind, f, now, bd, fusion_gain(f));
-        v = ntuple_value(w, spec, ntuple_nibbles(r0, r1, r2, r3));
+        v = ntuple_value(w, spec, ntuple_nibbles(now.x, now.y, now.z, now.w));
         const float q = r + v;
         key = (q == q) ? q : -INFINITY;
     }
@@ -1522,14 +1529,8 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const u
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
     if (i >= num_games || (mask && !mask[i])) return;
     const uint4 b = after[i];
-    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
     const float d = delta[i];
-    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
-        float *tab = w + spec.offset[k];
-        const uint32_t len = spec.len[k];
-#pragma unroll
-        for (uint32_t g = 0; g < 8; ++g) atomicAdd(tab + ntuple_index(nib, spec.src4[k][g], len), d);
-    }
+    ntuple_for_each_entry(spec, ntuple_nibbles(b.x, b.y, b.z, b.w), [&](uint32_t off, uint32_t idx) { atomicAdd(w + off + idx, d); });
 }
 
 // ---- temporal coherence (TC) learning ---------------------------------------------------------
@@ -1555,15 +1556,9 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_tc_accumulate_kernel(cons
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
     if (i >= num_games || (mask && !mask[i])) return;
     const uint4 b = after[i];
-    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
     const float d = delta[i];
     const float2 e = make_float2(d, fabsf(d));
-    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
-        float2 *tab = acc + spec.offset[k];
-        const uint32_t len = spec.len[k];
-#pragma unroll
-        for (uint32_t g = 0; g < 8; ++g) atomicAdd(tab + ntuple_index(nib, spec.src4[k][g], len), e);
-    }
+    ntuple_for_each_entry(spec, ntuple_nibbles(b.x, b.y, b.z, b.w), [&](uint32_t off, uint32_t idx) { atomicAdd(acc + off + idx, e); });
 }
 
 // TC, phase 3: one thread per masked-in game walks its own entries and claims each with a 64-bit exchange against 0; only
@@ -1580,24 +1575,19 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_tc_apply_kernel(const uin
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
     if (i >= num_games || (mask && !mask[i])) return;
     const uint4 b = after[i];
-    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
-    for (uint32_t k = 0; k < spec.num_tuples; ++k) {
-        const uint32_t off = spec.offset[k], len = spec.len[k];
-#pragma unroll
-        for (uint32_t g = 0; g < 8; ++g) {
-            const uint32_t j = off + ntuple_index(nib, spec.src4[k][g], len);
+    ntuple_for_each_entry(spec, ntuple_nibbles(b.x, b.y, b.z, b.w), [&](uint32_t off, uint32_t idx) {
+        const uint32_t j = off + idx;
 #if !defined(ML2048_TC_APPLY_ALWAYS_EXCHANGE)
-            if (__ldcg(acc + j) == 0ull) continue;
+        if (__ldcg(acc + j) == 0ull) return;
 #endif
-            const unsigned long long word = atomicExch(acc + j, 0ull);
-            const float dE = __uint_as_float((uint32_t)word), dA = __uint_as_float((uint32_t)(word >> 32));
-            if (dA == 0.0f) continue;  // NaN goes on
-            const float2 c = coh[j];
-            const float beta = c.y == 0.0f ? 1.0f : __fdiv_rn(fabsf(c.x), c.y);
-            w[j] = __fadd_rn(w[j], __fmul_rn(beta, dE));
-            coh[j] = make_float2(__fadd_rn(c.x, dE), __fadd_rn(c.y, dA));
-        }
-    }
+        const unsigned long long word = atomicExch(acc + j, 0ull);
+        const float dE = __uint_as_float((uint32_t)word), dA = __uint_as_float((uint32_t)(word >> 32));
+        if (dA == 0.0f) return;  // NaN goes on
+        const float2 c = coh[j];
+        const float beta = c.y == 0.0f ? 1.0f : __fdiv_rn(fabsf(c.x), c.y);
+        w[j] = __fadd_rn(w[j], __fmul_rn(beta, dE));
+        coh[j] = make_float2(__fadd_rn(c.x, dE), __fadd_rn(c.y, dA));
+    });
 }
 
 // ---- delayed TD(lambda) / TC(lambda) ------------------------------------------------------------
@@ -1709,7 +1699,7 @@ __device__ __forceinline__ float chance1(uint4 s, const float *w, const NTupleSp
         uint32_t r0 = s.x, r1 = s.y, r2 = s.z, r3 = s.w;
         put_cell_shift(r0, r1, r2, r3, kth_set_bit16(empties, live ? o / per_cell : 0u), law.tile(o));
         const uint4 sp = make_uint4(r0, r1, r2, r3);
-        Fusions f;
+        Fusions f;  // try_move written out: as a call it compiles this function to different SASS
         move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
         const bool moved = live && ((r0 ^ sp.x) | (r1 ^ sp.y) | (r2 ^ sp.z) | (r3 ^ sp.w)) != 0u;
         float key = -INFINITY;
@@ -1746,11 +1736,9 @@ __device__ __forceinline__ void expectimax_root(uint4 bd, float e, bool store, i
                                                 long long *action_i64, uint4 *after, float *reward, float *value, float *q_out)
 {
     const uint32_t a = threadIdx.x & 3u;
-    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    uint4 now;
     Fusions f;
-    move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
-    const uint4 now = make_uint4(r0, r1, r2, r3);
-    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
+    const bool moved = try_move(bd, a, now, f);
     float r = 0.0f, q = -INFINITY, key = -INFINITY;
     if (moved) {
         r = step_reward<false>(reward_kind, f, now, bd, fusion_gain(f));
@@ -1787,12 +1775,10 @@ __global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const u
     const int64_t g = (int64_t)blockIdx.x * kExpectimax1BoardsPerBlock + (warp >> 2);
     const bool live = g < num_games;
     const uint4 bd = live ? board[g] : make_uint4(0u, 0u, 0u, 0u);
-    uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+    uint4 now;
     Fusions f;
-    move_board_sel(r0, r1, r2, r3, d_move_sel + (warp & 3u) * kMoveSelRow, f);
-    const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
     float e = 0.0f;
-    if (moved) e = chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law);  // warp-uniform
+    if (try_move(bd, warp & 3u, now, f)) e = chance1(now, w, spec, reward_kind, law);  // warp-uniform
     if (lane == 0u) sh_e[warp] = e;
     __syncthreads();
     if (warp != 0u) return;
@@ -1817,11 +1803,10 @@ __global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const u
     const uint4 bd = board[g];
     float mine = 0.0f;
     for (uint32_t a = 0; a < 4u; ++a) {
-        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        uint4 now;
         Fusions f;
-        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
-        if (((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) == 0u) continue;
-        const float e = chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law);
+        if (!try_move(bd, a, now, f)) continue;
+        const float e = chance1(now, w, spec, reward_kind, law);
         if ((threadIdx.x & 3u) == a) mine = e;
     }
     expectimax_root(bd, mine, (threadIdx.x & 31u) < 4u, g, reward_kind, action_u8, action_i64, after, reward, value, q_out);
@@ -1847,11 +1832,9 @@ __global__ void __launch_bounds__(kExpectimaxThreads) expectimax2_kernel(const u
     uint32_t count[4];  // nodes under root direction a: 4 * outcomes of after(b, a), 0 for an invalid a
 #pragma unroll
     for (uint32_t a = 0; a < 4u; ++a) {
-        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        uint4 now;
         Fusions f;
-        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
-        const bool moved = ((r0 ^ bd.x) | (r1 ^ bd.y) | (r2 ^ bd.z) | (r3 ^ bd.w)) != 0u;
-        count[a] = moved ? 4u * per_cell * popc32(empty_cells(make_uint4(r0, r1, r2, r3))) : 0u;
+        count[a] = try_move(bd, a, now, f) ? 4u * per_cell * popc32(empty_cells(now)) : 0u;
     }
     const uint32_t total = count[0] + count[1] + count[2] + count[3];
     for (uint32_t j = threadIdx.x >> 5; j < total; j += kExpectimaxThreads / 32) {
@@ -1859,18 +1842,18 @@ __global__ void __launch_bounds__(kExpectimaxThreads) expectimax2_kernel(const u
 #pragma unroll
         for (uint32_t i = 0; i < 3u; ++i)
             if (a == i && rem >= count[i]) rem -= count[i], a = i + 1u;
-        uint32_t r0 = bd.x, r1 = bd.y, r2 = bd.z, r3 = bd.w;
+        uint4 s, now;
         Fusions f;
-        move_board_sel(r0, r1, r2, r3, d_move_sel + a * kMoveSelRow, f);
+        try_move(bd, a, s, f);  // a valid root direction: the others have no nodes
         const uint32_t o = rem >> 2, inner = rem & 3u;
-        put_cell_shift(r0, r1, r2, r3, kth_set_bit16(empty_cells(make_uint4(r0, r1, r2, r3)), o / per_cell), law.tile(o));
+        uint32_t r0 = s.x, r1 = s.y, r2 = s.z, r3 = s.w;
+        put_cell_shift(r0, r1, r2, r3, kth_set_bit16(empty_cells(s), o / per_cell), law.tile(o));
         const uint4 sp = make_uint4(r0, r1, r2, r3);
-        move_board_sel(r0, r1, r2, r3, d_move_sel + inner * kMoveSelRow, f);
-        const bool moved = ((r0 ^ sp.x) | (r1 ^ sp.y) | (r2 ^ sp.z) | (r3 ^ sp.w)) != 0u;
+        const bool moved = try_move(sp, inner, now, f);
         float key = -INFINITY;
         if (moved) {  // warp-uniform
-            const float rr = step_reward<false>(reward_kind, f, make_uint4(r0, r1, r2, r3), sp, fusion_gain(f));
-            const float q = __fadd_rn(rr, chance1(make_uint4(r0, r1, r2, r3), w, spec, reward_kind, law));
+            const float rr = step_reward<false>(reward_kind, f, now, sp, fusion_gain(f));
+            const float q = __fadd_rn(rr, chance1(now, w, spec, reward_kind, law));
             key = (q == q) ? q : -INFINITY;
         }
         if ((threadIdx.x & 31u) == 0u) sh_key[j] = key, sh_ok[j] = moved ? 1 : 0;
@@ -2466,23 +2449,73 @@ int ml2048_expectimax(const void *board, const float *weights, int64_t num_weigh
     return launch_status();
 }
 
+// Checks every n-tuple update shares: the batch, the afterstates (x_0's, or the ring that holds them), the float32 values the
+// delta starts from (the target, or the reward ring), the weights, the delta output and the network.  On success `spec` and
+// `grid` (one thread per game) are ready for the launches.
+static int check_update(const void *after, const float *values, const float *weights, const float *delta_out, int64_t num_weights,
+                        const uint8_t *cells, const uint8_t *len, int32_t num_tuples, int64_t num_games, NTupleSpec &spec, unsigned &grid)
+{
+    if (num_games <= 0) return ML2048_E_SIZE;
+    if (!after || !values || !weights || !delta_out) return ML2048_E_NULL;
+    if (misaligned(after, 16) || misaligned(values, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    const int64_t blocks = (num_games + kStepThreads - 1) / kStepThreads;
+    if (blocks > 0x7fffffff) return ML2048_E_SIZE;
+    grid = (unsigned)blocks;
+    return 0;
+}
+
+// Phase 1 of TD(0) and TC: delta = alpha * (target - V(after))
+static int target_delta(const uint4 *after, const float *target, const uint8_t *mask, float alpha, const float *weights,
+                        const NTupleSpec &spec, float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s)
+{
+    clear_stale_error();
+    ntuple_td_delta_kernel<<<grid, kStepThreads, 0, s>>>(after, target, mask, alpha, weights, spec, delta_out, num_games);
+    return launch_status();
+}
+
+// Phase 1 of TD(lambda) and TC(lambda): the checks only they make, then delta over the ring.  `x0` = x_0's slot of the ring.
+static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                        float lambda, const uint8_t *mask, float alpha, const float *weights, const NTupleSpec &spec, float *delta_out,
+                        unsigned grid, int64_t num_games, cudaStream_t s, const uint4 *&x0)
+{
+    if (!ended_ring) return ML2048_E_NULL;
+    if (horizon < 1 || horizon > kLambdaMaxHorizon || newest < 0 || newest > horizon) return ML2048_E_SIZE;
+    if (!(lambda >= 0.0f && lambda <= 1.0f)) return ML2048_E_ENUM;  // NaN fails both
+    x0 = ring + (int64_t)(newest == horizon ? 0 : newest + 1) * num_games;
+    const float c = 1.0f - lambda;
+    clear_stale_error();
+    ntuple_lambda_delta_kernel<<<grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha, weights,
+                                                             spec, delta_out, num_games);
+    return launch_status();
+}
+
+// The update of x_0's entries after phase 1, on the same stream (so every delta is computed before any weight is written):
+// TD(0)'s scatter when `coherence` is null, else TC's phases 2 and 3
+static int apply_update(const uint4 *x0, const uint8_t *mask, const float *delta, float *weights, float *coherence, float *accum,
+                        const NTupleSpec &spec, unsigned grid, int64_t num_games, cudaStream_t s)
+{
+    if (!coherence) {
+        ntuple_td_scatter_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, weights, spec, num_games);
+        return launch_status();
+    }
+    ntuple_tc_accumulate_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, reinterpret_cast<float2 *>(accum), spec, num_games);
+    if (const int rc = launch_status()) return rc;
+    ntuple_tc_apply_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
+                                                         reinterpret_cast<unsigned long long *>(accum), spec, num_games);
+    return launch_status();
+}
+
 int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
                             const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
 {
-    if (num_games <= 0) return ML2048_E_SIZE;
-    if (!after || !target || !weights || !delta_out) return ML2048_E_NULL;
-    if (misaligned(after, 16) || misaligned(target, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
     NTupleSpec spec;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
-    const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
-    if (grid > 0x7fffffff) return ML2048_E_SIZE;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    unsigned grid = 0;
+    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid)) return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
-    clear_stale_error();
-    ntuple_td_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, target, mask, alpha, weights, spec, delta_out, num_games);
-    if (const int rc = launch_status()) return rc;
-    ntuple_td_scatter_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, delta_out, weights, spec, num_games);
-    return launch_status();
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
+    return apply_update(b, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
 }
 
 int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
@@ -2490,64 +2523,31 @@ int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask
                      int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
-    if (!after || !target || !weights || !coherence || !accum || !delta_out) return ML2048_E_NULL;
-    if (misaligned(after, 16) || misaligned(target, 4) || misaligned(weights, 4) || misaligned(coherence, 8) || misaligned(accum, 8) ||
-        misaligned(delta_out, 4))
-        return ML2048_E_ALIGN;
+    if (!coherence || !accum) return ML2048_E_NULL;
+    if (misaligned(coherence, 8) || misaligned(accum, 8)) return ML2048_E_ALIGN;
     NTupleSpec spec;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
-    const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
-    if (grid > 0x7fffffff) return ML2048_E_SIZE;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    unsigned grid = 0;
+    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid)) return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
-    clear_stale_error();
-    ntuple_td_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, target, mask, alpha, weights, spec, delta_out, num_games);
-    if (const int rc = launch_status()) return rc;
-    ntuple_tc_accumulate_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, delta_out, reinterpret_cast<float2 *>(accum), spec,
-                                                                        num_games);
-    if (const int rc = launch_status()) return rc;
-    ntuple_tc_apply_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(b, mask, weights, reinterpret_cast<float2 *>(coherence),
-                                                                   reinterpret_cast<unsigned long long *>(accum), spec, num_games);
-    return launch_status();
-}
-
-// Checks and phase 1 shared by ml2048_lambda_td_update and ml2048_lambda_tc_update.  On success `x0` is x_0's slot of the
-// after ring, ready for the rule's own update launches.
-static int lambda_delta(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
-                        float lambda, const uint8_t *mask, float alpha, const float *weights, int64_t num_weights, const uint8_t *cells,
-                        const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, cudaStream_t s, NTupleSpec &spec,
-                        int64_t &grid, const uint4 *&x0)
-{
-    if (num_games <= 0) return ML2048_E_SIZE;
-    if (!after_ring || !reward_ring || !ended_ring || !weights || !delta_out) return ML2048_E_NULL;
-    if (misaligned(after_ring, 16) || misaligned(reward_ring, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
-    if (horizon < 1 || horizon > kLambdaMaxHorizon || newest < 0 || newest > horizon) return ML2048_E_SIZE;
-    if (!(lambda >= 0.0f && lambda <= 1.0f)) return ML2048_E_ENUM;  // NaN fails both
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
-    grid = (num_games + kStepThreads - 1) / kStepThreads;
-    if (grid > 0x7fffffff) return ML2048_E_SIZE;
-    const uint4 *ring = reinterpret_cast<const uint4 *>(after_ring);
-    x0 = ring + (int64_t)(newest == horizon ? 0 : newest + 1) * num_games;
-    const float c = 1.0f - lambda;
-    clear_stale_error();
-    ntuple_lambda_delta_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha,
-                                                                       weights, spec, delta_out, num_games);
-    return launch_status();
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
+    return apply_update(b, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
 }
 
 int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
                             float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights, const uint8_t *cells,
                             const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
 {
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
     NTupleSpec spec;
-    int64_t grid = 0;
-    const uint4 *x0 = nullptr;
-    if (const int rc = lambda_delta(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells,
-                                    len, num_tuples, delta_out, num_games, s, spec, grid, x0))
+    unsigned grid = 0;
+    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid))
         return rc;
-    ntuple_td_scatter_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, delta_out, weights, spec, num_games);
-    return launch_status();
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint4 *x0 = nullptr;
+    if (const int rc = lambda_delta(reinterpret_cast<const uint4 *>(after_ring), reward_ring, ended_ring, horizon, newest, lambda, mask, alpha,
+                                    weights, spec, delta_out, grid, num_games, s, x0))
+        return rc;
+    return apply_update(x0, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
 }
 
 int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
@@ -2558,19 +2558,16 @@ int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, co
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!coherence || !accum) return ML2048_E_NULL;
     if (misaligned(coherence, 8) || misaligned(accum, 8)) return ML2048_E_ALIGN;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
     NTupleSpec spec;
-    int64_t grid = 0;
-    const uint4 *x0 = nullptr;
-    if (const int rc = lambda_delta(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells,
-                                    len, num_tuples, delta_out, num_games, s, spec, grid, x0))
+    unsigned grid = 0;
+    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid))
         return rc;
-    ntuple_tc_accumulate_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, delta_out, reinterpret_cast<float2 *>(accum), spec,
-                                                                        num_games);
-    if (const int rc = launch_status()) return rc;
-    ntuple_tc_apply_kernel<<<(unsigned)grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
-                                                                   reinterpret_cast<unsigned long long *>(accum), spec, num_games);
-    return launch_status();
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint4 *x0 = nullptr;
+    if (const int rc = lambda_delta(reinterpret_cast<const uint4 *>(after_ring), reward_ring, ended_ring, horizon, newest, lambda, mask, alpha,
+                                    weights, spec, delta_out, grid, num_games, s, x0))
+        return rc;
+    return apply_update(x0, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
 }
 
 int ml2048_pack_flags(const void *valid, const uint8_t *terminated, const uint8_t *invalid, uint8_t *packed, int64_t num_games, void *stream)

@@ -122,6 +122,26 @@ def valid_actions(board: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def _out_arg(t, shape: tuple, dtype, device, name: str) -> torch.Tensor:
+    if t is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == dtype and tuple(t.shape) == shape
+            and t.device == device):
+        raise ValueError(f"{name} must be a contiguous {dtype} tensor {shape} on {device}")
+    return t
+
+
+def _out_dict(out, keys, op: str) -> dict:
+    """the ``out`` argument of an op that returns a dict of tensors: None or a dict holding any subset of ``keys``"""
+    out = {} if out is None else out
+    if not isinstance(out, dict):
+        raise ValueError("out must be a dict of tensors")
+    unknown = set(out) - set(keys)
+    if unknown:
+        raise ValueError(f"out has entries {op} does not write: {sorted(unknown)}")
+    return out
+
+
 # afterstates() outputs: key (VecStepResult's names) -> (shape after M, dtype)
 _AFTERSTATES = {
     "state": ((4, 16), torch.uint8),
@@ -150,25 +170,10 @@ def afterstates(board: torch.Tensor, *, reward_fn=None, merged: bool = False, ou
         raise ValueError("board must be uint8/int8 (M,16)")
     kind = reward_kind(reward_fn)
     keys = ("state", "reward", "valid_actions", "merged") if merged else ("state", "reward", "valid_actions")
-    out = {} if out is None else out
-    if not isinstance(out, dict):
-        raise ValueError("out must be a dict of tensors")
-    unknown = set(out) - set(keys)
-    if unknown:
-        raise ValueError(f"out has entries afterstates does not write: {sorted(unknown)}")
+    out = _out_dict(out, keys, "afterstates")
     _cuda(board, "board")
     m = board.shape[0]
-    res = {}
-    for k in keys:
-        shape, dtype = _AFTERSTATES[k]
-        shape = (m,) + shape
-        t = out.get(k)
-        if t is None:
-            t = torch.empty(shape, dtype=dtype, device=board.device)
-        elif not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == dtype and tuple(t.shape) == shape
-                  and t.device == board.device):
-            raise ValueError(f"out[{k!r}] must be a contiguous {dtype} tensor {shape} on {board.device}")
-        res[k] = t
+    res = {k: _out_arg(out.get(k), (m,) + _AFTERSTATES[k][0], _AFTERSTATES[k][1], board.device, f"out[{k!r}]") for k in keys}
     if m == 0:
         return res
     lib = _lib.load()
@@ -241,15 +246,6 @@ def _board_arg(board, name: str = "board") -> None:
     _cuda(board, name)
 
 
-def _out_arg(t, shape: tuple, dtype, device, name: str) -> torch.Tensor:
-    if t is None:
-        return torch.empty(shape, dtype=dtype, device=device)
-    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == dtype and tuple(t.shape) == shape
-            and t.device == device):
-        raise ValueError(f"{name} must be a contiguous {dtype} tensor {shape} on {device}")
-    return t
-
-
 def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """V(board) of an n-tuple network: (M,16) uint8/int8 boards -> (M,) float32.
 
@@ -276,6 +272,14 @@ def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Opt
 _NTUPLE_GREEDY = {"state": ((16,), torch.uint8), "reward": ((), torch.float32), "value": ((), torch.float32)}
 
 
+def _move_outputs(out, specs: dict, action_dtype, board, op: str) -> dict:
+    """the outputs of a move choice: "action" and ``specs`` (key -> (shape after M, dtype)), each ``out``'s tensor or a new one"""
+    specs = {"action": ((), action_dtype), **specs}
+    out = _out_dict(out, specs, op)
+    m = board.shape[0]
+    return {k: _out_arg(out.get(k), (m,) + shape, dtype, board.device, f"out[{k!r}]") for k, (shape, dtype) in specs.items()}
+
+
 def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
                   out: Optional[dict] = None) -> dict:
     """The greedy afterstate move of every board under an n-tuple network, in one kernel.
@@ -297,16 +301,8 @@ def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_
     kind = reward_kind(reward_fn)
     cells, lens, k, n = _spec_arrays(tuples)
     _weights_arg(weights, n, board.device)
-    out = {} if out is None else out
-    if not isinstance(out, dict):
-        raise ValueError("out must be a dict of tensors")
-    unknown = set(out) - {"action", *_NTUPLE_GREEDY}
-    if unknown:
-        raise ValueError(f"out has entries ntuple_greedy does not write: {sorted(unknown)}")
     m = board.shape[0]
-    res = {"action": _out_arg(out.get("action"), (m,), action_dtype, board.device, "out['action']")}
-    for key, (shape, dtype) in _NTUPLE_GREEDY.items():
-        res[key] = _out_arg(out.get(key), (m,) + shape, dtype, board.device, f"out[{key!r}]")
+    res = _move_outputs(out, _NTUPLE_GREEDY, action_dtype, board, "ntuple_greedy")
     if m == 0:
         return res
     act = res["action"].data_ptr()
@@ -363,16 +359,8 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
     kind = reward_kind(reward_fn)
     cells, lens, k, n = _spec_arrays(tuples)
     _weights_arg(weights, n, board.device)
-    out = {} if out is None else out
-    if not isinstance(out, dict):
-        raise ValueError("out must be a dict of tensors")
-    unknown = set(out) - {"action", *_NTUPLE_EXPECTIMAX}
-    if unknown:
-        raise ValueError(f"out has entries ntuple_expectimax does not write: {sorted(unknown)}")
     m = board.shape[0]
-    res = {"action": _out_arg(out.get("action"), (m,), action_dtype, board.device, "out['action']")}
-    for key, (shape, dtype) in _NTUPLE_EXPECTIMAX.items():
-        res[key] = _out_arg(out.get(key), (m,) + shape, dtype, board.device, f"out[{key!r}]")
+    res = _move_outputs(out, _NTUPLE_EXPECTIMAX, action_dtype, board, "ntuple_expectimax")
     if m == 0:
         return res
     act = res["action"].data_ptr()
@@ -386,15 +374,17 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
     return res
 
 
-def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, tuples, *, alpha: float,
-                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """One synchronous batch of TD(0) updates of an n-tuple network, in place on ``weights``; returns delta (M,) float32.
+def _coherence_args(coherence, accum, n: int, device) -> tuple[int, int]:
+    """checks of TC's ``coherence`` and ``accum``; returns their pointers"""
+    for name, t in (("coherence", coherence), ("accum", accum)):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float32
+                and tuple(t.shape) == (n, 2) and t.device == device):
+            raise ValueError(f"{name} must be a contiguous float32 ({n}, 2) tensor on {device}")
+    return coherence.data_ptr(), accum.data_ptr()
 
-    Phase 1: delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game
-    whose ``mask`` byte is 0 (``mask``: (M,) bool/uint8, None = every game).  Phase 2: every entry of every masked-in game,
-    8 per tuple, gets += delta_i.  Phase 2 adds with float atomics, so the order of the adds that several games make to one
-    entry is unspecified: the weights are reproducible only up to the fp32 rounding of that order.  delta is deterministic.
-    ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
+
+def _target_update(fn: str, afterstate, target, weights, tuples, alpha, mask, delta_out, tc=None) -> torch.Tensor:
+    """ntuple_td_update (tc None) and ntuple_tc_update (tc = (coherence, accum)) through library function ``fn``"""
     _board_arg(afterstate, "afterstate")
     m = afterstate.shape[0]
     _cuda(target, "target")
@@ -406,16 +396,29 @@ def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
             raise ValueError(f"mask must be bool/uint8 ({m},)")
     cells, lens, k, n = _spec_arrays(tuples)
     _weights_arg(weights, n, afterstate.device)
+    tc_ptrs = () if tc is None else _coherence_args(*tc, n, afterstate.device)
     delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
     if m == 0:
         return delta_out
     lib = _lib.load()
     with torch.cuda.device(afterstate.device):
-        rc = lib.ml2048_ntuple_td_update(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None,
-                                         float(alpha), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k,
-                                         delta_out.data_ptr(), m, _stream(afterstate))
-    _lib.check(rc, "ml2048_ntuple_td_update")
+        rc = getattr(lib, fn)(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None, float(alpha),
+                              weights.data_ptr(), *tc_ptrs, n, cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m,
+                              _stream(afterstate))
+    _lib.check(rc, fn)
     return delta_out
+
+
+def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, tuples, *, alpha: float,
+                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """One synchronous batch of TD(0) updates of an n-tuple network, in place on ``weights``; returns delta (M,) float32.
+
+    Phase 1: delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game
+    whose ``mask`` byte is 0 (``mask``: (M,) bool/uint8, None = every game).  Phase 2: every entry of every masked-in game,
+    8 per tuple, gets += delta_i.  Phase 2 adds with float atomics, so the order of the adds that several games make to one
+    entry is unspecified: the weights are reproducible only up to the fp32 rounding of that order.  delta is deterministic.
+    ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
+    return _target_update("ml2048_ntuple_td_update", afterstate, target, weights, tuples, alpha, mask, delta_out)
 
 
 def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, coherence: torch.Tensor,
@@ -439,38 +442,15 @@ def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
     older errors by the alpha they had.  ``coherence`` and ``accum``: contiguous float32 (N, 2) tensors on the weights'
     device; ``accum`` is scratch that must be all zero and is left all zero.  ``delta_out``: a preallocated (M,) float32
     tensor (CUDA-graph capture)."""
-    _board_arg(afterstate, "afterstate")
-    m = afterstate.shape[0]
-    _cuda(target, "target")
-    if target.dtype != torch.float32 or tuple(target.shape) != (m,):
-        raise ValueError(f"target must be float32 ({m},)")
-    if mask is not None:
-        _cuda(mask, "mask")
-        if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,):
-            raise ValueError(f"mask must be bool/uint8 ({m},)")
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, afterstate.device)
-    for name, t in (("coherence", coherence), ("accum", accum)):
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float32
-                and tuple(t.shape) == (n, 2) and t.device == afterstate.device):
-            raise ValueError(f"{name} must be a contiguous float32 ({n}, 2) tensor on {afterstate.device}")
-    delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
-    if m == 0:
-        return delta_out
-    lib = _lib.load()
-    with torch.cuda.device(afterstate.device):
-        rc = lib.ml2048_tc_update(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None,
-                                  float(alpha), weights.data_ptr(), coherence.data_ptr(), accum.data_ptr(), n, cells.ctypes.data,
-                                  lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(afterstate))
-    _lib.check(rc, "ml2048_tc_update")
-    return delta_out
+    return _target_update("ml2048_tc_update", afterstate, target, weights, tuples, alpha, mask, delta_out, (coherence, accum))
 
 
 NTUPLE_LAMBDA_MAX_HORIZON = 16
 
 
-def _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask) -> tuple[int, int, float]:
-    """checks of the ring, ``newest``, ``lam`` and ``mask`` shared by the two lambda updates; returns (h, M, lam)"""
+def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask, delta_out,
+                   tc=None) -> torch.Tensor:
+    """ntuple_td_lambda_update (tc None) and ntuple_tc_lambda_update (tc = (coherence, accum)) through library function ``fn``"""
     if not (isinstance(after_ring, torch.Tensor) and after_ring.dtype in (torch.uint8, torch.int8) and after_ring.ndim == 3
             and after_ring.shape[2] == 16):
         raise ValueError("after_ring must be uint8/int8 (h+1, M, 16)")
@@ -496,7 +476,19 @@ def _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask) -> tupl
         _cuda(mask, "mask")
         if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,) or mask.device != dev:
             raise ValueError(f"mask must be bool/uint8 ({m},) on {dev}")
-    return h, m, lam
+    cells, lens, k, n = _spec_arrays(tuples)
+    _weights_arg(weights, n, dev)
+    tc_ptrs = () if tc is None else _coherence_args(*tc, n, dev)
+    delta_out = _out_arg(delta_out, (m,), torch.float32, dev, "delta_out")
+    if m == 0:
+        return delta_out
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        rc = getattr(lib, fn)(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
+                              mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(), *tc_ptrs, n,
+                              cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(after_ring))
+    _lib.check(rc, fn)
+    return delta_out
 
 
 def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
@@ -521,19 +513,8 @@ def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor,
     (h+1, M) bool/uint8, all contiguous on one device, h = ``after_ring.shape[0] - 1`` in 1..16.  ``newest`` is the slot of
     x_h; x_k is in slot (newest - (h - k)) mod (h + 1), and ``ended_ring[newest]`` is not read.  ``mask``: (M,) bool/uint8,
     None = every game.  ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
-    h, m, lam = _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask)
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, after_ring.device)
-    delta_out = _out_arg(delta_out, (m,), torch.float32, after_ring.device, "delta_out")
-    if m == 0:
-        return delta_out
-    lib = _lib.load()
-    with torch.cuda.device(after_ring.device):
-        rc = lib.ml2048_lambda_td_update(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
-                                         mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(), n,
-                                         cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(after_ring))
-    _lib.check(rc, "ml2048_lambda_td_update")
-    return delta_out
+    return _lambda_update("ml2048_lambda_td_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask,
+                          delta_out)
 
 
 def ntuple_tc_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
@@ -545,21 +526,5 @@ def ntuple_tc_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor,
     entries is then ``ntuple_tc_update``'s phases 2 and 3: {dE, dA} += {delta, |delta|} into ``accum``, and w += beta * dE,
     beta = |E| / A (1 where A = 0), {E, A} += {dE, dA} for every entry with dA != 0.  ``coherence`` and ``accum``: contiguous
     float32 (N, 2) tensors on the ring's device; ``accum`` must be all zero and is left all zero."""
-    h, m, lam = _lambda_args(after_ring, reward_ring, ended_ring, newest, lam, mask)
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, after_ring.device)
-    for name, t in (("coherence", coherence), ("accum", accum)):
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and t.dtype == torch.float32
-                and tuple(t.shape) == (n, 2) and t.device == after_ring.device):
-            raise ValueError(f"{name} must be a contiguous float32 ({n}, 2) tensor on {after_ring.device}")
-    delta_out = _out_arg(delta_out, (m,), torch.float32, after_ring.device, "delta_out")
-    if m == 0:
-        return delta_out
-    lib = _lib.load()
-    with torch.cuda.device(after_ring.device):
-        rc = lib.ml2048_lambda_tc_update(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
-                                         mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(),
-                                         coherence.data_ptr(), accum.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k,
-                                         delta_out.data_ptr(), m, _stream(after_ring))
-    _lib.check(rc, "ml2048_lambda_tc_update")
-    return delta_out
+    return _lambda_update("ml2048_lambda_tc_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask,
+                          delta_out, (coherence, accum))

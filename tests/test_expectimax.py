@@ -21,24 +21,11 @@ import torch
 
 import _expectimax_ref as xref
 import _ntuple_ref as ref
+from _ntuple_gpu import _gpu, ops  # noqa: F401 (ops is a fixture)
 
 KINDS = ("normal", "improved", "rank", "maxcell")
 TWO_PROBS = (0.0, 0.3, 0.8, 1.0)
 CANARY = 0x5A5A5A5A
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from ml2048_b200 import _lib, build, ops
-
-    build.build()
-    _lib.load()
-    return ops
-
-
-def _gpu():
-    assert torch.cuda.is_available()
-    return torch.device("cuda")
 
 
 def _played_boards(m: int, steps: int, seed: int) -> np.ndarray:

@@ -24,23 +24,10 @@ import pytest
 import torch
 
 import _ntuple_ref as ref
+from _ntuple_gpu import _gpu, ops  # noqa: F401 (ops is a fixture)
 
 KINDS = ("normal", "improved", "rank", "maxcell")
 CANARY = 0x5A5A5A5A
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from ml2048_b200 import _lib, build, ops
-
-    build.build()
-    _lib.load()
-    return ops
-
-
-def _gpu():
-    assert torch.cuda.is_available()
-    return torch.device("cuda")
 
 
 def _boards(rng, m: int) -> np.ndarray:

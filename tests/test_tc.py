@@ -24,22 +24,9 @@ import torch
 
 import _ntuple_ref as nref
 import _tc_ref as ref
+from _ntuple_gpu import _gpu, ops  # noqa: F401 (ops is a fixture)
 
 CANARY = 0x5A5A5A5A
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from ml2048_b200 import _lib, build, ops
-
-    build.build()
-    _lib.load()
-    return ops
-
-
-def _gpu():
-    assert torch.cuda.is_available()
-    return torch.device("cuda")
 
 
 def _guarded(shape, dtype, dev, fill=None, pad: int = 64):

@@ -24,21 +24,8 @@ import torch
 import _lambda_ref as ref
 import _ntuple_ref as nref
 import _tc_ref as tref
+from _ntuple_gpu import _gpu, ops  # noqa: F401 (ops is a fixture)
 from test_tc import _coherence, _disjoint_rows, _guarded, _played_boards, _same_bits, _zero_bits
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from ml2048_b200 import _lib, build, ops
-
-    build.build()
-    _lib.load()
-    return ops
-
-
-def _gpu():
-    assert torch.cuda.is_available()
-    return torch.device("cuda")
 
 
 def _update(ops, rule, rings, newest, w_dev, c_dev, a_dev, tuples, **kw):
