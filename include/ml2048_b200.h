@@ -29,8 +29,9 @@ extern "C" {
 #endif
 
 /* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, ml2048_expectimax, ml2048_tc_update,
- * ml2048_lambda_td_update and ml2048_lambda_tc_update, added without a bump (unlike earlier additions): they change no existing
- * struct or signature, and a loader that binds them by name fails on a library without them. */
+ * ml2048_lambda_td_update, ml2048_lambda_tc_update and the seven ml2048_staged_* entries, added without a bump (unlike
+ * earlier additions): they change no existing struct or signature, and a loader that binds them by name fails on a library
+ * without them. */
 #define ML2048_ABI_VERSION 12
 
 #if defined(__GNUC__)
@@ -382,6 +383,44 @@ ML2048_API int ml2048_expectimax(const void *board, const float *weights, int64_
                                  int32_t num_tuples, int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8,
                                  int64_t *action_i64, void *after_out, float *reward_out, float *value_out, float *q_out, int64_t num_games,
                                  void *stream);
+
+/* multi-stage n-tuple networks (Yeh et al. 2016): one weight set per stage of the game, chosen by the board.  Each
+ * ml2048_staged_* entry is the n-tuple entry it names with `const uint8_t *stage_exp, int32_t num_stages` after num_tuples.
+ * S = num_stages (1..8) stages are given by the S - 1 strictly ascending tile exponents stage_exp[0] < ... < stage_exp[S-2],
+ * each in 1..15, a HOST array (may be null when S = 1).  m(b) = max over the 16 cells of min(b[c], 15), the index's own clamp;
+ * stage(b) = #{k : stage_exp[k] <= m(b)}: an empty board is in stage 0, a byte >= 16 counts as 15.  weights: S * N float32
+ * entries (N = sum_t 16^len[t]), stage s's tables at s * N in the single-stage layout; coherence and accum of the TC entries
+ * are [S * N][2], indexed like the weights.  V(b) = sum over t, g of weights[stage(b) * N + offset_t + idx_t,g(b)], float32
+ * adds from 0.0f in the single-stage order: greedy values each afterstate, expectimax each leaf and TD(lambda) each window
+ * board x_k with that board's own stage, and every update writes the entries of x_0's stage.  Everything else (deltas, tie
+ * and NaN rules, masks, the TC apply) is the single-stage entry's, word for word, and S = 1 is that entry bit for bit.
+ * E_NULL: stage_exp null with S > 1; E_SIZE: S outside 1..8 or num_weights != S * N; E_ENUM: a threshold outside 1..15 or
+ * the thresholds not strictly ascending.  Every other check is the single-stage entry's; all return before any launch. */
+ML2048_API int ml2048_staged_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                   int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, float *value_out, int64_t num_games,
+                                   void *stream);
+ML2048_API int ml2048_staged_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                    int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, uint8_t *action_u8,
+                                    int64_t *action_i64, void *after_out, float *reward_out, float *value_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_staged_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                       int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                       const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_staged_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                       float *coherence, float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                       int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games,
+                                       void *stream);
+ML2048_API int ml2048_staged_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                              int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights,
+                                              int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                              const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_staged_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                              int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                              float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                              const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_staged_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells,
+                                        const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind,
+                                        int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                                        float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream);
 
 /* _update_count (runner.py:120-136): hist[max exponent] += 1 for every game with terminated != 0;
  * with terminated == null: VecGame.summary's histogram over all live boards (game_numba.py:593-596).

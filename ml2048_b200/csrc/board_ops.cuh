@@ -768,9 +768,80 @@ ML2048_FN float load_weight(const float *p) { return __ldg(p); }
 ML2048_FN float load_weight(const float *p) { return *p; }
 #endif
 
+// ---- multi-stage n-tuple networks ----
+// S (1..8) weight sets, one per stage of the game, given by S - 1 strictly ascending tile exponents tau_1 < ... < tau_{S-1} in
+// 1..15.  m(b) = max over the 16 cells of min(b[c], 15) (the index's own clamp), stage(b) = #{k : tau_k <= m(b)}: an empty
+// board is in stage 0, a byte >= 16 counts as 15.  The weights are S * N entries (N = sum_t 16^len_t), stage s's tables at
+// s * N in the single-stage layout; every entry index s * N + offset_t + idx < 8 * 2^28 fits in 32 bits.  A board's value and
+// every update use the tables of the board's own stage.  NTupleSpec itself stays the single-stage network (S = 1 runs the
+// kernels' NTupleSpec instances); the staged spec extends it, so that the parameters of the existing kernels keep their offsets.
+constexpr int kNTupleMaxStages = 8;
+
+struct NTupleStagedSpec : NTupleSpec {
+    uint32_t stage_size;  // N
+    uint64_t stage_of;    // bits 4m..4m+3: the stage of a board whose largest clamped cell is m
+};
+
+// Host side: the stage table of validated thresholds (tau [S-1], ascending in 1..15)
+inline uint64_t ntuple_stage_table(const uint8_t *tau, int32_t num_stages)
+{
+    uint64_t t = 0;
+    for (uint32_t m = 0; m < 16u; ++m) {
+        uint64_t s = 0;
+        for (int k = 0; k + 1 < num_stages; ++k) s += tau[k] <= m ? 1u : 0u;
+        t |= s << (4u * m);
+    }
+    return t;
+}
+
+// the largest of the 4 bytes of x, in byte 0
+#if defined(__CUDACC__)
+ML2048_FN uint32_t max_byte(uint32_t x)
+{
+    x = __vmaxu4(x, x >> 16);
+    return __vmaxu4(x, x >> 8) & 0xffu;
+}
+ML2048_FN uint32_t max_bytes(uint32_t x, uint32_t y) { return __vmaxu4(x, y); }
+#else
+ML2048_FN uint32_t max_byte(uint32_t x)
+{
+    uint32_t m = 0;
+    for (int i = 0; i < 4; ++i) m = ((x >> (8 * i)) & 0xffu) > m ? (x >> (8 * i)) & 0xffu : m;
+    return m;
+}
+ML2048_FN uint32_t max_bytes(uint32_t x, uint32_t y)
+{
+    uint32_t d = 0;
+    for (int i = 0; i < 4; ++i) {
+        const uint32_t a = (x >> (8 * i)) & 0xffu, b = (y >> (8 * i)) & 0xffu;
+        d |= (a > b ? a : b) << (8 * i);
+    }
+    return d;
+}
+#endif
+
+// stage(b) from the board's clamped nibbles: the 16 fields split into two words of byte lanes, a byte-wise max, one shift of
+// the stage table
+ML2048_FN uint32_t ntuple_stage(const NTupleStagedSpec &s, uint64_t nib)
+{
+    const uint32_t lo = (uint32_t)nib, hi = (uint32_t)(nib >> 32);
+    const uint32_t m = max_byte(max_bytes(max_bytes(lo & 0x0f0f0f0fu, (lo >> 4) & 0x0f0f0f0fu),
+                                          max_bytes(hi & 0x0f0f0f0fu, (hi >> 4) & 0x0f0f0f0fu)));
+    return (uint32_t)(s.stage_of >> (4u * m)) & 15u;
+}
+
+// The staged visitor: ntuple_for_each_entry over the tables of the board's stage (offset + stage(b) * N)
+template <class Visit>
+ML2048_FN void ntuple_for_each_entry(const NTupleStagedSpec &s, uint64_t nib, Visit &&visit)
+{
+    const uint32_t base = ntuple_stage(s, nib) * s.stage_size;
+    ntuple_for_each_entry(static_cast<const NTupleSpec &>(s), nib, [&](uint32_t off, uint32_t idx) { visit(base + off, idx); });
+}
+
 // V(s): float32 adds from 0.0f in the fixed order t = 0..K-1, g = 0..7 -- bit-reproducible, and a sequential float32 reference
-// matches it exactly
-ML2048_FN float ntuple_value(const float *w, const NTupleSpec &s, uint64_t nib)
+// matches it exactly.  Spec = NTupleSpec, or NTupleStagedSpec (the tables of the board's stage).
+template <class Spec>
+ML2048_FN float ntuple_value(const float *w, const Spec &s, uint64_t nib)
 {
     float acc = 0.0f;
     ntuple_for_each_entry(s, nib, [&](uint32_t off, uint32_t idx) { acc += load_weight(w + off + idx); });

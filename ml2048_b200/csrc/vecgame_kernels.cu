@@ -1451,9 +1451,16 @@ __global__ void __launch_bounds__(kStepThreads) afterstates_kernel(const uint4 *
 // Value, greedy afterstate move and TD(0) update of an n-tuple network (board_ops.cuh: NTupleSpec, ntuple_value).  The spec is
 // a by-value __grid_constant__ parameter: the kernels index it in the constant bank, nothing is copied to local memory.
 // Board offsets are 64-bit (16 * game passes 2^31 at 2^27 games); table entry indices stay below 2^28.
+// Every n-tuple kernel below is a template over the spec: Spec = NTupleSpec is the single-stage network, Spec =
+// NTupleStagedSpec the multi-stage one (board_ops.cuh: one weight set per stage, stage(b) = #{k : tau_k <= max_c min(b[c], 15)},
+// stage s's tables at s * N; indices below 8 * 2^28).  The staged visitor adds stage(b) * N to every offset it reports, so
+// a board's value, greedy's afterstates, expectimax's leaves and the lambda window's boards each use their own stage's tables,
+// and the updates (scatter, TC accumulate and apply, whose claim is on j = off + idx) write the entries of x_0's stage.  One
+// stage launches the NTupleSpec instances (with_spec below).
 
 // one thread per board
-__global__ void __launch_bounds__(kStepThreads) ntuple_value_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+template <class Spec>
+__global__ void __launch_bounds__(kStepThreads) ntuple_value_kernel(const uint4 *board, const float *w, __grid_constant__ const Spec spec,
                                                                     float *value, int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
@@ -1467,7 +1474,8 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_value_kernel(const uint4 
 // four lanes pick the move with a shuffle argmax -- no afterstate goes to memory.  q = reward + V(afterstate) for a direction
 // that changes the board; NaN ranks as -inf; the largest q wins, ties go to the smallest direction.  A board without a valid
 // direction gets action 0 and its own board, reward 0, value 0.  The lane of the chosen direction writes the outputs.
-__global__ void __launch_bounds__(kStepThreads) ntuple_greedy_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+template <class Spec>
+__global__ void __launch_bounds__(kStepThreads) ntuple_greedy_kernel(const uint4 *board, const float *w, __grid_constant__ const Spec spec,
                                                                      int32_t reward_kind, uint8_t *action_u8, long long *action_i64,
                                                                      uint4 *after, float *reward, float *value, int64_t num_games)
 {
@@ -1506,8 +1514,9 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_greedy_kernel(const uint4
 
 // TD(0), phase 1: delta = alpha * (target - V(afterstate)) for every masked-in game with the weights as they were before the
 // update (phase 2 runs as a second launch); 0 for a masked-out game
+template <class Spec>
 __global__ void __launch_bounds__(kStepThreads) ntuple_td_delta_kernel(const uint4 *after, const float *target, const uint8_t *mask, float alpha,
-                                                                       const float *w, __grid_constant__ const NTupleSpec spec, float *delta,
+                                                                       const float *w, __grid_constant__ const Spec spec, float *delta,
                                                                        int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
@@ -1523,8 +1532,9 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_td_delta_kernel(const uin
 // TD(0), phase 2: w[entry] += delta for every masked-in game, tuple and image.  Float atomics (RED.ADD.F32): the order of the
 // adds that different games make to one entry is unspecified, so the weights are reproducible up to the fp32 rounding of
 // that order.
+template <class Spec>
 __global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const uint4 *after, const uint8_t *mask, const float *delta, float *w,
-                                                                         __grid_constant__ const NTupleSpec spec, int64_t num_games)
+                                                                         __grid_constant__ const Spec spec, int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
     if (i >= num_games || (mask && !mask[i])) return;
@@ -1549,8 +1559,9 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_td_scatter_kernel(const u
 // return.  Cost O(batch): phase 3 walks the batch's own entries, never the table.
 
 // TC, phase 2: one 8-byte vector atomic (RED.E.ADD.F32x2) per lookup into the interleaved {dE, dA} accumulator
+template <class Spec>
 __global__ void __launch_bounds__(kStepThreads) ntuple_tc_accumulate_kernel(const uint4 *after, const uint8_t *mask, const float *delta,
-                                                                            float2 *acc, __grid_constant__ const NTupleSpec spec,
+                                                                            float2 *acc, __grid_constant__ const Spec spec,
                                                                             int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
@@ -1568,8 +1579,9 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_tc_accumulate_kernel(cons
 // shared by thousands of games): the word only goes from non-zero to zero during this launch, so a zero read is final and a
 // stale non-zero read costs one exchange that returns 0.  The whole word is tested, not only dA, so that a -0 left in dE is
 // still cleared.  -DML2048_TC_APPLY_ALWAYS_EXCHANGE builds the variant without the load (tools/tc_bench.py times both).
+template <class Spec>
 __global__ void __launch_bounds__(kStepThreads) ntuple_tc_apply_kernel(const uint4 *after, const uint8_t *mask, float *w, float2 *coh,
-                                                                       unsigned long long *acc, __grid_constant__ const NTupleSpec spec,
+                                                                       unsigned long long *acc, __grid_constant__ const Spec spec,
                                                                        int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
@@ -1608,10 +1620,11 @@ constexpr int kLambdaMaxHorizon = 16;
 
 // one thread per game: the first end in the window fixes where the recursion starts, so the values after it are never
 // looked up (they would be multiplied away by the 0 anyway, and skipping them changes no bit)
+template <class Spec>
 __global__ void __launch_bounds__(kStepThreads) ntuple_lambda_delta_kernel(const uint4 *after, const float *reward, const uint8_t *ended,
                                                                            const uint8_t *mask, int32_t horizon, int32_t newest, float lf,
                                                                            float c, float alpha, const float *w,
-                                                                           __grid_constant__ const NTupleSpec spec, float *delta,
+                                                                           __grid_constant__ const Spec spec, float *delta,
                                                                            int64_t num_games)
 {
     const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
@@ -1686,7 +1699,8 @@ struct SpawnLaw {
 // E(s, 1) of an afterstate s that the whole warp holds (warp-uniform call; n >= 1 empty cells).  A pass covers 8 outcomes x
 // 4 inner directions: lane = 4 * outcome + direction, the move, reward and value in registers, M by lane4_argmax.  Every
 // lane then reads the pass's 8 M values by shuffle and adds the terms in ascending cell order, so all lanes return E.
-__device__ __forceinline__ float chance1(uint4 s, const float *w, const NTupleSpec &spec, int32_t reward_kind, SpawnLaw law)
+template <class Spec>
+__device__ __forceinline__ float chance1(uint4 s, const float *w, const Spec &spec, int32_t reward_kind, SpawnLaw law)
 {
     const uint32_t lane = threadIdx.x & 31u, a = lane & 3u;
     const uint32_t empties = empty_cells(s), n = popc32(empties);
@@ -1765,7 +1779,8 @@ constexpr int kExpectimax1BoardsPerBlock = kExpectimaxThreads / 128;
 
 // Depth 1, one warp per (board, root direction): warp w of a block takes board 2 * block + w / 4, direction w & 3, and
 // computes E(after, 1) with chance1; lanes 0..7 of warp 0 then pick both boards' moves from shared memory.
-__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+template <class Spec>
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const Spec spec,
                                                                          int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
                                                                          long long *action_i64, uint4 *after, float *reward,
                                                                          float *value, float *q_out, int64_t num_games)
@@ -1793,7 +1808,8 @@ constexpr int kExpectimax1BoardsPerBlock = kExpectimaxThreads / 32;
 
 // Depth 1, one warp per board (the alternative mapping; profiles/expectimax_bench.txt): the warp computes E(after(b,a), 1)
 // for a = 0..3 in turn, lane group 0 picks the move.  No shared memory, no barrier.
-__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+template <class Spec>
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const uint4 *board, const float *w, __grid_constant__ const Spec spec,
                                                                          int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
                                                                          long long *action_i64, uint4 *after, float *reward,
                                                                          float *value, float *q_out, int64_t num_games)
@@ -1819,7 +1835,8 @@ __global__ void __launch_bounds__(kExpectimaxThreads) expectimax1_kernel(const u
 // 0 then folds them, in the definition's fixed order, into M, t_c, S and E for each root direction and picks the move.
 constexpr int kExpectimax2Nodes = 4 * 2 * 15 * 4;
 
-__global__ void __launch_bounds__(kExpectimaxThreads) expectimax2_kernel(const uint4 *board, const float *w, __grid_constant__ const NTupleSpec spec,
+template <class Spec>
+__global__ void __launch_bounds__(kExpectimaxThreads) expectimax2_kernel(const uint4 *board, const float *w, __grid_constant__ const Spec spec,
                                                                          int32_t reward_kind, SpawnLaw law, uint8_t *action_u8,
                                                                          long long *action_i64, uint4 *after, float *reward,
                                                                          float *value, float *q_out)
@@ -1914,9 +1931,12 @@ inline int launch_status()
     return e == cudaSuccess ? 0 : (int)e;
 }
 
-// Check an n-tuple network given as host arrays (cells [K][6], len [K]) and expand it into the kernels' NTupleSpec: E_NULL,
-// E_SIZE for K or a length out of range or a weight count other than sum 16^len, E_ENUM for a cell > 15 or a repeated cell
-inline int ntuple_spec(const uint8_t *cells, const uint8_t *len, int32_t num_tuples, int64_t num_weights, NTupleSpec &spec)
+// Check an n-tuple network given as host arrays (cells [K][6], len [K], stage thresholds stage_exp [S-1]) and expand it into
+// the kernels' NTupleStagedSpec: E_NULL (stage_exp only when S > 1), E_SIZE for K, a length or S out of range or a weight
+// count other than S * sum 16^len, E_ENUM for a cell > 15, a repeated cell, or thresholds outside 1..15 or not strictly
+// ascending
+inline int ntuple_spec(const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                       int64_t num_weights, NTupleStagedSpec &spec)
 {
     if (!cells || !len) return ML2048_E_NULL;
     if (num_tuples < 1 || num_tuples > kNTupleMaxTuples) return ML2048_E_SIZE;
@@ -1929,7 +1949,24 @@ inline int ntuple_spec(const uint8_t *cells, const uint8_t *len, int32_t num_tup
             seen |= 1u << c;
         }
     }
-    return ntuple_expand(cells, len, num_tuples, spec) == num_weights ? 0 : ML2048_E_SIZE;
+    if (num_stages < 1 || num_stages > kNTupleMaxStages) return ML2048_E_SIZE;
+    if (num_stages > 1 && !stage_exp) return ML2048_E_NULL;
+    for (int k = 0; k + 1 < num_stages; ++k)
+        if (stage_exp[k] < 1 || stage_exp[k] > 15 || (k > 0 && stage_exp[k] <= stage_exp[k - 1])) return ML2048_E_ENUM;
+    const int64_t n = ntuple_expand(cells, len, num_tuples, spec);
+    spec.stage_size = (uint32_t)n;
+    spec.stage_of = ntuple_stage_table(stage_exp, num_stages);
+    return n * num_stages == num_weights ? 0 : ML2048_E_SIZE;
+}
+
+// Runs f(spec) with the spec's single-stage NTupleSpec for a one-stage network (its stage table is all zero: a threshold
+// <= 15 puts the board of largest cell 15 in stage >= 1), so S = 1 launches the NTupleSpec instances of the kernels; with
+// the staged spec otherwise.  f launches the kernels, templated on the spec type it is given.
+template <class F>
+inline int with_spec(const NTupleStagedSpec &spec, F &&f)
+{
+    if (spec.stage_of == 0) return f(static_cast<const NTupleSpec &>(spec));
+    return f(spec);
 }
 
 constexpr int kMaxDevices = 64;
@@ -2379,25 +2416,34 @@ int ml2048_afterstates(const void *board, void *after_out, float *reward_out, ui
     return launch_status();
 }
 
-int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
-                        int32_t num_tuples, float *value_out, int64_t num_games, void *stream)
+int ml2048_staged_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                        int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, float *value_out, int64_t num_games,
+                        void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || !value_out) return ML2048_E_NULL;
     if (misaligned(board, 16) || misaligned(weights, 4) || misaligned(value_out, 4)) return ML2048_E_ALIGN;
-    NTupleSpec spec;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    NTupleStagedSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, stage_exp, num_stages, num_weights, spec)) return rc;
     const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
     if (grid > 0x7fffffff) return ML2048_E_SIZE;
     clear_stale_error();
-    ntuple_value_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4 *>(board), weights,
-                                                                                             spec, value_out, num_games);
-    return launch_status();
+    return with_spec(spec, [&](const auto &sp) {
+        ntuple_value_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4 *>(board),
+                                                                                                 weights, sp, value_out, num_games);
+        return launch_status();
+    });
 }
 
-int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
-                         int32_t num_tuples, int32_t reward_kind, uint8_t *action_u8, int64_t *action_i64, void *after_out,
-                         float *reward_out, float *value_out, int64_t num_games, void *stream)
+int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                        int32_t num_tuples, float *value_out, int64_t num_games, void *stream)
+{
+    return ml2048_staged_value(board, weights, num_weights, cells, len, num_tuples, nullptr, 1, value_out, num_games, stream);
+}
+
+int ml2048_staged_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                         int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, uint8_t *action_u8,
+                         int64_t *action_i64, void *after_out, float *reward_out, float *value_out, int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out) return ML2048_E_NULL;
@@ -2405,20 +2451,31 @@ int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_we
         misaligned(reward_out, 4) || misaligned(value_out, 4))
         return ML2048_E_ALIGN;
     if (reward_kind < 0 || reward_kind > ML2048_REWARD_MAXCELL) return ML2048_E_ENUM;
-    NTupleSpec spec;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    NTupleStagedSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, stage_exp, num_stages, num_weights, spec)) return rc;
     const int64_t grid = (num_games + kStepThreads / 4 - 1) / (kStepThreads / 4);  // four threads per game
     if (grid > 0x7fffffff) return ML2048_E_SIZE;
     clear_stale_error();
-    ntuple_greedy_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-        reinterpret_cast<const uint4 *>(board), weights, spec, reward_kind, action_u8, reinterpret_cast<long long *>(action_i64),
-        reinterpret_cast<uint4 *>(after_out), reward_out, value_out, num_games);
-    return launch_status();
+    return with_spec(spec, [&](const auto &sp) {
+        ntuple_greedy_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+            reinterpret_cast<const uint4 *>(board), weights, sp, reward_kind, action_u8, reinterpret_cast<long long *>(action_i64),
+            reinterpret_cast<uint4 *>(after_out), reward_out, value_out, num_games);
+        return launch_status();
+    });
 }
 
-int ml2048_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
-                      int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out,
-                      float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream)
+int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                         int32_t num_tuples, int32_t reward_kind, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                         float *reward_out, float *value_out, int64_t num_games, void *stream)
+{
+    return ml2048_staged_greedy(board, weights, num_weights, cells, len, num_tuples, nullptr, 1, reward_kind, action_u8, action_i64,
+                                after_out, reward_out, value_out, num_games, stream);
+}
+
+int ml2048_staged_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                             int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, int32_t depth,
+                             double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out, float *reward_out,
+                             float *value_out, float *q_out, int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out || !q_out) return ML2048_E_NULL;
@@ -2427,8 +2484,8 @@ int ml2048_expectimax(const void *board, const float *weights, int64_t num_weigh
         return ML2048_E_ALIGN;
     if (reward_kind < 0 || reward_kind > ML2048_REWARD_MAXCELL || (depth != 1 && depth != 2) || !(two_prob >= 0.0 && two_prob <= 1.0))
         return ML2048_E_ENUM;
-    NTupleSpec spec;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    NTupleStagedSpec spec;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, stage_exp, num_stages, num_weights, spec)) return rc;
     SpawnLaw law;
     law.p2 = (float)two_prob;
     law.p4 = 1.0f - law.p2;
@@ -2440,25 +2497,36 @@ int ml2048_expectimax(const void *board, const float *weights, int64_t num_weigh
     uint4 *after = reinterpret_cast<uint4 *>(after_out);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     clear_stale_error();
-    if (depth == 1)
-        expectimax1_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, spec, reward_kind, law, action_u8, a64, after, reward_out,
-                                                                         value_out, q_out, num_games);
-    else
-        expectimax2_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, spec, reward_kind, law, action_u8, a64, after, reward_out,
-                                                                         value_out, q_out);
-    return launch_status();
+    return with_spec(spec, [&](const auto &sp) {
+        if (depth == 1)
+            expectimax1_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, sp, reward_kind, law, action_u8, a64, after,
+                                                                             reward_out, value_out, q_out, num_games);
+        else
+            expectimax2_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, sp, reward_kind, law, action_u8, a64, after,
+                                                                             reward_out, value_out, q_out);
+        return launch_status();
+    });
+}
+
+int ml2048_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                      int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                      float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream)
+{
+    return ml2048_staged_expectimax(board, weights, num_weights, cells, len, num_tuples, nullptr, 1, reward_kind, depth, two_prob, action_u8,
+                                    action_i64, after_out, reward_out, value_out, q_out, num_games, stream);
 }
 
 // Checks every n-tuple update shares: the batch, the afterstates (x_0's, or the ring that holds them), the float32 values the
-// delta starts from (the target, or the reward ring), the weights, the delta output and the network.  On success `spec` and
-// `grid` (one thread per game) are ready for the launches.
+// delta starts from (the target, or the reward ring), the weights, the delta output and the network with its stages.  On
+// success `spec` and `grid` (one thread per game) are ready for the launches.
 static int check_update(const void *after, const float *values, const float *weights, const float *delta_out, int64_t num_weights,
-                        const uint8_t *cells, const uint8_t *len, int32_t num_tuples, int64_t num_games, NTupleSpec &spec, unsigned &grid)
+                        const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                        int64_t num_games, NTupleStagedSpec &spec, unsigned &grid)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!after || !values || !weights || !delta_out) return ML2048_E_NULL;
     if (misaligned(after, 16) || misaligned(values, 4) || misaligned(weights, 4) || misaligned(delta_out, 4)) return ML2048_E_ALIGN;
-    if (const int rc = ntuple_spec(cells, len, num_tuples, num_weights, spec)) return rc;
+    if (const int rc = ntuple_spec(cells, len, num_tuples, stage_exp, num_stages, num_weights, spec)) return rc;
     const int64_t blocks = (num_games + kStepThreads - 1) / kStepThreads;
     if (blocks > 0x7fffffff) return ML2048_E_SIZE;
     grid = (unsigned)blocks;
@@ -2467,17 +2535,19 @@ static int check_update(const void *after, const float *values, const float *wei
 
 // Phase 1 of TD(0) and TC: delta = alpha * (target - V(after))
 static int target_delta(const uint4 *after, const float *target, const uint8_t *mask, float alpha, const float *weights,
-                        const NTupleSpec &spec, float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s)
+                        const NTupleStagedSpec &spec, float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s)
 {
     clear_stale_error();
-    ntuple_td_delta_kernel<<<grid, kStepThreads, 0, s>>>(after, target, mask, alpha, weights, spec, delta_out, num_games);
-    return launch_status();
+    return with_spec(spec, [&](const auto &sp) {
+        ntuple_td_delta_kernel<<<grid, kStepThreads, 0, s>>>(after, target, mask, alpha, weights, sp, delta_out, num_games);
+        return launch_status();
+    });
 }
 
 // Phase 1 of TD(lambda) and TC(lambda): the checks only they make, then delta over the ring.  `x0` = x_0's slot of the ring.
 static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
-                        float lambda, const uint8_t *mask, float alpha, const float *weights, const NTupleSpec &spec, float *delta_out,
-                        unsigned grid, int64_t num_games, cudaStream_t s, const uint4 *&x0)
+                        float lambda, const uint8_t *mask, float alpha, const float *weights, const NTupleStagedSpec &spec,
+                        float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s, const uint4 *&x0)
 {
     if (!ended_ring) return ML2048_E_NULL;
     if (horizon < 1 || horizon > kLambdaMaxHorizon || newest < 0 || newest > horizon) return ML2048_E_SIZE;
@@ -2485,62 +2555,88 @@ static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8
     x0 = ring + (int64_t)(newest == horizon ? 0 : newest + 1) * num_games;
     const float c = 1.0f - lambda;
     clear_stale_error();
-    ntuple_lambda_delta_kernel<<<grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha, weights,
-                                                             spec, delta_out, num_games);
-    return launch_status();
+    return with_spec(spec, [&](const auto &sp) {
+        ntuple_lambda_delta_kernel<<<grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha,
+                                                                 weights, sp, delta_out, num_games);
+        return launch_status();
+    });
 }
 
 // The update of x_0's entries after phase 1, on the same stream (so every delta is computed before any weight is written):
-// TD(0)'s scatter when `coherence` is null, else TC's phases 2 and 3
+// TD(0)'s scatter when `coherence` is null, else TC's phases 2 and 3.  The entries are those of x_0's stage.
 static int apply_update(const uint4 *x0, const uint8_t *mask, const float *delta, float *weights, float *coherence, float *accum,
-                        const NTupleSpec &spec, unsigned grid, int64_t num_games, cudaStream_t s)
+                        const NTupleStagedSpec &spec, unsigned grid, int64_t num_games, cudaStream_t s)
 {
-    if (!coherence) {
-        ntuple_td_scatter_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, weights, spec, num_games);
+    return with_spec(spec, [&](const auto &sp) {
+        if (!coherence) {
+            ntuple_td_scatter_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, weights, sp, num_games);
+            return launch_status();
+        }
+        ntuple_tc_accumulate_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, reinterpret_cast<float2 *>(accum), sp, num_games);
+        if (const int rc = launch_status()) return rc;
+        ntuple_tc_apply_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
+                                                             reinterpret_cast<unsigned long long *>(accum), sp, num_games);
         return launch_status();
-    }
-    ntuple_tc_accumulate_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, reinterpret_cast<float2 *>(accum), spec, num_games);
-    if (const int rc = launch_status()) return rc;
-    ntuple_tc_apply_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
-                                                         reinterpret_cast<unsigned long long *>(accum), spec, num_games);
-    return launch_status();
+    });
 }
 
-int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
-                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+int ml2048_staged_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                            float *delta_out, int64_t num_games, void *stream)
 {
-    NTupleSpec spec;
+    NTupleStagedSpec spec;
     unsigned grid = 0;
-    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid)) return rc;
+    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, stage_exp, num_stages, num_games,
+                                    spec, grid))
+        return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
     return apply_update(b, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
 }
 
-int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
-                     float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
-                     int64_t num_games, void *stream)
+int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+{
+    return ml2048_staged_td_update(after, target, mask, alpha, weights, num_weights, cells, len, num_tuples, nullptr, 1, delta_out, num_games,
+                                   stream);
+}
+
+int ml2048_staged_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                            float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                            const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!coherence || !accum) return ML2048_E_NULL;
     if (misaligned(coherence, 8) || misaligned(accum, 8)) return ML2048_E_ALIGN;
-    NTupleSpec spec;
+    NTupleStagedSpec spec;
     unsigned grid = 0;
-    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid)) return rc;
+    if (const int rc = check_update(after, target, weights, delta_out, num_weights, cells, len, num_tuples, stage_exp, num_stages, num_games,
+                                    spec, grid))
+        return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
     return apply_update(b, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
 }
 
-int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
-                            float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights, const uint8_t *cells,
-                            const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                     float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
+                     int64_t num_games, void *stream)
 {
-    NTupleSpec spec;
+    return ml2048_staged_tc_update(after, target, mask, alpha, weights, coherence, accum, num_weights, cells, len, num_tuples, nullptr, 1,
+                                   delta_out, num_games, stream);
+}
+
+int ml2048_staged_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                                   const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
+                                   int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+{
+    NTupleStagedSpec spec;
     unsigned grid = 0;
-    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid))
+    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, stage_exp, num_stages,
+                                    num_games, spec, grid))
         return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint4 *x0 = nullptr;
@@ -2550,17 +2646,26 @@ int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, co
     return apply_update(x0, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
 }
 
-int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
-                            float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence, float *accum,
-                            int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
-                            int64_t num_games, void *stream)
+int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                            float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights, const uint8_t *cells,
+                            const uint8_t *len, int32_t num_tuples, float *delta_out, int64_t num_games, void *stream)
+{
+    return ml2048_staged_lambda_td_update(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights,
+                                          cells, len, num_tuples, nullptr, 1, delta_out, num_games, stream);
+}
+
+int ml2048_staged_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                   float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                   const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!coherence || !accum) return ML2048_E_NULL;
     if (misaligned(coherence, 8) || misaligned(accum, 8)) return ML2048_E_ALIGN;
-    NTupleSpec spec;
+    NTupleStagedSpec spec;
     unsigned grid = 0;
-    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, num_games, spec, grid))
+    if (const int rc = check_update(after_ring, reward_ring, weights, delta_out, num_weights, cells, len, num_tuples, stage_exp, num_stages,
+                                    num_games, spec, grid))
         return rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint4 *x0 = nullptr;
@@ -2568,6 +2673,15 @@ int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, co
                                     weights, spec, delta_out, grid, num_games, s, x0))
         return rc;
     return apply_update(x0, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
+}
+
+int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
+                            float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence, float *accum,
+                            int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, float *delta_out,
+                            int64_t num_games, void *stream)
+{
+    return ml2048_staged_lambda_tc_update(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, coherence, accum,
+                                          num_weights, cells, len, num_tuples, nullptr, 1, delta_out, num_games, stream);
 }
 
 int ml2048_pack_flags(const void *valid, const uint8_t *terminated, const uint8_t *invalid, uint8_t *packed, int64_t num_games, void *stream)

@@ -6,7 +6,8 @@ choosing the greedy afterstate move with it and updating it are integer byte wor
 adds: each is one kernel here (``ops.ntuple_value``, ``ops.ntuple_greedy``, ``ops.ntuple_td_update``; temporal coherence
 learning, a step size per weight, is ``ops.ntuple_tc_update`` and ``TDAfterstateLearner(..., rule="tc")``; their delayed
 lambda-return forms are ``ops.ntuple_td_lambda_update`` / ``ntuple_tc_lambda_update`` and ``TDAfterstateLearner(...,
-horizon=h, lam=lam)``).
+horizon=h, lam=lam)``).  ``NTupleNetwork(..., stages=(tau_1, ...))`` is a multi-stage network (Yeh et al. 2016): one weight
+set per stage of the game, chosen by the board's largest tile (``ops.ntuple_stages``).
 
     net = NTupleNetwork(device="cuda")                        # the standard 4x6 network, zero weights (256 MiB)
     env = VecGame(16384, output="torch", sync_free=True)
@@ -33,7 +34,9 @@ STANDARD_4X6 = ((0, 1, 2, 3, 4, 5), (4, 5, 6, 7, 8, 9), (0, 1, 2, 4, 5, 6), (4, 
 # with M: a fixed alpha that learns at one batch size diverges to NaN at a larger one.  tools/ntuple_bench.py swept
 # alpha = c / M for c = 0.1 ... 3.2 at M = 4096, 2^14 and 2^16, 30 000 steps each (profiles/ntuple_bench.txt, B200): the
 # results depend on c alone, not on M (mean score 9.8k / 11.7k / 14.4k / 5.5k / 2.2k / 1.6-2.2k for c = 0.1 / 0.2 / 0.4 /
-# 0.8 / 1.6 / 3.2 at all three sizes), and c = 0.4 is the best of them.
+# 0.8 / 1.6 / 3.2 at all three sizes), and c = 0.4 is the best of them.  Every default step size in this module was swept for
+# single-stage networks only: no sweep has been run for multi-stage ones (NTupleNetwork(stages=...)), which use the same
+# defaults.
 DEFAULT_ALPHA_TIMES_GAMES = 0.4
 
 
@@ -64,10 +67,16 @@ class NTupleNetwork:
     """An n-tuple value function with its weights on one CUDA device.
 
     ``tuples``: 1..16 tuples of 1..6 distinct cells (cell = row*4 + col).  The weights are one zero-initialised float32 tensor
-    of sum 16^len entries, tuple t's table after those of the tuples before it (``offsets``)."""
+    of sum 16^len entries, tuple t's table after those of the tuples before it (``offsets``).
 
-    def __init__(self, tuples=STANDARD_4X6, device: Any = None):
+    ``stages``: 0..7 strictly ascending tile exponents tau_1 < ... in 1..15 (``ops.ntuple_stages``) make a multi-stage network
+    of S = len(stages) + 1 weight sets.  A board b is in stage #{k : tau_k <= max_c min(b[c], 15)}, and is valued and updated
+    with that stage's tables; the weights are S * N entries, stage s's tables at s * N (N = sum 16^len), and ``coherence``
+    is (S * N, 2).  ``stages=()`` is the single-stage network."""
+
+    def __init__(self, tuples=STANDARD_4X6, device: Any = None, *, stages=()):
         self.tuples = ops.ntuple_spec(tuples)
+        self.stages = ops.ntuple_stages(stages)
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device={device!r}: ml2048_b200 runs on CUDA only")
@@ -79,32 +88,34 @@ class NTupleNetwork:
         for t in self.tuples:
             self.offsets.append(total)
             total += 16 ** len(t)
-        self.weights = torch.zeros((total,), dtype=torch.float32, device=dev)
+        self.weights = torch.zeros(((len(self.stages) + 1) * total,), dtype=torch.float32, device=dev)
         # TC learning's {E, A} per weight and the TC updates' scratch (all zero between calls), allocated by the first TC update
         self.coherence: Optional[torch.Tensor] = None
         self._tc_accum: Optional[torch.Tensor] = None
 
     def value(self, board: torch.Tensor, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """V of (M,16) boards: (M,) float32 (``ops.ntuple_value``)."""
-        return ops.ntuple_value(board, self.weights, self.tuples, out=out)
+        return ops.ntuple_value(board, self.weights, self.tuples, out=out, stages=self.stages)
 
     def greedy(self, board: torch.Tensor, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
                out: Optional[dict] = None) -> dict:
         """The move maximising reward + V(afterstate): {"action", "state", "reward", "value"} (``ops.ntuple_greedy``)."""
-        return ops.ntuple_greedy(board, self.weights, self.tuples, reward_fn=reward_fn, action_dtype=action_dtype, out=out)
+        return ops.ntuple_greedy(board, self.weights, self.tuples, reward_fn=reward_fn, action_dtype=action_dtype, out=out,
+                                 stages=self.stages)
 
     def expectimax(self, board: torch.Tensor, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
                    action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None) -> dict:
         """The expectimax move ``depth`` (1 or 2) chance layers deep: {"action", "state", "reward", "value", "q"}
         (``ops.ntuple_expectimax``)."""
         return ops.ntuple_expectimax(board, self.weights, self.tuples, depth=depth, two_prob=two_prob, reward_fn=reward_fn,
-                                     action_dtype=action_dtype, out=out)
+                                     action_dtype=action_dtype, out=out, stages=self.stages)
 
     def td_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
                   delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One synchronous TD(0) batch toward ``target``; returns delta = alpha * (target - V) (``ops.ntuple_td_update``).
         The adds are float atomics: the weights are reproducible up to the fp32 rounding of their order."""
-        return ops.ntuple_td_update(afterstate, target, self.weights, self.tuples, alpha=alpha, mask=mask, delta_out=delta_out)
+        return ops.ntuple_td_update(afterstate, target, self.weights, self.tuples, alpha=alpha, mask=mask, delta_out=delta_out,
+                                    stages=self.stages)
 
     def _tc_alloc(self) -> None:
         if self.coherence is None:
@@ -115,11 +126,11 @@ class NTupleNetwork:
     def tc_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
                   delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One synchronous temporal coherence batch toward ``target``; returns delta = alpha * (target - V)
-        (``ops.ntuple_tc_update``).  The first call allocates ``coherence`` ((N, 2) float32 {E, A} per weight, zeros) and a
-        zero scratch accumulator of the same shape."""
+        (``ops.ntuple_tc_update``).  The first call allocates ``coherence`` ((S * N, 2) float32 {E, A} per weight, zeros)
+        and a zero scratch accumulator of the same shape."""
         self._tc_alloc()
         return ops.ntuple_tc_update(afterstate, target, self.weights, self.coherence, self._tc_accum, self.tuples, alpha=alpha,
-                                    mask=mask, delta_out=delta_out)
+                                    mask=mask, delta_out=delta_out, stages=self.stages)
 
     def td_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                          alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
@@ -127,7 +138,7 @@ class NTupleNetwork:
         """One synchronous delayed TD(lambda) batch over the caller's ring of each game's last h + 1 afterstates; returns
         delta = alpha * (R_0 - V(x_0)) (``ops.ntuple_td_lambda_update``)."""
         return ops.ntuple_td_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.tuples, alpha=alpha,
-                                           lam=lam, mask=mask, delta_out=delta_out)
+                                           lam=lam, mask=mask, delta_out=delta_out, stages=self.stages)
 
     def tc_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                          alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
@@ -136,19 +147,23 @@ class NTupleNetwork:
         accumulator are allocated as by ``tc_update``."""
         self._tc_alloc()
         return ops.ntuple_tc_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.coherence,
-                                           self._tc_accum, self.tuples, alpha=alpha, lam=lam, mask=mask, delta_out=delta_out)
+                                           self._tc_accum, self.tuples, alpha=alpha, lam=lam, mask=mask, delta_out=delta_out,
+                                           stages=self.stages)
 
     def state_dict(self) -> dict:
-        state = {"tuples": [list(t) for t in self.tuples], "weights": self.weights.detach().clone()}
+        state = {"tuples": [list(t) for t in self.tuples], "stages": list(self.stages), "weights": self.weights.detach().clone()}
         if self.coherence is not None:
             state["coherence"] = self.coherence.detach().clone()
         return state
 
     def load_state_dict(self, state: dict) -> None:
         """Loads the weights and, when ``state`` has them, the TC coherence sums; a dict without ``"coherence"`` drops any
-        coherence state this network has (the next ``tc_update`` starts from zeros)."""
+        coherence state this network has (the next ``tc_update`` starts from zeros).  A dict without ``"stages"`` is a
+        single-stage network's (``stages=()``)."""
         if ops.ntuple_spec(state["tuples"]) != self.tuples:
             raise ValueError(f"state_dict is for tuples {state['tuples']}, this network has {self.tuples}")
+        if ops.ntuple_stages(state.get("stages", ())) != self.stages:
+            raise ValueError(f"state_dict is for stages {tuple(state.get('stages', ()))}, this network has {self.stages}")
         w = state["weights"]
         if not isinstance(w, torch.Tensor) or w.dtype != torch.float32 or tuple(w.shape) != tuple(self.weights.shape):
             raise ValueError(f"weights must be float32 {tuple(self.weights.shape)}")
@@ -167,7 +182,7 @@ class NTupleNetwork:
 
 class GreedyPolicy:
     """The network's greedy afterstate move as a policy ``DeviceRunner`` accepts: ``sample_actions(state, valid_actions)``
-    returns (actions int64, log_probs 0).  ``reward_fn`` must be the environment's."""
+    returns (actions int64, log_probs 0).  ``reward_fn`` must be the environment's.  A multi-stage network works here as is."""
 
     def __init__(self, net: NTupleNetwork, reward_fn=None):
         self.net = net
@@ -182,7 +197,8 @@ class GreedyPolicy:
 class ExpectimaxPolicy:
     """The network's expectimax move (``NTupleNetwork.expectimax``) as a policy ``DeviceRunner`` accepts:
     ``sample_actions(state, valid_actions)`` returns (actions int64, log_probs 0).  ``reward_fn`` and ``two_prob`` must be the
-    environment's: the search scores moves with that reward and averages over spawns with that chance of a 2."""
+    environment's: the search scores moves with that reward and averages over spawns with that chance of a 2.  A multi-stage
+    network works here as is: each leaf is valued with its own stage's tables."""
 
     def __init__(self, net: NTupleNetwork, depth: int = 1, reward_fn=None, two_prob: float = 0.8):
         if isinstance(depth, bool) or depth not in (1, 2):
@@ -223,7 +239,10 @@ class TDAfterstateLearner:
     the afterstate of step T - h (slot (T + 1) mod (h + 1)) toward the lambda-return over the window up to x_T, truncated at
     the first end in it.  So the last h afterstates of a run are never updated.  ``delta`` is the delta of the afterstate
     updated in the step (0 while nothing is).  With ``rule="tc"`` and h > 1, ``alpha`` defaults to
-    ``DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES / M``.  ``horizon=1`` is the TD(0) / TC learner above, whatever ``lam`` is."""
+    ``DEFAULT_TC_LAMBDA_ALPHA_TIMES_GAMES / M``.  ``horizon=1`` is the TD(0) / TC learner above, whatever ``lam`` is.
+
+    A multi-stage network (``NTupleNetwork(..., stages=...)``) works with every rule: the learner only calls the network.
+    The default step sizes are the single-stage sweeps'; none has been run for staged networks."""
 
     def __init__(self, env, net: NTupleNetwork, alpha: Optional[float] = None, rule: str = "td0", horizon: int = 1,
                  lam: float = 0.5):

@@ -13,6 +13,8 @@
     ntuple_tc_update            a temporal coherence batch update of such a network: per-weight step sizes
     ntuple_td_lambda_update,    delayed TD(lambda) / TC(lambda): the afterstate of h steps ago toward a lambda-return over
     ntuple_tc_lambda_update     the caller's ring of each game's last h + 1 afterstates, valued in one kernel
+    ntuple_stages               every ntuple_* op takes ``stages=``: a multi-stage network, one weight set per stage of the
+                                game, chosen by the board's largest tile
 """
 
 from __future__ import annotations
@@ -207,12 +209,60 @@ def ntuple_spec(tuples) -> tuple:
     return spec
 
 
-def ntuple_num_weights(tuples) -> int:
-    """sum over the tuples of 16^len: the length of the network's one float32 weight tensor"""
-    return sum(16 ** len(t) for t in ntuple_spec(tuples))
+NTUPLE_MAX_STAGES = 8
+
+
+def ntuple_stages(stages) -> tuple:
+    """Check a multi-stage network's stage thresholds on the host and return them as a tuple of ints.
+
+    S - 1 = 0..7 strictly ascending tile exponents in 1..15 (ints, not bools) give S = 1..8 stages; () is the single-stage
+    network.  Raises ValueError otherwise.  With thresholds tau_1 < ... < tau_{S-1}, m(b) = max over the 16 cells of
+    min(b[c], 15) (the index's own clamp) and stage(b) = #{k : tau_k <= m(b)}: an empty board is in stage 0, a byte >= 16
+    counts as 15.  The weights are S * N float32 entries (N = sum 16^len), stage s's tables at s * N in the single-stage
+    layout.  V(b) uses the tables of b's own stage (greedy: each afterstate's; expectimax: each leaf's; TD(lambda): each
+    window board's), and every update writes the entries of x_0's stage.  Everything else is the single-stage op's, and
+    S = 1 is that op bit for bit."""
+    try:
+        got = tuple(stages)
+    except TypeError:
+        raise ValueError(f"stages must be a sequence of tile exponents, got {stages!r}") from None
+    if any(isinstance(t, bool) or not isinstance(t, (int, np.integer)) for t in got):
+        raise ValueError(f"stages must be ints, got {stages!r}")
+    got = tuple(int(t) for t in got)
+    if len(got) > NTUPLE_MAX_STAGES - 1:
+        raise ValueError(f"a network has at most {NTUPLE_MAX_STAGES} stages ({NTUPLE_MAX_STAGES - 1} thresholds), "
+                         f"got {len(got)} thresholds")
+    if any(t < 1 or t > 15 for t in got) or any(a >= b for a, b in zip(got, got[1:])):
+        raise ValueError(f"stage thresholds are strictly ascending tile exponents in 1..15, got {got}")
+    return got
+
+
+def ntuple_num_weights(tuples, stages=()) -> int:
+    """S * sum over the tuples of 16^len: the length of the network's one float32 weight tensor (S = len(stages) + 1)"""
+    return (len(ntuple_stages(stages)) + 1) * sum(16 ** len(t) for t in ntuple_spec(tuples))
 
 
 _SPEC_ARRAYS: dict = {}
+_STAGE_ARRAYS: dict = {}
+
+
+def _stage_array(stages):
+    """(host threshold array u8 [S-1] or None, S) of the checked stages.  Every call checks ``stages``; the array is cached
+    per checked tuple so that repeated calls do not build it again (the library reads it on the host, during the call)."""
+    st = ntuple_stages(stages)
+    got = _STAGE_ARRAYS.get(st)
+    if got is None:
+        got = (np.array(st, np.uint8) if st else None, len(st) + 1)
+        if len(_STAGE_ARRAYS) < 64:
+            _STAGE_ARRAYS[st] = got
+    return got
+
+
+def _network_args(tuples, stages):
+    """(cells, len, K, stage thresholds or None, S, number of weights S * N) of a checked network"""
+    cells, lens, k, n = _spec_arrays(tuples)
+    tau, s = _stage_array(stages)
+    return cells, lens, k, tau, s, s * n
 
 
 def _spec_arrays(tuples):
@@ -230,14 +280,20 @@ def _spec_arrays(tuples):
     return got
 
 
-def _weights_arg(weights: torch.Tensor, n: int, device) -> None:
+def _weights_arg(weights: torch.Tensor, n: int, device, stages: int = 1) -> None:
     if not (isinstance(weights, torch.Tensor) and weights.is_cuda and weights.is_contiguous() and weights.dtype == torch.float32
             and weights.ndim == 1):
         raise ValueError("weights must be a contiguous 1-D float32 CUDA tensor")
     if weights.numel() != n:
+        if stages > 1:
+            raise ValueError(f"weights has {weights.numel()} entries, the tuples and {stages} stages need S * sum 16^len = {n}")
         raise ValueError(f"weights has {weights.numel()} entries, the tuples need sum 16^len = {n}")
     if weights.device != device:
         raise ValueError(f"weights is on {weights.device}, the boards on {device}")
+
+
+def _ptr(a) -> Optional[int]:
+    return None if a is None else a.ctypes.data
 
 
 def _board_arg(board, name: str = "board") -> None:
@@ -246,26 +302,28 @@ def _board_arg(board, name: str = "board") -> None:
     _cuda(board, name)
 
 
-def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Optional[torch.Tensor] = None,
+                 stages=()) -> torch.Tensor:
     """V(board) of an n-tuple network: (M,16) uint8/int8 boards -> (M,) float32.
 
     ``tuples``: the network's cells (see ``ntuple_spec``); ``weights``: its one float32 tensor of sum 16^len entries, tuple t's
     table after those of tuples 0..t-1.  V sums, for t = 0..K-1 and then each of the board's 8 symmetric images g = 0..7,
     ``weights[offset_t + sum_j min(image_g[cell_tj], 15) << 4j]`` as float32 adds from 0 in that order: bit-reproducible.
     Every byte gives an in-bounds index; tiles 2^16 and above share the entries of 2^15.  ``out``: a preallocated (M,)
-    float32 tensor (CUDA-graph capture)."""
+    float32 tensor (CUDA-graph capture).  ``stages``: the thresholds of a multi-stage network (``ntuple_stages``); its
+    ``weights`` hold S * sum 16^len entries and each board is valued with the tables of its own stage."""
     _board_arg(board)
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, board.device)
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, board.device, s)
     m = board.shape[0]
     out = _out_arg(out, (m,), torch.float32, board.device, "out")
     if m == 0:
         return out
     lib = _lib.load()
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_ntuple_value(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, out.data_ptr(), m,
-                                     _stream(board))
-    _lib.check(rc, "ml2048_ntuple_value")
+        rc = lib.ml2048_staged_value(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
+                                     out.data_ptr(), m, _stream(board))
+    _lib.check(rc, "ml2048_staged_value")
     return out
 
 
@@ -281,7 +339,7 @@ def _move_outputs(out, specs: dict, action_dtype, board, op: str) -> dict:
 
 
 def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
-                  out: Optional[dict] = None) -> dict:
+                  out: Optional[dict] = None, stages=()) -> dict:
     """The greedy afterstate move of every board under an n-tuple network, in one kernel.
 
     For every direction a that changes the board, q_a = reward_a + V(afterstate_a) in float32, with reward_a and afterstate_a
@@ -294,13 +352,14 @@ def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_
         "value"   (M,)    float32  V(afterstate)
 
     A board without a valid move gets action 0, its own board, reward 0 and value 0 (so a TD target reward + value is 0).
-    ``out``: preallocated tensors under the same keys (any subset), so that the call can be captured in a CUDA graph."""
+    ``out``: preallocated tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.
+    ``stages``: a multi-stage network (``ntuple_stages``); each afterstate is valued with the tables of its own stage."""
     _board_arg(board)
     if action_dtype not in (torch.int64, torch.uint8):
         raise ValueError("action_dtype must be torch.int64 or torch.uint8")
     kind = reward_kind(reward_fn)
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, board.device)
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, board.device, s)
     m = board.shape[0]
     res = _move_outputs(out, _NTUPLE_GREEDY, action_dtype, board, "ntuple_greedy")
     if m == 0:
@@ -308,10 +367,10 @@ def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_
     act = res["action"].data_ptr()
     lib = _lib.load()
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_ntuple_greedy(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, kind,
+        rc = lib.ml2048_staged_greedy(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, kind,
                                       act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
                                       res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), m, _stream(board))
-    _lib.check(rc, "ml2048_ntuple_greedy")
+    _lib.check(rc, "ml2048_staged_greedy")
     return res
 
 
@@ -319,7 +378,7 @@ _NTUPLE_EXPECTIMAX = dict(_NTUPLE_GREEDY, q=((4,), torch.float32))
 
 
 def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
-                      action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None) -> dict:
+                      action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None, stages=()) -> dict:
     """The expectimax move of every board under an n-tuple network, ``depth`` (1 or 2) chance layers deep, in one kernel.
 
     Definition (every operation one float32 operation; after, r, valid as ``afterstates(board, reward_fn=reward_fn)`` gives
@@ -344,7 +403,8 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
         "q"       (M,4)   float32  q of every direction
 
     A board without a valid move gets action 0, its own board, reward 0, value 0 and q all -inf.  ``out``: preallocated
-    tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.  Cells must be 0..17."""
+    tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.  Cells must be 0..17.
+    ``stages``: a multi-stage network (``ntuple_stages``); each leaf is valued with the tables of its own stage."""
     _board_arg(board)
     if action_dtype not in (torch.int64, torch.uint8):
         raise ValueError("action_dtype must be torch.int64 or torch.uint8")
@@ -357,8 +417,8 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
     if not 0.0 <= p <= 1.0:
         raise ValueError(f"two_prob must be in [0, 1], got {two_prob!r}")
     kind = reward_kind(reward_fn)
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, board.device)
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, board.device, s)
     m = board.shape[0]
     res = _move_outputs(out, _NTUPLE_EXPECTIMAX, action_dtype, board, "ntuple_expectimax")
     if m == 0:
@@ -366,11 +426,11 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
     act = res["action"].data_ptr()
     lib = _lib.load()
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_expectimax(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, kind, int(depth), p,
-                                   act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
-                                   res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), res["q"].data_ptr(), m,
-                                   _stream(board))
-    _lib.check(rc, "ml2048_expectimax")
+        rc = lib.ml2048_staged_expectimax(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
+                                          kind, int(depth), p, act if action_dtype == torch.uint8 else None,
+                                          act if action_dtype == torch.int64 else None, res["state"].data_ptr(), res["reward"].data_ptr(),
+                                          res["value"].data_ptr(), res["q"].data_ptr(), m, _stream(board))
+    _lib.check(rc, "ml2048_staged_expectimax")
     return res
 
 
@@ -383,7 +443,7 @@ def _coherence_args(coherence, accum, n: int, device) -> tuple[int, int]:
     return coherence.data_ptr(), accum.data_ptr()
 
 
-def _target_update(fn: str, afterstate, target, weights, tuples, alpha, mask, delta_out, tc=None) -> torch.Tensor:
+def _target_update(fn: str, afterstate, target, weights, tuples, stages, alpha, mask, delta_out, tc=None) -> torch.Tensor:
     """ntuple_td_update (tc None) and ntuple_tc_update (tc = (coherence, accum)) through library function ``fn``"""
     _board_arg(afterstate, "afterstate")
     m = afterstate.shape[0]
@@ -394,8 +454,8 @@ def _target_update(fn: str, afterstate, target, weights, tuples, alpha, mask, de
         _cuda(mask, "mask")
         if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,):
             raise ValueError(f"mask must be bool/uint8 ({m},)")
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, afterstate.device)
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, afterstate.device, s)
     tc_ptrs = () if tc is None else _coherence_args(*tc, n, afterstate.device)
     delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
     if m == 0:
@@ -403,27 +463,28 @@ def _target_update(fn: str, afterstate, target, weights, tuples, alpha, mask, de
     lib = _lib.load()
     with torch.cuda.device(afterstate.device):
         rc = getattr(lib, fn)(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None, float(alpha),
-                              weights.data_ptr(), *tc_ptrs, n, cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m,
-                              _stream(afterstate))
+                              weights.data_ptr(), *tc_ptrs, n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
+                              delta_out.data_ptr(), m, _stream(afterstate))
     _lib.check(rc, fn)
     return delta_out
 
 
 def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, tuples, *, alpha: float,
-                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
     """One synchronous batch of TD(0) updates of an n-tuple network, in place on ``weights``; returns delta (M,) float32.
 
     Phase 1: delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game
     whose ``mask`` byte is 0 (``mask``: (M,) bool/uint8, None = every game).  Phase 2: every entry of every masked-in game,
     8 per tuple, gets += delta_i.  Phase 2 adds with float atomics, so the order of the adds that several games make to one
     entry is unspecified: the weights are reproducible only up to the fp32 rounding of that order.  delta is deterministic.
-    ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
-    return _target_update("ml2048_ntuple_td_update", afterstate, target, weights, tuples, alpha, mask, delta_out)
+    ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture).  ``stages``: a multi-stage network
+    (``ntuple_stages``); V(afterstate_i) and the update use the tables of afterstate_i's stage."""
+    return _target_update("ml2048_staged_td_update", afterstate, target, weights, tuples, stages, alpha, mask, delta_out)
 
 
 def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, coherence: torch.Tensor,
                      accum: torch.Tensor, tuples, *, alpha: float, mask: Optional[torch.Tensor] = None,
-                     delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                     delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
     """One synchronous batch of temporal coherence (TC) updates of an n-tuple network, in place on ``weights`` and
     ``coherence``; returns delta (M,) float32.
 
@@ -441,14 +502,16 @@ def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
     E and A sum alpha-scaled errors: with a constant alpha, beta is the same as for unscaled errors; a changing alpha weights
     older errors by the alpha they had.  ``coherence`` and ``accum``: contiguous float32 (N, 2) tensors on the weights'
     device; ``accum`` is scratch that must be all zero and is left all zero.  ``delta_out``: a preallocated (M,) float32
-    tensor (CUDA-graph capture)."""
-    return _target_update("ml2048_tc_update", afterstate, target, weights, tuples, alpha, mask, delta_out, (coherence, accum))
+    tensor (CUDA-graph capture).  ``stages``: a multi-stage network (``ntuple_stages``); ``weights`` has S * N entries,
+    ``coherence`` and ``accum`` are (S * N, 2), and afterstate_i's value and update use the entries of its stage."""
+    return _target_update("ml2048_staged_tc_update", afterstate, target, weights, tuples, stages, alpha, mask, delta_out,
+                          (coherence, accum))
 
 
 NTUPLE_LAMBDA_MAX_HORIZON = 16
 
 
-def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask, delta_out,
+def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha, lam, mask, delta_out,
                    tc=None) -> torch.Tensor:
     """ntuple_td_lambda_update (tc None) and ntuple_tc_lambda_update (tc = (coherence, accum)) through library function ``fn``"""
     if not (isinstance(after_ring, torch.Tensor) and after_ring.dtype in (torch.uint8, torch.int8) and after_ring.ndim == 3
@@ -476,8 +539,8 @@ def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights
         _cuda(mask, "mask")
         if mask.dtype not in (torch.bool, torch.uint8) or tuple(mask.shape) != (m,) or mask.device != dev:
             raise ValueError(f"mask must be bool/uint8 ({m},) on {dev}")
-    cells, lens, k, n = _spec_arrays(tuples)
-    _weights_arg(weights, n, dev)
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, dev, s)
     tc_ptrs = () if tc is None else _coherence_args(*tc, n, dev)
     delta_out = _out_arg(delta_out, (m,), torch.float32, dev, "delta_out")
     if m == 0:
@@ -486,14 +549,14 @@ def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights
     with torch.cuda.device(dev):
         rc = getattr(lib, fn)(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
                               mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(), *tc_ptrs, n,
-                              cells.ctypes.data, lens.ctypes.data, k, delta_out.data_ptr(), m, _stream(after_ring))
+                              cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, delta_out.data_ptr(), m, _stream(after_ring))
     _lib.check(rc, fn)
     return delta_out
 
 
 def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                             weights: torch.Tensor, tuples, *, alpha: float, lam: float, mask: Optional[torch.Tensor] = None,
-                            delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                            delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
     """One synchronous batch of delayed TD(lambda) updates of an n-tuple network (Jaskowski 2018), in place on ``weights``:
     each game's afterstate of h learner steps ago moves toward a lambda-return truncated at h.  Returns delta (M,) float32.
 
@@ -512,19 +575,21 @@ def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor,
     The ring is the caller's: ``after_ring`` (h+1, M, 16) uint8/int8, ``reward_ring`` (h+1, M) float32, ``ended_ring``
     (h+1, M) bool/uint8, all contiguous on one device, h = ``after_ring.shape[0] - 1`` in 1..16.  ``newest`` is the slot of
     x_h; x_k is in slot (newest - (h - k)) mod (h + 1), and ``ended_ring[newest]`` is not read.  ``mask``: (M,) bool/uint8,
-    None = every game.  ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture)."""
-    return _lambda_update("ml2048_lambda_td_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask,
-                          delta_out)
+    None = every game.  ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture).  ``stages``: a multi-stage
+    network (``ntuple_stages``); each V_k uses the tables of x_k's stage, and the update writes the entries of x_0's stage."""
+    return _lambda_update("ml2048_staged_lambda_td_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha,
+                          lam, mask, delta_out)
 
 
 def ntuple_tc_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                             weights: torch.Tensor, coherence: torch.Tensor, accum: torch.Tensor, tuples, *, alpha: float,
                             lam: float, mask: Optional[torch.Tensor] = None,
-                            delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                            delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
     """One synchronous batch of delayed TC(lambda) updates, in place on ``weights`` and ``coherence``; returns delta (M,)
     float32.  delta is ``ntuple_td_lambda_update``'s (the same window, ring, definition and arguments); the update of x_0's
     entries is then ``ntuple_tc_update``'s phases 2 and 3: {dE, dA} += {delta, |delta|} into ``accum``, and w += beta * dE,
     beta = |E| / A (1 where A = 0), {E, A} += {dE, dA} for every entry with dA != 0.  ``coherence`` and ``accum``: contiguous
-    float32 (N, 2) tensors on the ring's device; ``accum`` must be all zero and is left all zero."""
-    return _lambda_update("ml2048_lambda_tc_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, alpha, lam, mask,
-                          delta_out, (coherence, accum))
+    float32 (N, 2) tensors on the ring's device; ``accum`` must be all zero and is left all zero.  ``stages``: as for
+    ``ntuple_td_lambda_update``, with ``coherence`` and ``accum`` (S * N, 2)."""
+    return _lambda_update("ml2048_staged_lambda_tc_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha,
+                          lam, mask, delta_out, (coherence, accum))
