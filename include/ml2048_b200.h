@@ -29,7 +29,8 @@ extern "C" {
 #endif
 
 /* 12 also covers ml2048_alloc_compressible / ml2048_free_compressible, ml2048_expectimax, ml2048_tc_update,
- * ml2048_lambda_td_update, ml2048_lambda_tc_update and the seven ml2048_staged_* entries, added without a bump (unlike
+ * ml2048_lambda_td_update, ml2048_lambda_tc_update, the seven ml2048_staged_* and the seven ml2048_promoted_* entries, added
+ * without a bump (unlike
  * earlier additions): they change no existing struct or signature, and a loader that binds them by name fails on a library
  * without them. */
 #define ML2048_ABI_VERSION 12
@@ -421,6 +422,54 @@ ML2048_API int ml2048_staged_expectimax(const void *board, const float *weights,
                                         const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind,
                                         int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out,
                                         float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream);
+
+/* weight promotion of multi-stage networks (Jaskowski 2018): a stage's entry starts from the stage below on its first
+ * update.  Each ml2048_promoted_* entry is the ml2048_staged_* entry it names with `uint8_t *promoted` after num_stages
+ * (const for value, greedy and expectimax).  promoted: N bytes of device memory (N = sum_t 16^len[t], the single-stage entry
+ * count, whatever S is), 4-byte aligned, indexed like a single-stage table.  Bit s - 1 of promoted[e] is set once stage s's
+ * entry e has been written (s = 1..S-1); stage 0 has no mark, and bits S-1..7 are neither read nor written.
+ *   Effective weight: W(0, e) = weights[e]; for s >= 1, W(s, e) = weights[s * N + e] if the mark of (s, e) is set, else
+ *   W(s - 1, e).  Every value (value, greedy's afterstates, expectimax's leaves, the deltas' V(x_0) and every TD(lambda)
+ *   window board) is the staged entry's, in the same float32 order, with W in place of weights; the storage of an unmarked
+ *   entry is never read.
+ *   Updates: 1. the staged entry's delta with W before the call; 2. promote: for every masked-in game whose x_0 is in stage
+ *   s0 >= 1 (whatever its delta, 0 included) and each of its 8K entries e with (s0, e) unmarked, weights[s0 * N + e] =
+ *   W(s0 - 1, e), for TC coherence[s0 * N + e] = {0, 0} (the first TC step of a promoted entry has beta = 1), and the mark
+ *   is set; 3. the staged entry's TD(0) scatter or TC accumulate + apply on x_0's own-stage entries.  So promotion changes no
+ *   effective weight.  With every mark 0..S-2 set, each entry is the staged entry bit for bit and no mark changes; S = 1
+ *   reads and writes no mark and is the single-stage entry bit for bit.
+ * E_NULL: promoted null; E_ALIGN: promoted not 4-byte aligned (marks are set with word atomics).  Every other check is the
+ * staged entry's; all return before any launch. */
+ML2048_API int ml2048_promoted_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells,
+                                     const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                                     const uint8_t *promoted, float *value_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_promoted_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells,
+                                      const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                                      const uint8_t *promoted, int32_t reward_kind, uint8_t *action_u8, int64_t *action_i64, void *after_out,
+                                      float *reward_out, float *value_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_promoted_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                         int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                         const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games,
+                                         void *stream);
+ML2048_API int ml2048_promoted_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                                         float *coherence, float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                         int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted,
+                                         float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_promoted_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring,
+                                                int32_t horizon, int32_t newest, float lambda, const uint8_t *mask, float alpha,
+                                                float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                                                int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted,
+                                                float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_promoted_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring,
+                                                int32_t horizon, int32_t newest, float lambda, const uint8_t *mask, float alpha,
+                                                float *weights, float *coherence, float *accum, int64_t num_weights, const uint8_t *cells,
+                                                const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                                                uint8_t *promoted, float *delta_out, int64_t num_games, void *stream);
+ML2048_API int ml2048_promoted_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells,
+                                          const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                                          const uint8_t *promoted, int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8,
+                                          int64_t *action_i64, void *after_out, float *reward_out, float *value_out, float *q_out,
+                                          int64_t num_games, void *stream);
 
 /* _update_count (runner.py:120-136): hist[max exponent] += 1 for every game with terminated != 0;
  * with terminated == null: VecGame.summary's histogram over all live boards (game_numba.py:593-596).

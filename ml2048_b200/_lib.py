@@ -197,6 +197,17 @@ SYMBOLS = {
     "ml2048_staged_lambda_tc_update": (C.c_int, [_VP, _VP, _VP, _I32, _I32, C.c_float, _VP, C.c_float, _VP, _VP, _VP, _I64, _VP, _VP,
                                                  _I32, _VP, _I32, _VP, _I64, _VP]),
     "ml2048_staged_expectimax": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _I32, _I32, C.c_double] + [_VP] * 6 + [_I64, _VP]),
+    "ml2048_promoted_value": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _VP, _VP, _I64, _VP]),
+    "ml2048_promoted_greedy": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _VP, _I32, _VP, _VP, _VP, _VP, _VP, _I64, _VP]),
+    "ml2048_promoted_td_update": (C.c_int, [_VP, _VP, _VP, C.c_float, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _VP, _VP, _I64, _VP]),
+    "ml2048_promoted_tc_update": (C.c_int, [_VP, _VP, _VP, C.c_float, _VP, _VP, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _VP, _VP, _I64,
+                                            _VP]),
+    "ml2048_promoted_lambda_td_update": (C.c_int, [_VP, _VP, _VP, _I32, _I32, C.c_float, _VP, C.c_float, _VP, _I64, _VP, _VP, _I32, _VP,
+                                                   _I32, _VP, _VP, _I64, _VP]),
+    "ml2048_promoted_lambda_tc_update": (C.c_int, [_VP, _VP, _VP, _I32, _I32, C.c_float, _VP, C.c_float, _VP, _VP, _VP, _I64, _VP, _VP,
+                                                   _I32, _VP, _I32, _VP, _VP, _I64, _VP]),
+    "ml2048_promoted_expectimax": (C.c_int, [_VP, _VP, _I64, _VP, _VP, _I32, _VP, _I32, _VP, _I32, _I32, C.c_double] + [_VP] * 6
+                                   + [_I64, _VP]),
     "ml2048_max_tile_hist": (C.c_int, [_VP, _VP, _I64, _VP, _VP]),
     "ml2048_copy_async": (C.c_int, [_VP, _VP, _I64, _VP]),
     "ml2048_stream_wait": (C.c_int, [_VP]),

@@ -848,4 +848,45 @@ ML2048_FN float ntuple_value(const float *w, const Spec &s, uint64_t nib)
     return acc;
 }
 
+// ---- weight promotion of multi-stage networks (Jaskowski 2018) ----
+// promoted: N bytes (N = sum_t 16^len_t, the single-stage entry count, for any S), indexed like a single-stage table.  Bit
+// s - 1 of byte e is set once stage s's entry e has been written (s = 1..S-1); stage 0 has no mark, and bits S-1..7 are
+// neither read nor written.  The effective weight is W(0, e) = w[e] and, for s >= 1, W(s, e) = w[s * N + e] if the mark of
+// (s, e) is set, else W(s - 1, e): the source stage src(s, m) is the highest k <= s with k = 0 or bit k - 1 of m set.  Every
+// read computes today's value, in the same float32 order, with W in place of w, so the storage of an unmarked entry is never
+// read.  An update (ml2048_promoted_* in the header) first computes its deltas this way, then promotes: every masked-in game
+// whose x_0 is in stage s0 >= 1 sets, for each of its entries e with (s0, e) unmarked, w[s0 * N + e] := W(s0 - 1, e) (TC:
+// coherence {0, 0}) and the mark; then it applies the rule to x_0's own-stage entries as a staged update does.  So
+// promotion changes no effective weight, and only the apply step does.
+struct NTuplePromotedSpec : NTupleStagedSpec {
+    const uint8_t *promoted;  // [N]
+};
+
+#if defined(__CUDACC__)
+ML2048_FN uint32_t clz32(uint32_t x) { return (uint32_t)__clz(x); }
+ML2048_FN uint32_t load_mark(const uint8_t *p) { return __ldg(p); }
+#else
+ML2048_FN uint32_t clz32(uint32_t x) { return (uint32_t)__builtin_clz(x); }
+ML2048_FN uint32_t load_mark(const uint8_t *p) { return *p; }
+#endif
+
+// src(s, m) for a stage s in 0..7 and a mark byte m: bit 0 of the operand stands for stage 0, which is always written
+ML2048_FN uint32_t ntuple_source_stage(uint32_t s, uint32_t m)
+{
+    return 31u - clz32(((m << 1) | 1u) & ((2u << s) - 1u));
+}
+
+// V(s) of a promoting network: each entry of the board's stage is read from its source stage.  A stage-0 board reads no mark.
+ML2048_FN float ntuple_value(const float *w, const NTuplePromotedSpec &s, uint64_t nib)
+{
+    const uint32_t stage = ntuple_stage(s, nib);
+    float acc = 0.0f;
+    ntuple_for_each_entry(static_cast<const NTupleSpec &>(s), nib, [&](uint32_t off, uint32_t idx) {
+        const uint32_t e = off + idx;
+        const uint32_t src = stage ? ntuple_source_stage(stage, load_mark(s.promoted + e)) : 0u;
+        acc += load_weight(w + src * s.stage_size + e);
+    });
+    return acc;
+}
+
 }  // namespace ml2048

@@ -1602,6 +1602,52 @@ __global__ void __launch_bounds__(kStepThreads) ntuple_tc_apply_kernel(const uin
     });
 }
 
+// ---- weight promotion (board_ops.cuh: NTuplePromotedSpec) ------------------------------------------
+// The reads and the delta phases of a promoting network are the kernels of this file instantiated with NTuplePromotedSpec:
+// only ntuple_value differs, and it reads the marks with __ldg because no read launch writes them.  An update then runs this
+// promote phase between its delta and apply launches on the same stream, and applies with the staged kernels, which write
+// the entries of x_0's own stage.  `mark_words` = the marks as 32-bit words.
+
+// Mark byte e, read with an acquire load of its whole 32-bit word (the size the atomicOr below writes): the weight and
+// coherence stores of the thread that set a bit seen here are visible after it
+__device__ __forceinline__ uint32_t load_mark_acquire(const uint32_t *words, uint32_t e)
+{
+    uint32_t m;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(m) : "l"(words + (e >> 2)) : "memory");
+    return (m >> (8u * (e & 3u))) & 0xffu;
+}
+
+// One thread per masked-in game with x_0 in stage s0 >= 1 walks x_0's entries e; where the mark of (s0, e) is clear it
+// stores w[s0 * N + e] = W(s0 - 1, e) (and TC's coherence {0, 0}), then __threadfence() and an atomicOr of the bit into the
+// mark's 32-bit word (release).  Two games of one launch can meet the same e in different stages, so a game at stage s0 may
+// find the mark of a lower stage k being set while it reads.  It reads marks with acquire loads and weights with L2 loads
+// (__ldcg, not the read-only path), so it sees either the bit clear, and reads a lower source whose storage this launch
+// does not write, or the bit set, and reads the copy that bit publishes.  Either way it gets W_before(k, e): stage k's copy
+// is W_before(k - 1, e) = W_before(k, e) when its mark was clear before the call, and untouched when it was set.  So every
+// writer of an entry stores the same value, no add happens in this launch, and the result does not depend on the order.
+// Stage 0 is never written here.
+__global__ void __launch_bounds__(kStepThreads) ntuple_promote_kernel(const uint4 *after, const uint8_t *mask, float *w, float2 *coh,
+                                                                      uint32_t *mark_words, __grid_constant__ const NTupleStagedSpec spec,
+                                                                      int64_t num_games)
+{
+    const int64_t i = (int64_t)blockIdx.x * kStepThreads + threadIdx.x;
+    if (i >= num_games || (mask && !mask[i])) return;
+    const uint4 b = after[i];
+    const uint64_t nib = ntuple_nibbles(b.x, b.y, b.z, b.w);
+    const uint32_t s0 = ntuple_stage(spec, nib);
+    if (s0 == 0u) return;
+    const uint32_t bit = 1u << (s0 - 1u), n = spec.stage_size;
+    ntuple_for_each_entry(static_cast<const NTupleSpec &>(spec), nib, [&](uint32_t off, uint32_t idx) {
+        const uint32_t e = off + idx;
+        const uint32_t m = load_mark_acquire(mark_words, e);
+        if (m & bit) return;
+        w[s0 * n + e] = __ldcg(w + ntuple_source_stage(s0, m) * n + e);
+        if (coh) coh[s0 * n + e] = make_float2(0.0f, 0.0f);
+        __threadfence();
+        atomicOr(mark_words + (e >> 2), bit << (8u * (e & 3u)));
+    });
+}
+
 // ---- delayed TD(lambda) / TC(lambda) ------------------------------------------------------------
 // Definition (ml2048_lambda_td_update in the header, ops.ntuple_td_lambda_update and tests/_lambda_ref.py say the same; every
 // operation is one float32 operation, __fadd_rn / __fmul_rn, no contraction).  Game i's window is x_0 ... x_h: x_0 the
@@ -1967,6 +2013,25 @@ inline int with_spec(const NTupleStagedSpec &spec, F &&f)
 {
     if (spec.stage_of == 0) return f(static_cast<const NTupleSpec &>(spec));
     return f(spec);
+}
+
+// with_spec for the reads and delta phases: a multi-stage network with marks (`promoted` non-null) runs the
+// NTuplePromotedSpec instances.  One stage has no mark to read, so it stays the NTupleSpec instances.
+template <class F>
+inline int with_spec(const NTupleStagedSpec &spec, const uint8_t *promoted, F &&f)
+{
+    if (!promoted || spec.stage_of == 0) return with_spec(spec, f);
+    NTuplePromotedSpec p;
+    static_cast<NTupleStagedSpec &>(p) = spec;
+    p.promoted = promoted;
+    return f(p);
+}
+
+// E_NULL / E_ALIGN of the marks of an ml2048_promoted_* entry (4-byte aligned: the promote phase sets them with word atomics)
+inline int check_promoted(const uint8_t *promoted)
+{
+    if (!promoted) return ML2048_E_NULL;
+    return misaligned(promoted, 4) ? ML2048_E_ALIGN : 0;
 }
 
 constexpr int kMaxDevices = 64;
@@ -2416,9 +2481,9 @@ int ml2048_afterstates(const void *board, void *after_out, float *reward_out, ui
     return launch_status();
 }
 
-int ml2048_staged_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
-                        int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, float *value_out, int64_t num_games,
-                        void *stream)
+static int value_entry(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                       int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted, float *value_out,
+                       int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || !value_out) return ML2048_E_NULL;
@@ -2428,11 +2493,26 @@ int ml2048_staged_value(const void *board, const float *weights, int64_t num_wei
     const int64_t grid = (num_games + kStepThreads - 1) / kStepThreads;
     if (grid > 0x7fffffff) return ML2048_E_SIZE;
     clear_stale_error();
-    return with_spec(spec, [&](const auto &sp) {
+    return with_spec(spec, promoted, [&](const auto &sp) {
         ntuple_value_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4 *>(board),
                                                                                                  weights, sp, value_out, num_games);
         return launch_status();
     });
+}
+
+int ml2048_staged_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                        int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, float *value_out, int64_t num_games,
+                        void *stream)
+{
+    return value_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, nullptr, value_out, num_games, stream);
+}
+
+int ml2048_promoted_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                          int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted, float *value_out,
+                          int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return value_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, promoted, value_out, num_games, stream);
 }
 
 int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
@@ -2441,9 +2521,10 @@ int ml2048_ntuple_value(const void *board, const float *weights, int64_t num_wei
     return ml2048_staged_value(board, weights, num_weights, cells, len, num_tuples, nullptr, 1, value_out, num_games, stream);
 }
 
-int ml2048_staged_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
-                         int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, uint8_t *action_u8,
-                         int64_t *action_i64, void *after_out, float *reward_out, float *value_out, int64_t num_games, void *stream)
+static int greedy_entry(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                        int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted, int32_t reward_kind,
+                        uint8_t *action_u8, int64_t *action_i64, void *after_out, float *reward_out, float *value_out, int64_t num_games,
+                        void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out) return ML2048_E_NULL;
@@ -2456,12 +2537,30 @@ int ml2048_staged_greedy(const void *board, const float *weights, int64_t num_we
     const int64_t grid = (num_games + kStepThreads / 4 - 1) / (kStepThreads / 4);  // four threads per game
     if (grid > 0x7fffffff) return ML2048_E_SIZE;
     clear_stale_error();
-    return with_spec(spec, [&](const auto &sp) {
+    return with_spec(spec, promoted, [&](const auto &sp) {
         ntuple_greedy_kernel<<<(unsigned)grid, kStepThreads, 0, static_cast<cudaStream_t>(stream)>>>(
             reinterpret_cast<const uint4 *>(board), weights, sp, reward_kind, action_u8, reinterpret_cast<long long *>(action_i64),
             reinterpret_cast<uint4 *>(after_out), reward_out, value_out, num_games);
         return launch_status();
     });
+}
+
+int ml2048_staged_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                         int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, uint8_t *action_u8,
+                         int64_t *action_i64, void *after_out, float *reward_out, float *value_out, int64_t num_games, void *stream)
+{
+    return greedy_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, nullptr, reward_kind, action_u8,
+                        action_i64, after_out, reward_out, value_out, num_games, stream);
+}
+
+int ml2048_promoted_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                           int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted, int32_t reward_kind,
+                           uint8_t *action_u8, int64_t *action_i64, void *after_out, float *reward_out, float *value_out,
+                           int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return greedy_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, promoted, reward_kind, action_u8,
+                        action_i64, after_out, reward_out, value_out, num_games, stream);
 }
 
 int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
@@ -2472,10 +2571,10 @@ int ml2048_ntuple_greedy(const void *board, const float *weights, int64_t num_we
                                 after_out, reward_out, value_out, num_games, stream);
 }
 
-int ml2048_staged_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
-                             int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, int32_t depth,
-                             double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out, float *reward_out,
-                             float *value_out, float *q_out, int64_t num_games, void *stream)
+static int expectimax_entry(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                            int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted,
+                            int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64,
+                            void *after_out, float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!board || !weights || (!action_u8 && !action_i64) || !after_out || !reward_out || !value_out || !q_out) return ML2048_E_NULL;
@@ -2497,7 +2596,7 @@ int ml2048_staged_expectimax(const void *board, const float *weights, int64_t nu
     uint4 *after = reinterpret_cast<uint4 *>(after_out);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     clear_stale_error();
-    return with_spec(spec, [&](const auto &sp) {
+    return with_spec(spec, promoted, [&](const auto &sp) {
         if (depth == 1)
             expectimax1_kernel<<<(unsigned)grid, kExpectimaxThreads, 0, s>>>(b, weights, sp, reward_kind, law, action_u8, a64, after,
                                                                              reward_out, value_out, q_out, num_games);
@@ -2506,6 +2605,25 @@ int ml2048_staged_expectimax(const void *board, const float *weights, int64_t nu
                                                                              reward_out, value_out, q_out);
         return launch_status();
     });
+}
+
+int ml2048_staged_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                             int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, int32_t reward_kind, int32_t depth,
+                             double two_prob, uint8_t *action_u8, int64_t *action_i64, void *after_out, float *reward_out,
+                             float *value_out, float *q_out, int64_t num_games, void *stream)
+{
+    return expectimax_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, nullptr, reward_kind, depth,
+                            two_prob, action_u8, action_i64, after_out, reward_out, value_out, q_out, num_games, stream);
+}
+
+int ml2048_promoted_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len,
+                               int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages, const uint8_t *promoted,
+                               int32_t reward_kind, int32_t depth, double two_prob, uint8_t *action_u8, int64_t *action_i64,
+                               void *after_out, float *reward_out, float *value_out, float *q_out, int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return expectimax_entry(board, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, promoted, reward_kind, depth,
+                            two_prob, action_u8, action_i64, after_out, reward_out, value_out, q_out, num_games, stream);
 }
 
 int ml2048_expectimax(const void *board, const float *weights, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
@@ -2535,10 +2653,11 @@ static int check_update(const void *after, const float *values, const float *wei
 
 // Phase 1 of TD(0) and TC: delta = alpha * (target - V(after))
 static int target_delta(const uint4 *after, const float *target, const uint8_t *mask, float alpha, const float *weights,
-                        const NTupleStagedSpec &spec, float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s)
+                        const NTupleStagedSpec &spec, const uint8_t *promoted, float *delta_out, unsigned grid, int64_t num_games,
+                        cudaStream_t s)
 {
     clear_stale_error();
-    return with_spec(spec, [&](const auto &sp) {
+    return with_spec(spec, promoted, [&](const auto &sp) {
         ntuple_td_delta_kernel<<<grid, kStepThreads, 0, s>>>(after, target, mask, alpha, weights, sp, delta_out, num_games);
         return launch_status();
     });
@@ -2547,7 +2666,7 @@ static int target_delta(const uint4 *after, const float *target, const uint8_t *
 // Phase 1 of TD(lambda) and TC(lambda): the checks only they make, then delta over the ring.  `x0` = x_0's slot of the ring.
 static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
                         float lambda, const uint8_t *mask, float alpha, const float *weights, const NTupleStagedSpec &spec,
-                        float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s, const uint4 *&x0)
+                        const uint8_t *promoted, float *delta_out, unsigned grid, int64_t num_games, cudaStream_t s, const uint4 *&x0)
 {
     if (!ended_ring) return ML2048_E_NULL;
     if (horizon < 1 || horizon > kLambdaMaxHorizon || newest < 0 || newest > horizon) return ML2048_E_SIZE;
@@ -2555,7 +2674,7 @@ static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8
     x0 = ring + (int64_t)(newest == horizon ? 0 : newest + 1) * num_games;
     const float c = 1.0f - lambda;
     clear_stale_error();
-    return with_spec(spec, [&](const auto &sp) {
+    return with_spec(spec, promoted, [&](const auto &sp) {
         ntuple_lambda_delta_kernel<<<grid, kStepThreads, 0, s>>>(ring, reward_ring, ended_ring, mask, horizon, newest, lambda, c, alpha,
                                                                  weights, sp, delta_out, num_games);
         return launch_status();
@@ -2563,10 +2682,16 @@ static int lambda_delta(const uint4 *ring, const float *reward_ring, const uint8
 }
 
 // The update of x_0's entries after phase 1, on the same stream (so every delta is computed before any weight is written):
-// TD(0)'s scatter when `coherence` is null, else TC's phases 2 and 3.  The entries are those of x_0's stage.
+// with marks (`promoted` non-null) and S > 1 first the promote phase, then TD(0)'s scatter when `coherence` is null, else
+// TC's phases 2 and 3.  The entries are those of x_0's stage.
 static int apply_update(const uint4 *x0, const uint8_t *mask, const float *delta, float *weights, float *coherence, float *accum,
-                        const NTupleStagedSpec &spec, unsigned grid, int64_t num_games, cudaStream_t s)
+                        const NTupleStagedSpec &spec, uint8_t *promoted, unsigned grid, int64_t num_games, cudaStream_t s)
 {
+    if (promoted && spec.stage_of != 0) {
+        ntuple_promote_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, weights, reinterpret_cast<float2 *>(coherence),
+                                                            reinterpret_cast<uint32_t *>(promoted), spec, num_games);
+        if (const int rc = launch_status()) return rc;
+    }
     return with_spec(spec, [&](const auto &sp) {
         if (!coherence) {
             ntuple_td_scatter_kernel<<<grid, kStepThreads, 0, s>>>(x0, mask, delta, weights, sp, num_games);
@@ -2580,9 +2705,9 @@ static int apply_update(const uint4 *x0, const uint8_t *mask, const float *delta
     });
 }
 
-int ml2048_staged_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
-                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
-                            float *delta_out, int64_t num_games, void *stream)
+static int td_update_entry(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                           const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                           uint8_t *promoted, float *delta_out, int64_t num_games, void *stream)
 {
     NTupleStagedSpec spec;
     unsigned grid = 0;
@@ -2591,8 +2716,25 @@ int ml2048_staged_td_update(const void *after, const float *target, const uint8_
         return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
-    return apply_update(b, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
+    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, promoted, delta_out, grid, num_games, s)) return rc;
+    return apply_update(b, mask, delta_out, weights, nullptr, nullptr, spec, promoted, grid, num_games, s);
+}
+
+int ml2048_staged_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                            const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp, int32_t num_stages,
+                            float *delta_out, int64_t num_games, void *stream)
+{
+    return td_update_entry(after, target, mask, alpha, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, nullptr,
+                           delta_out, num_games, stream);
+}
+
+int ml2048_promoted_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights,
+                              int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
+                              int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return td_update_entry(after, target, mask, alpha, weights, num_weights, cells, len, num_tuples, stage_exp, num_stages, promoted,
+                           delta_out, num_games, stream);
 }
 
 int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
@@ -2602,9 +2744,10 @@ int ml2048_ntuple_td_update(const void *after, const float *target, const uint8_
                                    stream);
 }
 
-int ml2048_staged_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
-                            float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
-                            const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+static int tc_update_entry(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                           float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                           const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games,
+                           void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!coherence || !accum) return ML2048_E_NULL;
@@ -2616,8 +2759,26 @@ int ml2048_staged_tc_update(const void *after, const float *target, const uint8_
         return rc;
     const uint4 *b = reinterpret_cast<const uint4 *>(after);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, delta_out, grid, num_games, s)) return rc;
-    return apply_update(b, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
+    if (const int rc = target_delta(b, target, mask, alpha, weights, spec, promoted, delta_out, grid, num_games, s)) return rc;
+    return apply_update(b, mask, delta_out, weights, coherence, accum, spec, promoted, grid, num_games, s);
+}
+
+int ml2048_staged_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                            float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                            const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+{
+    return tc_update_entry(after, target, mask, alpha, weights, coherence, accum, num_weights, cells, len, num_tuples, stage_exp, num_stages,
+                           nullptr, delta_out, num_games, stream);
+}
+
+int ml2048_promoted_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                              float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                              const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games,
+                              void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return tc_update_entry(after, target, mask, alpha, weights, coherence, accum, num_weights, cells, len, num_tuples, stage_exp, num_stages,
+                           promoted, delta_out, num_games, stream);
 }
 
 int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask, float alpha, float *weights, float *coherence,
@@ -2628,10 +2789,10 @@ int ml2048_tc_update(const void *after, const float *target, const uint8_t *mask
                                    delta_out, num_games, stream);
 }
 
-int ml2048_staged_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
-                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
-                                   const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
-                                   int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+static int lambda_td_update_entry(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                  int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                                  const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
+                                  int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games, void *stream)
 {
     NTupleStagedSpec spec;
     unsigned grid = 0;
@@ -2641,9 +2802,28 @@ int ml2048_staged_lambda_td_update(const void *after_ring, const float *reward_r
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint4 *x0 = nullptr;
     if (const int rc = lambda_delta(reinterpret_cast<const uint4 *>(after_ring), reward_ring, ended_ring, horizon, newest, lambda, mask, alpha,
-                                    weights, spec, delta_out, grid, num_games, s, x0))
+                                    weights, spec, promoted, delta_out, grid, num_games, s, x0))
         return rc;
-    return apply_update(x0, mask, delta_out, weights, nullptr, nullptr, spec, grid, num_games, s);
+    return apply_update(x0, mask, delta_out, weights, nullptr, nullptr, spec, promoted, grid, num_games, s);
+}
+
+int ml2048_staged_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                                   const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
+                                   int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+{
+    return lambda_td_update_entry(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells, len,
+                                  num_tuples, stage_exp, num_stages, nullptr, delta_out, num_games, stream);
+}
+
+int ml2048_promoted_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                     int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, int64_t num_weights,
+                                     const uint8_t *cells, const uint8_t *len, int32_t num_tuples, const uint8_t *stage_exp,
+                                     int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return lambda_td_update_entry(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, num_weights, cells, len,
+                                  num_tuples, stage_exp, num_stages, promoted, delta_out, num_games, stream);
 }
 
 int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,
@@ -2654,10 +2834,11 @@ int ml2048_lambda_td_update(const void *after_ring, const float *reward_ring, co
                                           cells, len, num_tuples, nullptr, 1, delta_out, num_games, stream);
 }
 
-int ml2048_staged_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
-                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
-                                   float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
-                                   const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+static int lambda_tc_update_entry(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                  int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                  float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                  const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted, float *delta_out, int64_t num_games,
+                                  void *stream)
 {
     if (num_games <= 0) return ML2048_E_SIZE;
     if (!coherence || !accum) return ML2048_E_NULL;
@@ -2670,9 +2851,29 @@ int ml2048_staged_lambda_tc_update(const void *after_ring, const float *reward_r
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint4 *x0 = nullptr;
     if (const int rc = lambda_delta(reinterpret_cast<const uint4 *>(after_ring), reward_ring, ended_ring, horizon, newest, lambda, mask, alpha,
-                                    weights, spec, delta_out, grid, num_games, s, x0))
+                                    weights, spec, promoted, delta_out, grid, num_games, s, x0))
         return rc;
-    return apply_update(x0, mask, delta_out, weights, coherence, accum, spec, grid, num_games, s);
+    return apply_update(x0, mask, delta_out, weights, coherence, accum, spec, promoted, grid, num_games, s);
+}
+
+int ml2048_staged_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                   int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                   float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                   const uint8_t *stage_exp, int32_t num_stages, float *delta_out, int64_t num_games, void *stream)
+{
+    return lambda_tc_update_entry(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, coherence, accum,
+                                  num_weights, cells, len, num_tuples, stage_exp, num_stages, nullptr, delta_out, num_games, stream);
+}
+
+int ml2048_promoted_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon,
+                                     int32_t newest, float lambda, const uint8_t *mask, float alpha, float *weights, float *coherence,
+                                     float *accum, int64_t num_weights, const uint8_t *cells, const uint8_t *len, int32_t num_tuples,
+                                     const uint8_t *stage_exp, int32_t num_stages, uint8_t *promoted, float *delta_out,
+                                     int64_t num_games, void *stream)
+{
+    if (const int rc = check_promoted(promoted)) return rc;
+    return lambda_tc_update_entry(after_ring, reward_ring, ended_ring, horizon, newest, lambda, mask, alpha, weights, coherence, accum,
+                                  num_weights, cells, len, num_tuples, stage_exp, num_stages, promoted, delta_out, num_games, stream);
 }
 
 int ml2048_lambda_tc_update(const void *after_ring, const float *reward_ring, const uint8_t *ended_ring, int32_t horizon, int32_t newest,

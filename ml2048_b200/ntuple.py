@@ -7,7 +7,8 @@ adds: each is one kernel here (``ops.ntuple_value``, ``ops.ntuple_greedy``, ``op
 learning, a step size per weight, is ``ops.ntuple_tc_update`` and ``TDAfterstateLearner(..., rule="tc")``; their delayed
 lambda-return forms are ``ops.ntuple_td_lambda_update`` / ``ntuple_tc_lambda_update`` and ``TDAfterstateLearner(...,
 horizon=h, lam=lam)``).  ``NTupleNetwork(..., stages=(tau_1, ...))`` is a multi-stage network (Yeh et al. 2016): one weight
-set per stage of the game, chosen by the board's largest tile (``ops.ntuple_stages``).
+set per stage of the game, chosen by the board's largest tile (``ops.ntuple_stages``); with ``promotion=True`` a stage's entry
+starts from the stage below on its first update (Jaskowski 2018).
 
     net = NTupleNetwork(device="cuda")                        # the standard 4x6 network, zero weights (256 MiB)
     env = VecGame(16384, output="torch", sync_free=True)
@@ -72,11 +73,18 @@ class NTupleNetwork:
     ``stages``: 0..7 strictly ascending tile exponents tau_1 < ... in 1..15 (``ops.ntuple_stages``) make a multi-stage network
     of S = len(stages) + 1 weight sets.  A board b is in stage #{k : tau_k <= max_c min(b[c], 15)}, and is valued and updated
     with that stage's tables; the weights are S * N entries, stage s's tables at s * N (N = sum 16^len), and ``coherence``
-    is (S * N, 2).  ``stages=()`` is the single-stage network."""
+    is (S * N, 2).  ``stages=()`` is the single-stage network.
 
-    def __init__(self, tuples=STANDARD_4X6, device: Any = None, *, stages=()):
+    ``promotion=True`` (multi-stage only) adds weight promotion (Jaskowski 2018): ``promoted`` is an (N,) uint8 tensor of
+    marks, all clear at first, so that every stage >= 1 starts as stage 0.  Each op reads an unwritten entry of stage s
+    through stage s - 1, and an update first copies that value into every entry it is about to change (``ops.ntuple_value``,
+    ``ops.ntuple_td_update``).  ``promoted`` is None without promotion."""
+
+    def __init__(self, tuples=STANDARD_4X6, device: Any = None, *, stages=(), promotion: bool = False):
         self.tuples = ops.ntuple_spec(tuples)
         self.stages = ops.ntuple_stages(stages)
+        if promotion and not self.stages:
+            raise ValueError("promotion=True needs a multi-stage network (stages=...)")
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device={device!r}: ml2048_b200 runs on CUDA only")
@@ -89,33 +97,34 @@ class NTupleNetwork:
             self.offsets.append(total)
             total += 16 ** len(t)
         self.weights = torch.zeros(((len(self.stages) + 1) * total,), dtype=torch.float32, device=dev)
+        self.promoted: Optional[torch.Tensor] = torch.zeros((total,), dtype=torch.uint8, device=dev) if promotion else None
         # TC learning's {E, A} per weight and the TC updates' scratch (all zero between calls), allocated by the first TC update
         self.coherence: Optional[torch.Tensor] = None
         self._tc_accum: Optional[torch.Tensor] = None
 
     def value(self, board: torch.Tensor, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """V of (M,16) boards: (M,) float32 (``ops.ntuple_value``)."""
-        return ops.ntuple_value(board, self.weights, self.tuples, out=out, stages=self.stages)
+        return ops.ntuple_value(board, self.weights, self.tuples, out=out, stages=self.stages, promoted=self.promoted)
 
     def greedy(self, board: torch.Tensor, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
                out: Optional[dict] = None) -> dict:
         """The move maximising reward + V(afterstate): {"action", "state", "reward", "value"} (``ops.ntuple_greedy``)."""
         return ops.ntuple_greedy(board, self.weights, self.tuples, reward_fn=reward_fn, action_dtype=action_dtype, out=out,
-                                 stages=self.stages)
+                                 stages=self.stages, promoted=self.promoted)
 
     def expectimax(self, board: torch.Tensor, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
                    action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None) -> dict:
         """The expectimax move ``depth`` (1 or 2) chance layers deep: {"action", "state", "reward", "value", "q"}
         (``ops.ntuple_expectimax``)."""
         return ops.ntuple_expectimax(board, self.weights, self.tuples, depth=depth, two_prob=two_prob, reward_fn=reward_fn,
-                                     action_dtype=action_dtype, out=out, stages=self.stages)
+                                     action_dtype=action_dtype, out=out, stages=self.stages, promoted=self.promoted)
 
     def td_update(self, afterstate: torch.Tensor, target: torch.Tensor, alpha: float, *, mask: Optional[torch.Tensor] = None,
                   delta_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """One synchronous TD(0) batch toward ``target``; returns delta = alpha * (target - V) (``ops.ntuple_td_update``).
         The adds are float atomics: the weights are reproducible up to the fp32 rounding of their order."""
         return ops.ntuple_td_update(afterstate, target, self.weights, self.tuples, alpha=alpha, mask=mask, delta_out=delta_out,
-                                    stages=self.stages)
+                                    stages=self.stages, promoted=self.promoted)
 
     def _tc_alloc(self) -> None:
         if self.coherence is None:
@@ -130,7 +139,7 @@ class NTupleNetwork:
         and a zero scratch accumulator of the same shape."""
         self._tc_alloc()
         return ops.ntuple_tc_update(afterstate, target, self.weights, self.coherence, self._tc_accum, self.tuples, alpha=alpha,
-                                    mask=mask, delta_out=delta_out, stages=self.stages)
+                                    mask=mask, delta_out=delta_out, stages=self.stages, promoted=self.promoted)
 
     def td_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                          alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
@@ -138,7 +147,7 @@ class NTupleNetwork:
         """One synchronous delayed TD(lambda) batch over the caller's ring of each game's last h + 1 afterstates; returns
         delta = alpha * (R_0 - V(x_0)) (``ops.ntuple_td_lambda_update``)."""
         return ops.ntuple_td_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.tuples, alpha=alpha,
-                                           lam=lam, mask=mask, delta_out=delta_out, stages=self.stages)
+                                           lam=lam, mask=mask, delta_out=delta_out, stages=self.stages, promoted=self.promoted)
 
     def tc_lambda_update(self, after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                          alpha: float, lam: float, *, mask: Optional[torch.Tensor] = None,
@@ -148,18 +157,25 @@ class NTupleNetwork:
         self._tc_alloc()
         return ops.ntuple_tc_lambda_update(after_ring, reward_ring, ended_ring, newest, self.weights, self.coherence,
                                            self._tc_accum, self.tuples, alpha=alpha, lam=lam, mask=mask, delta_out=delta_out,
-                                           stages=self.stages)
+                                           stages=self.stages, promoted=self.promoted)
 
     def state_dict(self) -> dict:
         state = {"tuples": [list(t) for t in self.tuples], "stages": list(self.stages), "weights": self.weights.detach().clone()}
         if self.coherence is not None:
             state["coherence"] = self.coherence.detach().clone()
+        if self.promoted is not None:
+            state["promoted"] = self.promoted.detach().clone()
         return state
 
     def load_state_dict(self, state: dict) -> None:
         """Loads the weights and, when ``state`` has them, the TC coherence sums; a dict without ``"coherence"`` drops any
         coherence state this network has (the next ``tc_update`` starts from zeros).  A dict without ``"stages"`` is a
-        single-stage network's (``stages=()``)."""
+        single-stage network's (``stages=()``).
+
+        Promotion marks (``"promoted"``): a promoting network copies them from a dict that has them; from a dict without them
+        it sets every stage's mark (bits 0..S-2) of every entry, so that it values every board as the saved network did.  A
+        non-promoting network loads a dict with marks as its effective weights (``ops.ntuple_promoted_weights``), with the
+        coherence of every unmarked entry of stages >= 1 zeroed, as a promotion would set it."""
         if ops.ntuple_spec(state["tuples"]) != self.tuples:
             raise ValueError(f"state_dict is for tuples {state['tuples']}, this network has {self.tuples}")
         if ops.ntuple_stages(state.get("stages", ())) != self.stages:
@@ -171,7 +187,26 @@ class NTupleNetwork:
         shape = (self.weights.numel(), 2)
         if c is not None and (not isinstance(c, torch.Tensor) or c.dtype != torch.float32 or tuple(c.shape) != shape):
             raise ValueError(f"coherence must be float32 {shape}")
+        p = state.get("promoted")
+        n = self.weights.numel() // (len(self.stages) + 1)
+        if p is not None and (not isinstance(p, torch.Tensor) or p.dtype != torch.uint8 or tuple(p.shape) != (n,)):
+            raise ValueError(f"promoted must be uint8 ({n},)")
+        if p is not None and self.promoted is None:
+            # marks into a network without them: the effective weights, and the coherence a promotion would leave
+            p = p.detach().to(self.device).contiguous()
+            w = ops.ntuple_promoted_weights(w.detach().to(self.device).contiguous(), p, self.tuples, self.stages)
+            if c is not None:
+                c = c.detach().to(self.device, copy=True).contiguous()
+                marked = torch.ones((len(self.stages) + 1, n), dtype=torch.bool, device=self.device)
+                for s in range(1, len(self.stages) + 1):
+                    marked[s] = (p & (1 << (s - 1))) != 0
+                c[~marked.view(-1)] = 0.0
         self.weights.copy_(w)
+        if self.promoted is not None:
+            if p is None:
+                self.promoted.fill_((1 << len(self.stages)) - 1)
+            else:
+                self.promoted.copy_(p)
         if c is None:
             self.coherence = None
         elif self.coherence is None:

@@ -292,6 +292,36 @@ def _weights_arg(weights: torch.Tensor, n: int, device, stages: int = 1) -> None
         raise ValueError(f"weights is on {weights.device}, the boards on {device}")
 
 
+def _promoted_arg(promoted, n: int, device) -> tuple:
+    """() without marks, else (pointer,) of checked marks: a contiguous (N,) uint8 CUDA tensor on ``device``, 4-byte aligned"""
+    if promoted is None:
+        return ()
+    if not (isinstance(promoted, torch.Tensor) and promoted.is_cuda and promoted.is_contiguous() and promoted.dtype == torch.uint8
+            and tuple(promoted.shape) == (n,) and promoted.device == device):
+        raise ValueError(f"promoted must be a contiguous uint8 ({n},) tensor on {device}")
+    if promoted.data_ptr() % 4:
+        raise ValueError("promoted must be 4-byte aligned (the marks are set with 32-bit atomics)")
+    return (promoted.data_ptr(),)
+
+
+def _entry(name: str, promoted: tuple) -> str:
+    """the library entry of op ``name``: ml2048_staged_* without marks, ml2048_promoted_* with them"""
+    return f"ml2048_{'promoted' if promoted else 'staged'}_{name}"
+
+
+def ntuple_promoted_weights(weights: torch.Tensor, promoted: torch.Tensor, tuples, stages) -> torch.Tensor:
+    """The S * N effective weights of a promoting network, a new tensor in the layout of ``weights``: W(0, e) = weights[e]
+    and, for s >= 1, W(s, e) = weights[s * N + e] where bit s - 1 of ``promoted[e]`` is set, else W(s - 1, e).  A staged op
+    on these weights gives what the op with ``promoted=promoted`` gives on ``weights``."""
+    cells, lens, k, tau, s, n = _network_args(tuples, stages)
+    _weights_arg(weights, n, getattr(weights, "device", None), s)
+    _promoted_arg(promoted, n // s, weights.device)
+    eff = weights.view(s, n // s).clone()
+    for st in range(1, s):
+        eff[st] = torch.where((promoted & (1 << (st - 1))) != 0, eff[st], eff[st - 1])
+    return eff.view(-1)
+
+
 def _ptr(a) -> Optional[int]:
     return None if a is None else a.ctypes.data
 
@@ -303,7 +333,7 @@ def _board_arg(board, name: str = "board") -> None:
 
 
 def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Optional[torch.Tensor] = None,
-                 stages=()) -> torch.Tensor:
+                 stages=(), promoted: Optional[torch.Tensor] = None) -> torch.Tensor:
     """V(board) of an n-tuple network: (M,16) uint8/int8 boards -> (M,) float32.
 
     ``tuples``: the network's cells (see ``ntuple_spec``); ``weights``: its one float32 tensor of sum 16^len entries, tuple t's
@@ -311,19 +341,27 @@ def ntuple_value(board: torch.Tensor, weights: torch.Tensor, tuples, *, out: Opt
     ``weights[offset_t + sum_j min(image_g[cell_tj], 15) << 4j]`` as float32 adds from 0 in that order: bit-reproducible.
     Every byte gives an in-bounds index; tiles 2^16 and above share the entries of 2^15.  ``out``: a preallocated (M,)
     float32 tensor (CUDA-graph capture).  ``stages``: the thresholds of a multi-stage network (``ntuple_stages``); its
-    ``weights`` hold S * sum 16^len entries and each board is valued with the tables of its own stage."""
+    ``weights`` hold S * sum 16^len entries and each board is valued with the tables of its own stage.
+
+    ``promoted``: the marks of a multi-stage network with weight promotion (Jaskowski 2018), a contiguous (N,) uint8 CUDA
+    tensor, N = sum 16^len for any S, or None (no promotion).  Bit s - 1 of ``promoted[e]`` is set once stage s's entry e has
+    been written; every op then reads the effective weight W(s, e) = weights[s * N + e] if that bit is set, else W(s - 1, e)
+    (W(0, e) = weights[e]), in the same float32 order as without marks (``ntuple_promoted_weights``).  The storage of an
+    unmarked entry is never read.  With one stage the marks are neither read nor written."""
     _board_arg(board)
     cells, lens, k, tau, s, n = _network_args(tuples, stages)
     _weights_arg(weights, n, board.device, s)
+    pm = _promoted_arg(promoted, n // s, board.device)
     m = board.shape[0]
     out = _out_arg(out, (m,), torch.float32, board.device, "out")
     if m == 0:
         return out
     lib = _lib.load()
+    fn = _entry("value", pm)
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_staged_value(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
-                                     out.data_ptr(), m, _stream(board))
-    _lib.check(rc, "ml2048_staged_value")
+        rc = getattr(lib, fn)(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, *pm,
+                              out.data_ptr(), m, _stream(board))
+    _lib.check(rc, fn)
     return out
 
 
@@ -339,7 +377,7 @@ def _move_outputs(out, specs: dict, action_dtype, board, op: str) -> dict:
 
 
 def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_fn=None, action_dtype: torch.dtype = torch.int64,
-                  out: Optional[dict] = None, stages=()) -> dict:
+                  out: Optional[dict] = None, stages=(), promoted: Optional[torch.Tensor] = None) -> dict:
     """The greedy afterstate move of every board under an n-tuple network, in one kernel.
 
     For every direction a that changes the board, q_a = reward_a + V(afterstate_a) in float32, with reward_a and afterstate_a
@@ -353,24 +391,27 @@ def ntuple_greedy(board: torch.Tensor, weights: torch.Tensor, tuples, *, reward_
 
     A board without a valid move gets action 0, its own board, reward 0 and value 0 (so a TD target reward + value is 0).
     ``out``: preallocated tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.
-    ``stages``: a multi-stage network (``ntuple_stages``); each afterstate is valued with the tables of its own stage."""
+    ``stages``: a multi-stage network (``ntuple_stages``); each afterstate is valued with the tables of its own stage.
+    ``promoted``: the network's promotion marks (``ntuple_value``), or None."""
     _board_arg(board)
     if action_dtype not in (torch.int64, torch.uint8):
         raise ValueError("action_dtype must be torch.int64 or torch.uint8")
     kind = reward_kind(reward_fn)
     cells, lens, k, tau, s, n = _network_args(tuples, stages)
     _weights_arg(weights, n, board.device, s)
+    pm = _promoted_arg(promoted, n // s, board.device)
     m = board.shape[0]
     res = _move_outputs(out, _NTUPLE_GREEDY, action_dtype, board, "ntuple_greedy")
     if m == 0:
         return res
     act = res["action"].data_ptr()
     lib = _lib.load()
+    fn = _entry("greedy", pm)
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_staged_greedy(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, kind,
-                                      act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
-                                      res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), m, _stream(board))
-    _lib.check(rc, "ml2048_staged_greedy")
+        rc = getattr(lib, fn)(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, *pm, kind,
+                              act if action_dtype == torch.uint8 else None, act if action_dtype == torch.int64 else None,
+                              res["state"].data_ptr(), res["reward"].data_ptr(), res["value"].data_ptr(), m, _stream(board))
+    _lib.check(rc, fn)
     return res
 
 
@@ -378,7 +419,8 @@ _NTUPLE_EXPECTIMAX = dict(_NTUPLE_GREEDY, q=((4,), torch.float32))
 
 
 def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, depth: int = 1, two_prob: float = 0.8, reward_fn=None,
-                      action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None, stages=()) -> dict:
+                      action_dtype: torch.dtype = torch.int64, out: Optional[dict] = None, stages=(),
+                      promoted: Optional[torch.Tensor] = None) -> dict:
     """The expectimax move of every board under an n-tuple network, ``depth`` (1 or 2) chance layers deep, in one kernel.
 
     Definition (every operation one float32 operation; after, r, valid as ``afterstates(board, reward_fn=reward_fn)`` gives
@@ -404,7 +446,8 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
 
     A board without a valid move gets action 0, its own board, reward 0, value 0 and q all -inf.  ``out``: preallocated
     tensors under the same keys (any subset), so that the call can be captured in a CUDA graph.  Cells must be 0..17.
-    ``stages``: a multi-stage network (``ntuple_stages``); each leaf is valued with the tables of its own stage."""
+    ``stages``: a multi-stage network (``ntuple_stages``); each leaf is valued with the tables of its own stage.
+    ``promoted``: the network's promotion marks (``ntuple_value``), or None."""
     _board_arg(board)
     if action_dtype not in (torch.int64, torch.uint8):
         raise ValueError("action_dtype must be torch.int64 or torch.uint8")
@@ -419,18 +462,20 @@ def ntuple_expectimax(board: torch.Tensor, weights: torch.Tensor, tuples, *, dep
     kind = reward_kind(reward_fn)
     cells, lens, k, tau, s, n = _network_args(tuples, stages)
     _weights_arg(weights, n, board.device, s)
+    pm = _promoted_arg(promoted, n // s, board.device)
     m = board.shape[0]
     res = _move_outputs(out, _NTUPLE_EXPECTIMAX, action_dtype, board, "ntuple_expectimax")
     if m == 0:
         return res
     act = res["action"].data_ptr()
     lib = _lib.load()
+    fn = _entry("expectimax", pm)
     with torch.cuda.device(board.device):
-        rc = lib.ml2048_staged_expectimax(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
-                                          kind, int(depth), p, act if action_dtype == torch.uint8 else None,
-                                          act if action_dtype == torch.int64 else None, res["state"].data_ptr(), res["reward"].data_ptr(),
-                                          res["value"].data_ptr(), res["q"].data_ptr(), m, _stream(board))
-    _lib.check(rc, "ml2048_staged_expectimax")
+        rc = getattr(lib, fn)(board.data_ptr(), weights.data_ptr(), n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, *pm, kind,
+                              int(depth), p, act if action_dtype == torch.uint8 else None,
+                              act if action_dtype == torch.int64 else None, res["state"].data_ptr(), res["reward"].data_ptr(),
+                              res["value"].data_ptr(), res["q"].data_ptr(), m, _stream(board))
+    _lib.check(rc, fn)
     return res
 
 
@@ -443,8 +488,9 @@ def _coherence_args(coherence, accum, n: int, device) -> tuple[int, int]:
     return coherence.data_ptr(), accum.data_ptr()
 
 
-def _target_update(fn: str, afterstate, target, weights, tuples, stages, alpha, mask, delta_out, tc=None) -> torch.Tensor:
-    """ntuple_td_update (tc None) and ntuple_tc_update (tc = (coherence, accum)) through library function ``fn``"""
+def _target_update(op: str, afterstate, target, weights, tuples, stages, promoted, alpha, mask, delta_out, tc=None) -> torch.Tensor:
+    """ntuple_td_update (tc None) and ntuple_tc_update (tc = (coherence, accum)) through the library entry of ``op``
+    (``_entry``)"""
     _board_arg(afterstate, "afterstate")
     m = afterstate.shape[0]
     _cuda(target, "target")
@@ -457,20 +503,23 @@ def _target_update(fn: str, afterstate, target, weights, tuples, stages, alpha, 
     cells, lens, k, tau, s, n = _network_args(tuples, stages)
     _weights_arg(weights, n, afterstate.device, s)
     tc_ptrs = () if tc is None else _coherence_args(*tc, n, afterstate.device)
+    pm = _promoted_arg(promoted, n // s, afterstate.device)
     delta_out = _out_arg(delta_out, (m,), torch.float32, afterstate.device, "delta_out")
     if m == 0:
         return delta_out
     lib = _lib.load()
+    fn = _entry(op, pm)
     with torch.cuda.device(afterstate.device):
         rc = getattr(lib, fn)(afterstate.data_ptr(), target.data_ptr(), mask.data_ptr() if mask is not None else None, float(alpha),
-                              weights.data_ptr(), *tc_ptrs, n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s,
+                              weights.data_ptr(), *tc_ptrs, n, cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, *pm,
                               delta_out.data_ptr(), m, _stream(afterstate))
     _lib.check(rc, fn)
     return delta_out
 
 
 def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, tuples, *, alpha: float,
-                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
+                     mask: Optional[torch.Tensor] = None, delta_out: Optional[torch.Tensor] = None, stages=(),
+                     promoted: Optional[torch.Tensor] = None) -> torch.Tensor:
     """One synchronous batch of TD(0) updates of an n-tuple network, in place on ``weights``; returns delta (M,) float32.
 
     Phase 1: delta_i = alpha * (target_i - V(afterstate_i)) with the weights as they were before the call, 0 for a game
@@ -478,13 +527,18 @@ def ntuple_td_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
     8 per tuple, gets += delta_i.  Phase 2 adds with float atomics, so the order of the adds that several games make to one
     entry is unspecified: the weights are reproducible only up to the fp32 rounding of that order.  delta is deterministic.
     ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture).  ``stages``: a multi-stage network
-    (``ntuple_stages``); V(afterstate_i) and the update use the tables of afterstate_i's stage."""
-    return _target_update("ml2048_staged_td_update", afterstate, target, weights, tuples, stages, alpha, mask, delta_out)
+    (``ntuple_stages``); V(afterstate_i) and the update use the tables of afterstate_i's stage.
+
+    ``promoted``: the marks of a network with weight promotion (``ntuple_value``), updated in place.  delta is computed with
+    the effective weights before the call; then every masked-in game whose afterstate is in a stage s >= 1 (whatever its
+    delta, 0 included) promotes each of its entries e whose mark of (s, e) is clear: weights[s * N + e] = W(s - 1, e), and
+    the mark is set.  Promotion changes no effective weight.  Phase 2 then adds to the entries of the afterstate's stage."""
+    return _target_update("td_update", afterstate, target, weights, tuples, stages, promoted, alpha, mask, delta_out)
 
 
 def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: torch.Tensor, coherence: torch.Tensor,
                      accum: torch.Tensor, tuples, *, alpha: float, mask: Optional[torch.Tensor] = None,
-                     delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
+                     delta_out: Optional[torch.Tensor] = None, stages=(), promoted: Optional[torch.Tensor] = None) -> torch.Tensor:
     """One synchronous batch of temporal coherence (TC) updates of an n-tuple network, in place on ``weights`` and
     ``coherence``; returns delta (M,) float32.
 
@@ -503,17 +557,20 @@ def ntuple_tc_update(afterstate: torch.Tensor, target: torch.Tensor, weights: to
     older errors by the alpha they had.  ``coherence`` and ``accum``: contiguous float32 (N, 2) tensors on the weights'
     device; ``accum`` is scratch that must be all zero and is left all zero.  ``delta_out``: a preallocated (M,) float32
     tensor (CUDA-graph capture).  ``stages``: a multi-stage network (``ntuple_stages``); ``weights`` has S * N entries,
-    ``coherence`` and ``accum`` are (S * N, 2), and afterstate_i's value and update use the entries of its stage."""
-    return _target_update("ml2048_staged_tc_update", afterstate, target, weights, tuples, stages, alpha, mask, delta_out,
+    ``coherence`` and ``accum`` are (S * N, 2), and afterstate_i's value and update use the entries of its stage.
+    ``promoted``: as for ``ntuple_td_update``; a promoted entry's coherence is set to (0, 0), so its first TC step has
+    beta = 1."""
+    return _target_update("tc_update", afterstate, target, weights, tuples, stages, promoted, alpha, mask, delta_out,
                           (coherence, accum))
 
 
 NTUPLE_LAMBDA_MAX_HORIZON = 16
 
 
-def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha, lam, mask, delta_out,
-                   tc=None) -> torch.Tensor:
-    """ntuple_td_lambda_update (tc None) and ntuple_tc_lambda_update (tc = (coherence, accum)) through library function ``fn``"""
+def _lambda_update(op: str, after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, promoted, alpha, lam, mask,
+                   delta_out, tc=None) -> torch.Tensor:
+    """ntuple_td_lambda_update (tc None) and ntuple_tc_lambda_update (tc = (coherence, accum)) through the library entry of
+    ``op`` (``_entry``)"""
     if not (isinstance(after_ring, torch.Tensor) and after_ring.dtype in (torch.uint8, torch.int8) and after_ring.ndim == 3
             and after_ring.shape[2] == 16):
         raise ValueError("after_ring must be uint8/int8 (h+1, M, 16)")
@@ -542,21 +599,24 @@ def _lambda_update(fn: str, after_ring, reward_ring, ended_ring, newest, weights
     cells, lens, k, tau, s, n = _network_args(tuples, stages)
     _weights_arg(weights, n, dev, s)
     tc_ptrs = () if tc is None else _coherence_args(*tc, n, dev)
+    pm = _promoted_arg(promoted, n // s, dev)
     delta_out = _out_arg(delta_out, (m,), torch.float32, dev, "delta_out")
     if m == 0:
         return delta_out
     lib = _lib.load()
+    fn = _entry(op, pm)
     with torch.cuda.device(dev):
         rc = getattr(lib, fn)(after_ring.data_ptr(), reward_ring.data_ptr(), ended_ring.data_ptr(), h, newest, lam,
                               mask.data_ptr() if mask is not None else None, float(alpha), weights.data_ptr(), *tc_ptrs, n,
-                              cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, delta_out.data_ptr(), m, _stream(after_ring))
+                              cells.ctypes.data, lens.ctypes.data, k, _ptr(tau), s, *pm, delta_out.data_ptr(), m, _stream(after_ring))
     _lib.check(rc, fn)
     return delta_out
 
 
 def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                             weights: torch.Tensor, tuples, *, alpha: float, lam: float, mask: Optional[torch.Tensor] = None,
-                            delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
+                            delta_out: Optional[torch.Tensor] = None, stages=(),
+                            promoted: Optional[torch.Tensor] = None) -> torch.Tensor:
     """One synchronous batch of delayed TD(lambda) updates of an n-tuple network (Jaskowski 2018), in place on ``weights``:
     each game's afterstate of h learner steps ago moves toward a lambda-return truncated at h.  Returns delta (M,) float32.
 
@@ -576,20 +636,23 @@ def ntuple_td_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor,
     (h+1, M) bool/uint8, all contiguous on one device, h = ``after_ring.shape[0] - 1`` in 1..16.  ``newest`` is the slot of
     x_h; x_k is in slot (newest - (h - k)) mod (h + 1), and ``ended_ring[newest]`` is not read.  ``mask``: (M,) bool/uint8,
     None = every game.  ``delta_out``: a preallocated (M,) float32 tensor (CUDA-graph capture).  ``stages``: a multi-stage
-    network (``ntuple_stages``); each V_k uses the tables of x_k's stage, and the update writes the entries of x_0's stage."""
-    return _lambda_update("ml2048_staged_lambda_td_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha,
+    network (``ntuple_stages``); each V_k uses the tables of x_k's stage, and the update writes the entries of x_0's stage.
+    ``promoted``: as for ``ntuple_td_update``: every V_k reads the effective weights, and x_0's entries are promoted before
+    the adds."""
+    return _lambda_update("lambda_td_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, promoted, alpha,
                           lam, mask, delta_out)
 
 
 def ntuple_tc_lambda_update(after_ring: torch.Tensor, reward_ring: torch.Tensor, ended_ring: torch.Tensor, newest: int,
                             weights: torch.Tensor, coherence: torch.Tensor, accum: torch.Tensor, tuples, *, alpha: float,
                             lam: float, mask: Optional[torch.Tensor] = None,
-                            delta_out: Optional[torch.Tensor] = None, stages=()) -> torch.Tensor:
+                            delta_out: Optional[torch.Tensor] = None, stages=(),
+                            promoted: Optional[torch.Tensor] = None) -> torch.Tensor:
     """One synchronous batch of delayed TC(lambda) updates, in place on ``weights`` and ``coherence``; returns delta (M,)
     float32.  delta is ``ntuple_td_lambda_update``'s (the same window, ring, definition and arguments); the update of x_0's
     entries is then ``ntuple_tc_update``'s phases 2 and 3: {dE, dA} += {delta, |delta|} into ``accum``, and w += beta * dE,
     beta = |E| / A (1 where A = 0), {E, A} += {dE, dA} for every entry with dA != 0.  ``coherence`` and ``accum``: contiguous
     float32 (N, 2) tensors on the ring's device; ``accum`` must be all zero and is left all zero.  ``stages``: as for
-    ``ntuple_td_lambda_update``, with ``coherence`` and ``accum`` (S * N, 2)."""
-    return _lambda_update("ml2048_staged_lambda_tc_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, alpha,
+    ``ntuple_td_lambda_update``, with ``coherence`` and ``accum`` (S * N, 2).  ``promoted``: as for ``ntuple_tc_update``."""
+    return _lambda_update("lambda_tc_update", after_ring, reward_ring, ended_ring, newest, weights, tuples, stages, promoted, alpha,
                           lam, mask, delta_out, (coherence, accum))
