@@ -144,6 +144,22 @@ def tc_update_f32(after, delta, weights, coherence, tuples, stages, mask=None):
     return tc_apply_f32(de, da, weights, coherence)
 
 
+def tc_apply_f64(after, delta, weights, coherence, tuples, stages, mask=None):
+    """tref.tc_apply_f64 per stage: (weights, E, A, adds per entry, sum |delta| per entry), each (S * N,)"""
+    n = nref.num_weights(tuples)
+    w = _slices(np.asarray(weights, np.float64), tuples, stages).copy()
+    c = np.asarray(coherence, np.float32).reshape(num_stages(stages), n, 2)
+    e64, a64 = c[..., 0].astype(np.float64), c[..., 1].astype(np.float64)
+    adds, sabs = np.zeros(w.shape, np.int64), np.zeros(w.shape, np.float64)
+    mask = np.ones(after.shape[0], bool) if mask is None else np.asarray(mask).astype(bool)
+
+    def run(sel, s):
+        w[s], e64[s], a64[s], adds[s], sabs[s] = tref.tc_apply_f64(after[sel], delta[sel], w[s], c[s], tuples, mask[sel])
+
+    _per_stage(after, tuples, stages, run)
+    return w.reshape(-1), e64.reshape(-1), a64.reshape(-1), adds.reshape(-1), sabs.reshape(-1)
+
+
 def ring_delta(after_ring, reward_ring, ended_ring, newest: int, weights, tuples, stages, lam: float, alpha: float, mask=None):
     """(delta, x_0 boards) of a ring: lref.lambda_delta over values that each window board takes on its own stage"""
     after = lref.window(np.asarray(after_ring), newest)

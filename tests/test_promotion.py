@@ -8,6 +8,9 @@ Weight promotion of multi-stage n-tuple networks on the GPU (the ``promoted=`` a
 - Updates (TD(0), TC, TD(lambda), TC(lambda)) on integer data: weights, coherence, marks and delta bit for bit, canaries
   around every buffer, stage 0 and the stages no x_0 is in untouched; crafted boards that hit one entry in two or three
   stages within one call; a second call promotes nothing new.
+- The promote kernel's race at scale: M = 2^20 + 3 games over 2048 race boards in stages 1..7 of S = 8, every mark clear
+  and NaN behind it; alpha = 0 (promotion only) bit for bit for all four rules, a second call promotes nothing, then one
+  alpha = 1/16 call whose every partial sum is exact, bit for bit.
 - All marks set is the staged op bit for bit and leaves the marks; S = 1 with marks is the single-stage op bit for bit.
 - CUDA-graph replay of greedy + each update equals eager; the learner, state_dict's three load rules and both policies.
 """
@@ -84,15 +87,15 @@ def test_reads_bit_exact(ops, played, case):
     assert torch.equal(pm.cpu(), torch.from_numpy(marks)), "a read wrote the marks"
 
 
-def _race_boards(stages, tuples) -> np.ndarray:
+def _race_boards(stages, tuples, bases: int = 24, seed: int = 7) -> np.ndarray:
     """boards with identical tuple cells but their largest tile outside every tuple, one per stage: the same entry e of
     several stages in one call"""
     cells = sorted({c for t in tuples for c in t})
     free = [c for c in range(16) if c not in cells]
     assert free, "every cell is in a tuple"
-    rng = np.random.default_rng(7)
+    rng = np.random.default_rng(seed)
     out = []
-    for _ in range(24):
+    for _ in range(bases):
         base = np.zeros(16, np.uint8)
         base[cells] = rng.integers(0, 2, len(cells))
         for top in [1] + list(stages):
@@ -201,6 +204,96 @@ def test_updates_exact(ops, played, case, rule):
             np.testing.assert_array_equal(got_m, m_before, "a second call promoted something new")
     for ok in (w_ok, pm_ok, d_ok, c_ok, acc_ok):
         ok()
+
+
+def _race_call(ops, rule, dev, x0, k, w_dev, c_dev, acc, tuples, stages, pm, mk, d_dev, alpha):
+    """one update whose every x_0 is x0 and whose delta is alpha * k: TD(0) / TC toward V(x0) + k; the lambda rules with
+    h = 1, x_1 = x_0 and reward k, whose return is then k + V(x0) as well"""
+    b = torch.from_numpy(x0).to(dev)
+    kk = torch.from_numpy(k).to(dev)
+    kw = dict(alpha=alpha, mask=mk, delta_out=d_dev, stages=stages, promoted=pm)
+    if rule in ("td0", "tc"):
+        target = ops.ntuple_value(b, w_dev, tuples, stages=stages, promoted=pm) + kk
+        if rule == "td0":
+            ops.ntuple_td_update(b, target, w_dev, tuples, **kw)
+        else:
+            ops.ntuple_tc_update(b, target, w_dev, c_dev, acc, tuples, **kw)
+        return
+    ring = (torch.stack([b, b]), torch.stack([kk, kk]), torch.zeros((2, b.shape[0]), dtype=torch.uint8, device=dev), 1)
+    if rule == "lambda_td":
+        ops.ntuple_td_lambda_update(*ring, w_dev, tuples, lam=0.5, **kw)
+    else:
+        ops.ntuple_tc_lambda_update(*ring, w_dev, c_dev, acc, tuples, lam=0.5, **kw)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("rule", ["td0", "tc", "lambda_td", "lambda_tc"])
+def test_promotion_race_at_scale(ops, rule):
+    """M = 2^20 + 3 games over 2048 race boards (256 bases, one board per stage 1..7 of S = 8), so that every entry is met by
+    many games in several stages within one launch, from clear marks and NaN behind every one of them.
+
+    alpha = 0: the call only promotes, and what it promotes does not depend on the order in which the games meet an entry,
+    so weights, marks and coherence must equal the reference bit for bit; no touched effective weight is NaN; a second call
+    promotes nothing.  Then one alpha = 1/16 call, again from clear marks, with delta = k / 16 (k in {-1, 0, 1}): every
+    partial sum of an entry is a multiple of 1/16 below 2^24 / 16 (asserted), so it is exact in any order, and weights,
+    coherence and marks are bit for bit too.  4.7 s per rule on one B200 (power limit not recorded), most of it the host
+    reference."""
+    dev = _gpu()
+    stages, tuples = tuple(range(1, 8)), RACE_TUPLES
+    n = nref.num_weights(tuples)
+    rng = np.random.default_rng(600 + ["td0", "tc", "lambda_td", "lambda_tc"].index(rule))
+    pool = _race_boards(stages, tuples, bases=256, seed=11)
+    m = (1 << 20) + 3
+    x0 = pool[rng.integers(0, pool.shape[0], m)]
+    mask = (rng.random(m) < 0.9).astype(np.uint8)
+    keep = mask.astype(bool)
+    assert set(sref.stage(x0[keep], stages).tolist()) == set(range(1, 8))
+    distinct = np.unique(x0[keep], axis=0)  # promotion is idempotent: duplicates of a board promote nothing more
+    w = _poisoned(_stage_weights(rng, tuples, stages, integer=True), np.zeros(n, np.uint8), tuples, stages)
+    coh = rng.integers(-20, 21, size=(w.size, 2)).astype(np.float32)
+    coh[:, 1] = np.abs(coh[:, 1]) + np.abs(coh[:, 0])
+    tc = rule in ("tc", "lambda_tc")
+    w_dev = torch.from_numpy(w).to(dev)
+    c_dev = torch.from_numpy(coh).to(dev)
+    acc = torch.zeros((w.size, 2), device=dev)
+    pm = torch.zeros(n, dtype=torch.uint8, device=dev)
+    mk = torch.from_numpy(mask).to(dev)
+    d_dev = torch.empty(m, device=dev)
+    k = rng.integers(-1, 2, size=m).astype(np.float32)
+    want_w, want_m, want_c = pref.promote(distinct, w, np.zeros(n, np.uint8), tuples, stages, None, coh if tc else None)
+    ent = sref.entries(distinct, tuples, stages)
+    for call in range(2):
+        _race_call(ops, rule, dev, x0, k, w_dev, c_dev, acc, tuples, stages, pm, mk, d_dev, 0.0)
+        _same_bits(w_dev.cpu().numpy(), want_w, f"weights, call {call}")
+        np.testing.assert_array_equal(pm.cpu().numpy(), want_m, f"marks, call {call}")
+        _same_bits(c_dev.cpu().numpy(), want_c if tc else coh, f"coherence, call {call}")
+        assert not bool((d_dev != 0).any()), "alpha = 0 gave a delta other than +-0"
+        eff = ops.ntuple_promoted_weights(w_dev, pm, tuples, stages).cpu().numpy()
+        assert not np.isnan(eff[ent]).any(), "an effective weight of a touched entry is NaN"
+        assert not bool(acc.view(torch.int32).any())
+    # alpha = 1/16: every partial sum exact
+    adds = np.bincount(sref.entries(x0[keep], tuples, stages).ravel(), minlength=w.size)
+    start = max(np.abs(w[~np.isnan(w)]).max(), np.abs(coh).max())
+    assert 16 * start + adds.max() * 1 < 2 ** 24, (start, adds.max())  # in units of 1/16, |delta| <= 1/16
+    w = _poisoned(_stage_weights(rng, tuples, stages, integer=True), np.zeros(n, np.uint8), tuples, stages)
+    w_dev.copy_(torch.from_numpy(w))
+    c_dev.copy_(torch.from_numpy(coh))
+    pm.zero_()
+    _race_call(ops, rule, dev, x0, k, w_dev, c_dev, acc, tuples, stages, pm, mk, d_dev, 0.0625)
+    want_d = np.where(keep, k * np.float32(0.0625), np.float32(0)).astype(np.float32)
+    np.testing.assert_array_equal(d_dev.cpu().numpy(), want_d)
+    wp, want_m, cp = pref.promote(distinct, w, np.zeros(n, np.uint8), tuples, stages, None, coh if tc else None)
+    if tc:
+        _, e64, a64, _, _ = sref.tc_apply_f64(x0, want_d, wp, cp, tuples, stages, mask)
+        de, da = e64 - cp[:, 0].astype(np.float64), a64 - cp[:, 1].astype(np.float64)  # exact: small multiples of 1/16
+        want_w, want_c = sref.tc_apply_f32(de.astype(np.float32), da.astype(np.float32), wp, cp)
+        _same_bits(c_dev.cpu().numpy(), want_c, "coherence")
+    else:
+        want_w = sref.td_apply_f64(x0, want_d, wp, tuples, stages, mask)[0].astype(np.float32)
+        _same_bits(c_dev.cpu().numpy(), coh, "coherence")
+    _same_bits(w_dev.cpu().numpy(), want_w, "weights")
+    np.testing.assert_array_equal(pm.cpu().numpy(), want_m, "marks")
+    assert not bool(acc.view(torch.int32).any())
 
 
 @pytest.mark.gpu

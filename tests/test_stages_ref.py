@@ -177,6 +177,14 @@ def test_staged_references_against_loops():
     w2, c2 = sref.tc_update_f32(boards, d, w, coh, tuples, stages, mask)
     w3, c3 = tref.tc_apply_f32(de, da, w, coh)
     np.testing.assert_array_equal(w2.view(np.uint32), w3.view(np.uint32))
+    # TC in float64: sums per entry of x_0's stage, beta from the coherence before the call
+    coh = np.abs(rng.standard_normal((n, 2))).astype(np.float32)
+    w64, e64, a64, cnt, sabs = sref.tc_apply_f64(boards, d, w, coh, tuples, stages, mask)
+    beta = tref.tc_beta_f32(coh).astype(np.float64)
+    hit = sabs != 0
+    np.testing.assert_allclose(w64, np.where(hit, w + beta * de64, w), rtol=0, atol=1e-9)
+    np.testing.assert_allclose(e64, np.where(hit, coh[:, 0] + de64, coh[:, 0]), rtol=0, atol=1e-9)
+    np.testing.assert_array_equal(cnt, sref.td_apply_f64(boards, d, w, tuples, stages, mask)[1])
     # TD(lambda): every window board valued on its own stage
     h = 3
     ring = _boards(rng, (h + 1) * m).reshape(h + 1, m, 16)

@@ -6,6 +6,9 @@ definition in tests/_lambda_ref.py.
 - Exact cases, both rules: delta bit for bit for K = 1 / 4 / 16, M = 1, 255, 257, h = 1, 3, 16, every newest slot, ends inside
   the windows, with and without a mask; weights (and E / A for TC) bit for bit where x_0's entries are pairwise disjoint
   (K = 1 / 4) or where every sum is exact in any order (K = 16, dyadic values); canary words around every buffer.
+- h = 16 at M = 2^23 + 5, where the after ring passes 2^31 bytes, both rules and once with stages: x_0 in the first and in
+  the last slot, a mask of rows at both ends and a seeded sample; delta bit for bit there and 0 elsewhere, the weights
+  within the float32 bound of the float64 reference over the sampled rows.
 - h = 1 equals ntuple_td_update and ntuple_tc_update on colliding games: delta, weights and coherence bit for bit.
 - CUDA-graph replay against eager, both rules.
 - The learner with horizon=3, both rules: the first 3 steps after reset() update nothing; each later delta equals the
@@ -23,6 +26,7 @@ import torch
 
 import _lambda_ref as ref
 import _ntuple_ref as nref
+import _stage_ref as sref
 import _tc_ref as tref
 from _ntuple_gpu import _gpu, ops  # noqa: F401 (ops is a fixture)
 from test_tc import _coherence, _disjoint_rows, _guarded, _played_boards, _same_bits, _zero_bits
@@ -103,6 +107,58 @@ def test_lambda_update_exact_cases(ops, shape, rule):
     w_ok()
     c_ok()
     a_ok()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("rule,stages", [("td0", ()), ("tc", ()), ("tc", (3, 5))])
+def test_lambda_update_beyond_2gib_of_ring(ops, rule, stages):
+    """h = 16, M = 2^23 + 5: the after ring is (17, M, 16) bytes, 2.28 GB, so the byte offsets of slots 8 and up pass 2^31.
+    newest = 16 (x_0 in slot 0, x_h in the last slot) and newest = 15 (x_0 in the last slot).  The mask selects rows at both
+    ends of M and a seeded sample: delta is 0 everywhere else (checked on the device), bit for bit the reference's on the
+    selected rows, and the weights (and E / A) within the float32 bound of the float64 reference over those rows alone.
+    0.5-0.8 s per case on one B200 (power limit not recorded)."""
+    from test_ntuple import _td_tolerance_check
+    from test_stages import SMALL
+    from test_tc import _tc_tolerance_check
+
+    dev = _gpu()
+    h, m, lam, alpha = 16, (1 << 23) + 5, 0.5, 0.01
+    tuples = SMALL
+    n = sref.num_weights(tuples, stages)
+    rng = np.random.default_rng(50 + len(stages) + (rule == "tc"))
+    g = torch.Generator(device=dev)
+    g.manual_seed(51)
+    after = torch.randint(0, 18, (h + 1, m, 16), dtype=torch.uint8, device=dev, generator=g)
+    table = torch.tensor([0.0, 4.0, 8.0, 256.0], device=dev)
+    reward = table[torch.randint(0, 4, (h + 1, m), device=dev, generator=g)]
+    ended = (torch.rand((h + 1, m), device=dev, generator=g) < 0.05).to(torch.uint8)
+    rows = np.unique(np.concatenate([np.arange(256), np.arange(m - 256, m), rng.integers(0, m, 8192)]))
+    r_dev = torch.from_numpy(rows).to(dev)
+    mask = torch.zeros(m, dtype=torch.uint8, device=dev)
+    mask[r_dev] = 1
+    rings = (after[:, r_dev].cpu().numpy(), reward[:, r_dev].cpu().numpy(), ended[:, r_dev].cpu().numpy())
+    w = (rng.standard_normal(n) * 10).astype(np.float32)
+    c = _coherence(rng, n, "random")
+    for newest in (16, 15):
+        w_dev, c_dev = torch.from_numpy(w).to(dev), torch.from_numpy(c).to(dev)
+        acc = torch.zeros((n, 2), device=dev)
+        d = _update(ops, rule, (after, reward, ended), newest, w_dev, c_dev, acc, tuples, alpha=alpha, lam=lam, mask=mask,
+                    stages=stages)
+        assert not bool(d[mask == 0].any()), "a masked-out game has a delta"
+        want_d, x0 = sref.ring_delta(*rings, newest, w, tuples, stages, lam, alpha)
+        np.testing.assert_array_equal(x0, after[(newest + 1) % (h + 1)][r_dev].cpu().numpy())
+        _same_bits(d[r_dev].cpu().numpy(), want_d)
+        if rule == "tc":
+            w64, e64, a64, adds, sabs = sref.tc_apply_f64(x0, want_d, w, c, tuples, stages)
+            _tc_tolerance_check(w_dev.cpu().numpy(), c_dev.cpu().numpy(), w, c, w64, e64, a64, adds, sabs)
+            _zero_bits(acc)
+        else:
+            w64, adds, sabs = sref.td_apply_f64(x0, want_d, w, tuples, stages)
+            _td_tolerance_check(w_dev.cpu().numpy(), w, w64, adds, sabs)
+            assert torch.equal(c_dev.cpu(), torch.from_numpy(c))
+        assert adds.any()
+    del after, reward, ended, mask, d
+    torch.cuda.empty_cache()
 
 
 # ---- h = 1 is TD(0) / TC ------------------------------------------------------------------------------
